@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the flow-based temporal-consistency hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 A step = one pass of the fused warp + occlusion-mask + masked-error kernel over this rank's shard
 of synthetic frame pairs (default workload: the full Sintel-shape evaluation, 23 sequences /
@@ -24,6 +24,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the benchmark leaves the tree as it found it (it may be read-only)
 
 BYTES_PER_PX = {"fp32": 40, "bf16": 28}  # SURVEY.md 8(d): ff 8 + bf 8 + prev 4C|2C + cur 4C|2C, C = 3
 
@@ -39,7 +40,18 @@ def parse():
     ap.add_argument("--frames", default="smooth", choices=["smooth", "white"])
     ap.add_argument("--no-extras", action="store_true", help="skip e2e / cpu_baseline / other workloads")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float64)")
     return ap.parse_args()
+
+
+def dump_outputs(out_dir, out):
+    """The arrays the timed call (tcl_b200.evaluate_sharded) returned in its last step, one DIR/<name>.npy each.  The inputs
+    are seeded, so two builds run with the same arguments can be compared output for output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().cpu().numpy().astype(np.float64))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -742,6 +754,8 @@ def main():
     torch.cuda.synchronize()
     torch.cuda.cudart().cudaProfilerStop()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:     # (the aggregate is all-reduced: every rank holds the same arrays)
+        dump_outputs(args.dump_outputs, last["out"])
     n_launches = int(lib.tclb200_debug_launch_count(0))   # kernels of libtcl_b200.so launched inside the timed region
     import ctypes
     tile_stats = (ctypes.c_ulonglong * 2)()

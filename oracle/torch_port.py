@@ -6,9 +6,9 @@ may import it.  The product package never does.
 
 It issues the SAME sequence of ATen ops as the reference functions it restates, so that
 
-* on CPU it is bit-identical to the imported reference (checked in
-  ``tests/test_oracle_pinning.py`` whenever ``/root/reference`` is present), and
-* on the GPU box (where ``/root/reference`` does not exist) it reproduces what the
+* on CPU it is bit-identical to the reference (checked in ``tests/test_oracle_pinning.py``
+  against the reference's outputs stored in ``tests/golden/ref_cpu_*.npz``), and
+* on a GPU it reproduces what the
   reference would compute on CUDA -- the arithmetic lives in ATen's ``grid_sampler_2d``,
   ``linalg_vector_norm``, ``constant_pad_nd`` and elementwise kernels, not in the
   reference's Python.

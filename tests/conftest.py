@@ -10,7 +10,6 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-REFERENCE_ROOT = os.environ.get("TCL_REFERENCE_ROOT", "/root/reference")
 
 
 def pytest_configure(config):
@@ -49,17 +48,3 @@ def oracle_mod():
     import oracle
     oracle.build()
     return oracle
-
-
-@pytest.fixture(scope="session")
-def reference():
-    """The reference's own modules, imported by path (build container only)."""
-    if not os.path.isdir(os.path.join(REFERENCE_ROOT, "utils")):
-        pytest.skip("reference checkout not present (GPU box)")
-    import torch
-    torch.Tensor.cuda = lambda self, *a, **k: self  # flowtools.py:25 hard-codes .cuda()
-    sys.path.insert(0, os.path.join(REFERENCE_ROOT, "utils"))
-    sys.path.insert(0, os.path.join(REFERENCE_ROOT, "methods", "learning-based"))
-    import flowtools
-    import fs_lib
-    return flowtools, fs_lib

@@ -1,10 +1,10 @@
 """Generate tests/golden/ref_cpu_*.npz by RUNNING THE REFERENCE'S OWN FUNCTIONS (imported by path,
-never copied) on small seeded inputs.  Run in the build container, where /root/reference is mounted:
+never copied) on small seeded inputs, with TCL_REFERENCE_ROOT naming a checkout of the reference repository:
 
-    python tests/golden/make_golden.py
+    TCL_REFERENCE_ROOT=<reference checkout> python tests/golden/make_golden.py
 
-The reference hard-codes ``.cuda()`` (utils/flowtools.py:25) and ``device="cuda"``; on this CPU-only
-container the former is neutralised by patching ``torch.Tensor.cuda`` to the identity and the latter
+The reference hard-codes ``.cuda()`` (utils/flowtools.py:25) and ``device="cuda"``; on a CPU-only
+machine the former is neutralised by patching ``torch.Tensor.cuda`` to the identity and the latter
 by passing ``device="cpu"`` -- the arithmetic then runs in ATen's CPU kernels (torch 2.11.0).
 The CUDA-flavour vectors (``ref_cuda_*.npz``) are produced on a B200 by tests/golden/make_golden_cuda.py with
 oracle/torch_port.py, which tests/test_oracle_pinning.py proves bit-identical to these functions on CPU.
@@ -15,7 +15,7 @@ import sys
 import numpy as np
 import torch
 
-REF = os.environ.get("TCL_REFERENCE_ROOT", "/root/reference")
+REF = os.environ["TCL_REFERENCE_ROOT"]
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 

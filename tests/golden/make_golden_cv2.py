@@ -1,10 +1,10 @@
 """Generate tests/golden/ref_cv2_*.npz by RUNNING THE REFERENCE'S OWN dataset-generation functions (cv2 + NumPy):
 
-    python tests/golden/make_golden_cv2.py
+    TCL_REFERENCE_ROOT=<reference checkout> python tests/golden/make_golden_cv2.py
 
 The generator scripts import ``imageio`` (absent here), so their def blocks -- warp_image / warp_flow / fb_check,
 methods/learning-based/dataset-generation/coco-generation.py:66-113 and hollywood2-generation.py:63-111 -- are executed
-from the source files where they lie under /root/reference (never copied).  cv2 4.13.0, numpy 2.3.
+from the source files where they lie under TCL_REFERENCE_ROOT (never copied).  cv2 4.13.0, numpy 2.3.
 """
 import os
 import sys
@@ -12,7 +12,7 @@ import sys
 import cv2
 import numpy as np
 
-REF = os.environ.get("TCL_REFERENCE_ROOT", "/root/reference")
+REF = os.environ["TCL_REFERENCE_ROOT"]
 GEN = os.path.join(REF, "methods", "learning-based", "dataset-generation")
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(HERE))

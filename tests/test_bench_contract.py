@@ -1,10 +1,12 @@
 """CPU suite: the bench.py contract that can be checked without a GPU -- the reference arm prints one JSON line with the
-keys the driver reads, and the product arm refuses to run (no CPU fallback) instead of silently measuring something else."""
+contract's keys, and the product arm refuses to run (no CPU fallback) instead of silently measuring something else.
+GPU suite: the product arm's --dump-outputs and --steps."""
 import json
 import os
 import subprocess
 import sys
 
+import pytest
 import torch
 
 from conftest import ROOT
@@ -37,6 +39,28 @@ def test_product_arm_refuses_to_run_without_a_gpu():
         pytest.skip("this check is for the GPU-less build container")
     r = run("--steps", "1", "--warmup", "1")
     assert r.returncode != 0 and "no CPU fallback" in (r.stderr + r.stdout)
+
+
+@pytest.mark.gpu
+def test_dump_outputs_repeat_and_steps_set_the_timed_steps(tmp_path):
+    """--dump-outputs writes the last timed step's arrays (evaluate_sharded's dict) as float64 .npy; the seeded inputs make
+    them identical from run to run, whatever the step count.  --steps K runs K timed steps: twice the steps, twice the
+    library launches inside the timed region."""
+    import numpy as np
+    dumps, lines = [], []
+    for steps in (3, 6):
+        out = tmp_path / f"steps{steps}"
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", "1", "--pairs", "16",
+                            "--no-extras", "--dump-outputs", str(out)], capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-2000:]
+        lines.append(json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1]))
+        dumps.append({p.stem: np.load(p) for p in out.glob("*.npy")})
+    assert [d["steps"] for d in lines] == [3, 6] and lines[1]["gpu_launches"] == 2 * lines[0]["gpu_launches"] > 0
+    assert set(dumps[0]) == {"per_sequence_mean", "mean_over_sequences", "mean_over_pairs", "pooled_rmse", "n_pairs"}
+    for k, a in dumps[0].items():
+        assert a.dtype == np.float64 and np.array_equal(a, dumps[1][k]), k
+    assert float(dumps[0]["n_pairs"]) == 16
+    assert float(dumps[0]["mean_over_sequences"]) == float.fromhex(lines[0]["result_check"]["mean_over_sequences_rmse_hex"])
 
 
 def test_committed_product_lines_carry_the_contract_and_are_self_consistent():

@@ -1,35 +1,17 @@
 """NumPy / OpenCV flavour of the path (SURVEY.md section 8f rank 4): oracle pinning on CPU, kernel parity on the GPU.
 
 CPU suite: ``oracle/cv2_port.py`` (a NumPy restatement of cv2.remap's fixed-point bilinear sampling and of the
-generators' ``fb_check``) is pinned bit for bit against ``cv2.remap`` itself and against the reference's own functions,
-executed from their source in the build container; small golden vectors made by those functions
-(tests/golden/make_golden_cv2.py) travel to the GPU box.
+generators' ``fb_check``) is pinned bit for bit against ``cv2.remap`` itself and against small golden vectors made by the
+reference's own functions (tests/golden/make_golden_cv2.py).
 GPU suite: ``tcl_b200.cv2compat`` (csrc/tcl_cv2.cu) against the oracle -- bit-exact for the remap (tolerance 0) and the
 mask -- and against the golden vectors.
 """
-import os
-
 import numpy as np
 import pytest
 import torch
 
-from conftest import GOLDEN, REFERENCE_ROOT, golden_files, load_npz
+from conftest import golden_files, load_npz
 from oracle import cv2_port as cp
-
-GEN_DIR = os.path.join(REFERENCE_ROOT, "methods", "learning-based", "dataset-generation")
-
-
-def load_reference_defs(fname, first, last):
-    """exec the def blocks of a generator script (the scripts import imageio, which is absent, so they cannot be
-    imported as modules); build container only."""
-    path = os.path.join(GEN_DIR, fname)
-    if not os.path.exists(path):
-        pytest.skip("reference checkout not present (GPU box)")
-    cv2 = pytest.importorskip("cv2")
-    src = "".join(open(path).readlines()[first - 1:last])
-    ns = {"np": np, "cv2": cv2}
-    exec(compile(src, fname, "exec"), ns)
-    return ns
 
 
 def flows(H, W, amp, seed):
@@ -68,21 +50,10 @@ def test_oracle_remap_extreme_coordinates_equal_cv2():
     assert np.array_equal(cp.remap_linear(A, x, y), cv2.remap(A, x, y, cv2.INTER_LINEAR))
 
 
-@pytest.mark.parametrize("H,W,amp,seed", CASES)
-def test_oracle_equals_reference_functions_bitwise(H, W, amp, seed):
-    coco = load_reference_defs("coco-generation.py", 66, 113)          # fb_check with the boundary test commented out
-    holly = load_reference_defs("hollywood2-generation.py", 63, 111)   # both tests
-    ff, bf, img = flows(H, W, amp, seed)
-    assert np.array_equal(cp.warp_flow(img, bf), coco["warp_image"](img, bf))
-    wf = cp.warp_flow(ff, bf)
-    assert np.array_equal(wf, coco["warp_flow"](ff, bf))
-    assert np.array_equal(wf, holly["warp_flow"](ff, bf))
-    assert np.array_equal(cp.fb_check(wf, bf, motion_boundaries=False), coco["fb_check"](wf, bf))
-    assert np.array_equal(cp.fb_check(wf, bf, motion_boundaries=True), holly["fb_check"](wf, bf))
-
-
 @pytest.mark.parametrize("path", golden_files("ref_cv2_"))
 def test_oracle_equals_golden(path):
+    """ref_cv2_*.npz: outputs of the generators' warp_flow / warp_image (coco-generation.py:66-113) and of both fb_check
+    variants (coco: occlusion test only; hollywood2-generation.py:63-111: both tests)."""
     g = load_npz(path)
     wf = cp.warp_flow(g["ff"], g["bf"])
     assert np.array_equal(wf, g["warped_flow"])

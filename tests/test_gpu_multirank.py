@@ -44,7 +44,7 @@ def _worker(rank, world, port, out_dir):
 @pytest.mark.gpu
 def test_two_rank_sharded_evaluation_equals_single_gpu(tcl, tmp_path):
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs two visible GPUs (run with gpurun --gpus 2)")
+        pytest.skip("needs two visible GPUs")
     port = 29600 + (os.getpid() % 2000)
     mp.spawn(_worker, args=(2, port, str(tmp_path)), nprocs=2, join=True)
     device = torch.device("cuda", 0)

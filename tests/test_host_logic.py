@@ -109,20 +109,20 @@ def test_cpu_and_device_forms_of_the_aggregation_share_one_definition(tcl):
     assert float(u["pooled_rmse"]) == 1.0 and float(u["n_pairs"]) == 4.0
 
 
+def _raft_pad(ht, wd, mode):
+    """InputPadder._pad as RAFT publishes it (core/utils/utils.py; vendored upstream as utils/raft/raft/utils/utils.py:7-24)."""
+    pad_ht = (((ht // 8) + 1) * 8 - ht) % 8
+    pad_wd = (((wd // 8) + 1) * 8 - wd) % 8
+    if mode == "sintel":
+        return [pad_wd // 2, pad_wd - pad_wd // 2, pad_ht // 2, pad_ht - pad_ht // 2]
+    return [pad_wd // 2, pad_wd - pad_wd // 2, 0, pad_ht]
+
+
 def test_input_padder_is_the_reference_one(tcl):
-    """sintel_eval.InputPadder against utils/raft/raft/utils/utils.py:7-24 (when the reference checkout is present) and against
+    """sintel_eval.InputPadder against RAFT's InputPadder (its padding, replicate-padded images and unpad) and against
     its definition: replicate padding to multiples of 8, rows split top / bottom in 'sintel' mode."""
-    import importlib.util
-    import os
-    from conftest import REFERENCE_ROOT
+    import torch.nn.functional as F
     ours = tcl.sintel_eval.InputPadder
-    ref_path = os.path.join(REFERENCE_ROOT, "utils", "raft", "raft", "utils", "utils.py")
-    theirs = None
-    if os.path.exists(ref_path):
-        spec = importlib.util.spec_from_file_location("raft_utils_ref", ref_path)
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)
-        theirs = mod.InputPadder
     g = torch.Generator().manual_seed(3)
     for H, W in ((436, 1024), (432, 1024), (44, 61), (8, 8), (7, 9), (1080, 1920)):
         x = torch.rand(1, 3, H, W, generator=g)
@@ -131,9 +131,9 @@ def test_input_padder_is_the_reference_one(tcl):
             (y,) = p.pad(x)
             assert y.shape[-2] % 8 == 0 and y.shape[-1] % 8 == 0 and y.shape[-2] - H < 8 and y.shape[-1] - W < 8
             assert torch.equal(p.unpad(y), x)
-            if theirs is not None:
-                q = theirs(x.shape, mode)
-                assert q._pad == p._pad and torch.equal(q.pad(x)[0], y) and torch.equal(q.unpad(y), x)
+            q = _raft_pad(H, W, mode)
+            assert q == p._pad and torch.equal(F.pad(x, q, mode="replicate"), y)
+            assert torch.equal(y[..., q[2]:y.shape[-2] - q[3], q[0]:y.shape[-1] - q[1]], x)
     assert ours((436, 1024))._pad == [0, 0, 2, 2] and ours((436, 1024), "kitti")._pad == [0, 0, 0, 4]
 
 

@@ -1,7 +1,7 @@
 """CPU suite: pin the oracle (oracle/tcl_oracle.c + oracle/torch_port.py) to the reference.
 
 Chain of evidence:
-  1. torch_port == imported reference functions, bit for bit, on CPU  (same ATen ops)
+  1. torch_port == the reference functions' outputs stored in ref_cpu_*.npz, bit for bit, on CPU  (same ATen ops)
   2. C oracle (ATEN_CPU flavour) == golden vectors produced by the imported reference, bit for bit
   3. C oracle (ATEN_CUDA flavour) == vectors produced on a B200 by torch_port (ref_cuda_*.npz), bit for bit
 The GPU suite then compares the CUDA kernels with the ATEN_CUDA flavour and with torch_port live.
@@ -58,40 +58,45 @@ def test_border_is_masked_for_nonzero_flow(oracle_mod):
 
 
 # ---------------------------------------------------------------- 1. torch_port == reference (CPU)
-@pytest.mark.parametrize("shape", [(2, 24, 40), (1, 61, 33), (1, 108, 192)])
-def test_torch_port_bit_identical_to_reference(reference, tcl, shape):
-    flowtools, fs_lib = reference
-    B, H, W = shape
-    ff, bf, prev, cur = _synth_case(tcl, B, H, W, seed=11, max_shift=6.0)
-    assert torch.equal(flowtools.warp(prev, bf), tp.backward_warp(prev, bf))
-    assert torch.equal(flowtools.fbcCheckTorch(ff, bf, device="cpu"), tp.fb_consistency(ff, bf))
-    assert torch.equal(flowtools.gradient(bf[:, 0]), tp.central_diff(bf[:, 0]))
-    assert torch.equal(fs_lib.warp(prev, bf), tp.validity_warp(prev, bf))
-    m = flowtools.fbcCheckTorch(ff, bf, device="cpu")
-    w = flowtools.warp(prev, bf)
-    assert torch.equal(((m * (cur - w)) ** 2).mean() ** 0.5, tp.temporal_error(ff, bf, prev, cur))
+def _golden_tensors(path):
+    return {k: torch.from_numpy(v) for k, v in load_npz(path).items() if v.dtype.kind == "f"}
 
 
-def test_long_term_step_is_the_upstream_lines(reference, tcl):
-    """obst_eval.py:515-516 (inside a string literal upstream), executed with the imported flowtools functions."""
-    flowtools, _ = reference
-    ff, bf, styled, pre = _synth_case(tcl, 1, 64, 96, seed=5, kind="smooth", max_shift=6.0)
-    mask_last = (torch.rand(1, 1, 64, 96, generator=torch.Generator().manual_seed(1)) > 0.3).float()
-    m = torch.clamp(mask_last - flowtools.fbcCheckTorch(ff, bf, device="cpu"), 0.0, 1.0)
-    want = m * flowtools.warp(styled, bf) + (1 - m) * pre
+@pytest.mark.parametrize("path", golden_files("ref_cpu_"))
+def test_torch_port_bit_identical_to_reference(path):
+    """ref_cpu_*.npz hold what the reference's own flowtools / fs_lib functions returned on CPU (tests/golden/make_golden.py)."""
+    g = _golden_tensors(path)
+    ff, bf, prev, cur = g["ff"], g["bf"], g["prev"], g["cur"]
+    assert torch.equal(g["warp"], tp.backward_warp(prev, bf))
+    assert torch.equal(g["mask"], tp.fb_consistency(ff, bf))
+    assert torch.equal(g["grad_u"], tp.central_diff(bf[:, 0]))
+    assert torch.equal(g["fs_warp"], tp.validity_warp(prev, bf))
+    assert torch.equal(g["rmse"], tp.temporal_error(ff, bf, prev, cur))
+    w = tp.backward_warp(prev, bf)
+    assert torch.equal(g["rmse_per_sample"], tp.tcl_rmse_per_sample(g["mask"], cur, w))
+    assert torch.equal(g["l2"], tp.tcl_l2(g["mask"], cur, w)) and torch.equal(g["l1"], tp.tcl_l1(g["mask"], cur, w))
+
+
+def test_long_term_step_is_the_upstream_lines():
+    """obst_eval.py:515-516 (inside a string literal upstream), composed from the reference's fbcCheckTorch and warp outputs."""
+    g = _golden_tensors(golden_files("ref_cpu_smooth")[0])
+    ff, bf, styled, pre = g["ff"], g["bf"], g["prev"], g["cur"]
+    mask_last = (torch.rand(g["mask"].shape, generator=torch.Generator().manual_seed(1)) > 0.3).float()
+    m = torch.clamp(mask_last - g["mask"], 0.0, 1.0)
+    want = m * g["warp"] + (1 - m) * pre
     got_m, got = tp.long_term_step(mask_last, ff, bf, styled, pre)
     assert torch.equal(got_m, m) and torch.equal(got, want) and 0 < float(m.mean()) < 1
 
 
-def test_reference_autograd_matches_port(reference, tcl):
-    flowtools, _ = reference
-    ff, bf, prev, cur = _synth_case(tcl, 1, 20, 28, seed=3, max_shift=3.0)
-    outs = []
-    for fn in (flowtools.warp, tp.backward_warp):
-        p, f = prev.clone().requires_grad_(True), bf.clone().requires_grad_(True)
-        ((cur - fn(p, f)) ** 2).mean().backward()
-        outs.append((p.grad, f.grad))
-    assert torch.equal(outs[0][0], outs[1][0]) and torch.equal(outs[0][1], outs[1][1])
+def test_reference_autograd_matches_port():
+    """Gradients of the masked L2 loss through the reference's warp (stored by make_golden.py) == through torch_port."""
+    paths = golden_files("ref_cpu_")
+    assert paths
+    for path in paths:
+        g = _golden_tensors(path)
+        p, f, c = (g[k].clone().requires_grad_(True) for k in ("prev", "bf", "cur"))
+        ((g["mask"] * (c - tp.backward_warp(p, f))) ** 2).mean().backward()
+        assert torch.equal(p.grad, g["grad_prev"]) and torch.equal(f.grad, g["grad_flow"]) and torch.equal(c.grad, g["grad_cur"])
 
 
 # ---------------------------------------------------------------- 2. C oracle == golden (reference on CPU)
@@ -130,20 +135,19 @@ def test_c_oracle_backward_matches_reference_autograd(oracle_mod, path):
 
 
 @pytest.mark.parametrize("shape,shift", [((2, 37, 53), 8.0), ((1, 96, 160), 20.0)])
-def test_c_oracle_matches_reference_live_bitwise(reference, oracle_mod, tcl, shape, shift):
-    flowtools, fs_lib = reference
+def test_c_oracle_matches_port_bitwise(oracle_mod, tcl, shape, shift):
+    """Shapes and displacements beyond the golden cases, against torch_port (bit-identical to the reference's outputs, 1. above)."""
     B, H, W = shape
     ff, bf, prev, cur = _synth_case(tcl, B, H, W, seed=21, max_shift=shift)
     v = oracle_mod.ATEN_CPU
-    assert np.array_equal(oracle_mod.warp(prev.numpy(), bf.numpy(), v), flowtools.warp(prev, bf).numpy())
-    ref_mask = flowtools.fbcCheckTorch(ff, bf, device="cpu").numpy()
+    assert np.array_equal(oracle_mod.warp(prev.numpy(), bf.numpy(), v), tp.backward_warp(prev, bf).numpy())
+    ref_mask, pmo, pmm = tp.fb_consistency(ff, bf, return_margins=True)
     mask, mo, mm = oracle_mod.fbcheck(ff.numpy(), bf.numpy(), variant=v, margins=True)
-    assert np.array_equal(mask, ref_mask)
+    assert np.array_equal(mask, ref_mask.numpy())
     # margins (the quantities the 1e-6 exemption band is defined on) are bit-identical too
-    _, pmo, pmm = tp.fb_consistency(ff, bf, return_margins=True)
     assert np.array_equal(mo, pmo.numpy()) and np.array_equal(mm, pmm.numpy())
-    assert 0.2 < ref_mask.mean() < 0.98
-    assert np.array_equal(oracle_mod.validity_warp(prev.numpy(), bf.numpy(), v), fs_lib.warp(prev, bf).numpy())
+    assert 0.2 < float(ref_mask.mean()) < 0.98
+    assert np.array_equal(oracle_mod.validity_warp(prev.numpy(), bf.numpy(), v), tp.validity_warp(prev, bf).numpy())
 
 
 def test_mob_only_variant(oracle_mod, tcl):
@@ -179,26 +183,24 @@ def test_cuda_and_cpu_flavours_differ_only_at_ulp_level(oracle_mod, tcl):
     assert (ma != mb).mean() < 1e-3
 
 
+def _raft_upsample_flow(flow, mask):
+    """RAFT.upsample_flow as published with RAFT (core/raft.py; vendored upstream as utils/raft/raft/raft.py:72-83):
+    softmax over the 9 logits, unfold of 8*flow, weighted sum, permute -- the formulation torch_port restates with shifts."""
+    import torch.nn.functional as F
+    N, _, H, W = flow.shape
+    mask = torch.softmax(mask.view(N, 1, 9, 8, 8, H, W), dim=2)
+    up_flow = F.unfold(8 * flow, [3, 3], padding=1).view(N, 2, 9, 1, 1, H, W)
+    up_flow = torch.sum(mask * up_flow, dim=2).permute(0, 1, 4, 2, 5, 3)
+    return up_flow.reshape(N, 2, 8 * H, 8 * W)
+
+
 def test_upsample_restatement_matches_reference_raft():
-    """oracle/torch_port.upsample_flow against the reference's own RAFT.upsample_flow (imported by path, CPU)."""
-    import os
-    import sys
-    import torch
-    from conftest import REFERENCE_ROOT
-    raft_dir = os.path.join(REFERENCE_ROOT, "utils", "raft", "raft")
-    if not os.path.isdir(raft_dir):
-        pytest.skip("reference checkout not present (GPU box)")
-    sys.path.insert(0, raft_dir)
-    try:
-        import raft as ref_raft
-    except Exception as ex:   # the vendored RAFT has path-dependent imports
-        pytest.skip(f"reference RAFT not importable here: {ex!r}")
-    from oracle import torch_port as tp
+    """oracle/torch_port.upsample_flow against RAFT's own unfold formulation of upsample_flow (CPU)."""
     g = torch.Generator().manual_seed(7)
     for (n, h, w) in [(1, 6, 7), (2, 9, 11), (1, 55, 128)]:
         flow = torch.randn(n, 2, h, w, generator=g) * 5
         mask = torch.randn(n, 576, h, w, generator=g) * 3
-        want = ref_raft.RAFT.upsample_flow(None, flow, mask)     # utils/raft/raft/raft.py:72-83
+        want = _raft_upsample_flow(flow, mask)
         got = tp.upsample_flow(flow, mask)
         assert got.shape == want.shape
         assert torch.allclose(got, want, rtol=1e-6, atol=1e-6)
