@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 LIB_PATH = os.environ.get("TCL_B200_LIB") or os.path.join(CSRC, "libtcl_b200.so")  # env override: tuning sweeps only
 HEADER = os.path.join(os.path.dirname(_HERE), "include", "tcl_b200.h")
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 # enums mirrored from include/tcl_b200.h
 F32, BF16 = 0, 1
@@ -123,6 +123,10 @@ _PROTOTYPES = {
     "tclb200_tcl_forward_host": (_c.c_int, [_c.POINTER(HostArgs), _vp]),
     "tclb200_tcl_backward": (_c.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "tclb200_tcl_backward_scaled": (_c.c_int, [_vp, _vp, _vp, _vp, _vp, _c.c_float, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
+    "tclb200_backward_workspace_bytes": (_c.c_size_t, [_i, _i, _i, _i, _i]),
+    "tclb200_warp_backward_dt": (_c.c_int, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _c.c_size_t, _vp]),
+    "tclb200_tcl_backward_dt": (_c.c_int, [_vp, _vp, _vp, _vp, _vp, _c.c_float, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp,
+                                           _c.c_size_t, _vp]),
     "tclb200_hwc_split": (_c.c_int, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
     "tclb200_occlusion_u8_to_mask": (_c.c_int, [_vp, _vp, _c.c_size_t, _vp]),
     "tclb200_upsample_flow": (_c.c_int, [_vp, _vp, _vp, _i, _i, _i, _vp]),

@@ -28,6 +28,9 @@ __device__ __forceinline__ float ld_stream(const float* p) { return __ldcs(p); }
 __device__ __forceinline__ float ld_stream(const __nv_bfloat16* p) {
   return __bfloat162float(__ushort_as_bfloat16(__ldcs(reinterpret_cast<const unsigned short*>(p))));
 }
+// read-only gather through the non-coherent cache (bilinear taps that neighbouring lanes re-read)
+__device__ __forceinline__ float ld_gather(const float* p) { return __ldg(p); }
+__device__ __forceinline__ float ld_gather(const __nv_bfloat16* p) { return __bfloat162float(__ldg(p)); }
 __device__ __forceinline__ void st_stream(float* p, float v) { __stcs(p, v); }
 __device__ __forceinline__ void st_stream(__nv_bfloat16* p, float v) {
   __stcs(reinterpret_cast<unsigned short*>(p), __bfloat16_as_ushort(__float2bfloat16_rn(v)));

@@ -1629,18 +1629,19 @@ __global__ void __launch_bounds__(kThreads) gradient_vec4_kernel(const float* __
 
 // ---------------------------------------------------------------------------------------------
 // backward kernels.  One lane per target pixel; grad_prev is a bilinear scatter-add (red.global.add.f32).
+// Frames (x / prev, cur, grad_out, grad_cur) are fp32 or bf16; flows, masks and the scatter target are always fp32.
 // ---------------------------------------------------------------------------------------------
 struct BwdParams {
-  const float* grad_out;   // warp_backward: (B,C,H,W); tcl_backward: unused
-  const float* x;          // source frame (prev)
+  const void* grad_out;    // warp_backward: (B,C,H,W) frame dtype; tcl_backward: unused
+  const void* x;           // source frame (prev), frame dtype
   const float* f;          // flow
   const float* mask;       // tcl_backward only
-  const float* cur;        // tcl_backward only
+  const void* cur;         // tcl_backward only, frame dtype
   const float* grad_scale; // tcl_backward only (device scalar)
   float scale_mul;         // tcl_backward only: host factor applied to *grad_scale (1/(B*C*H*W) for the mean loss)
-  float* grad_x;
+  float* grad_x;           // fp32 frames: the output itself; bf16 frames: the fp32 accumulator (workspace) it is rounded from
   float* grad_f;
-  float* grad_cur;
+  void* grad_cur;          // frame dtype
   Geo geo;
   int B, C, flags, loss;
 };
@@ -1656,12 +1657,19 @@ struct BwdParams {
 // FUSED_LOSS: the upstream gradient of warp is derived in-kernel from the masked loss.
 // CT > 0 fixes the channel count at compile time: all 4*CT gathers and the CT `cur` / grad_out loads of a pixel are then
 // issued back to back (the kernel is latency-bound otherwise: measured 10 long-scoreboard stall cycles per issue).
-template <bool FUSED_LOSS, int CT>
+// FrameT = __nv_bfloat16: frame loads are converted to fp32 and the arithmetic is the fp32 kernel's, so grad_f and the
+// fp32 grad_cur are bit for bit those of the fp32 kernel on the upcast frames; grad_cur is rounded once on the store.
+// grad_x goes to an fp32 accumulator (red.add.bf16x2 would round on every add) that bwd_acc_to_bf16_kernel rounds behind.
+template <bool FUSED_LOSS, int CT, typename FrameT>
 #ifndef TCL_BWD_MINB
 #define TCL_BWD_MINB 5   // measured: 5 CTAs per SM (48 registers) beats 4 (59) and 6 (40, spills)
 #endif
 __global__ void __launch_bounds__(256, TCL_BWD_MINB) warp_backward_kernel(const BwdParams p) {
+  if constexpr (sizeof(FrameT) == 2) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");   // the bf16 rounding kernel
   const Geo& g = p.geo;
+  const FrameT* const frame_x = static_cast<const FrameT*>(p.x);
+  const FrameT* const frame_in = static_cast<const FrameT*>(FUSED_LOSS ? p.cur : p.grad_out);
+  FrameT* const frame_gc = static_cast<FrameT*>(p.grad_cur);
   const int W = g.W, H = g.H, C = CT > 0 ? CT : p.C;
   const size_t plane = (size_t)H * W;
   // 32 x 8 pixel tiles: lanes along x (coalesced loads / stores, neighbouring lanes scatter into neighbouring addresses)
@@ -1715,7 +1723,7 @@ __global__ void __launch_bounds__(256, TCL_BWD_MINB) warp_backward_kernel(const 
         const float d = wv - in;
         gc = -scale * m * (d > 0.0f ? 1.0f : (d < 0.0f ? -1.0f : 0.0f));
       }
-      if (p.grad_cur) __stcs(p.grad_cur + base + o, gc);
+      if (frame_gc) st_stream(frame_gc + base + o, gc);
       go = -gc;
     } else {
       go = in;
@@ -1738,28 +1746,48 @@ __global__ void __launch_bounds__(256, TCL_BWD_MINB) warp_backward_kernel(const 
 #pragma unroll
     for (int c = 0; c < CU; ++c) {   // every load of this pixel in flight before the first use
       const size_t base = ((size_t)b * C + c) * plane;
-      const float* xp = p.x + base;
-      v00[c] = (need_taps && p00) ? __ldg(xp + o00) : 0.0f;
-      v10[c] = (need_taps && p10) ? __ldg(xp + o00 + 1) : 0.0f;
-      v01[c] = (need_taps && p01) ? __ldg(xp + o00 + W) : 0.0f;
-      v11[c] = (need_taps && p11) ? __ldg(xp + o00 + W + 1) : 0.0f;
-      in[c] = FUSED_LOSS ? __ldcs(p.cur + base + o) : __ldcs(p.grad_out + base + o);
+      const FrameT* xp = frame_x + base;
+      v00[c] = (need_taps && p00) ? ld_gather(xp + o00) : 0.0f;
+      v10[c] = (need_taps && p10) ? ld_gather(xp + o00 + 1) : 0.0f;
+      v01[c] = (need_taps && p01) ? ld_gather(xp + o00 + W) : 0.0f;
+      v11[c] = (need_taps && p11) ? ld_gather(xp + o00 + W + 1) : 0.0f;
+      in[c] = ld_stream(frame_in + base + o);
     }
 #pragma unroll
     for (int c = 0; c < CU; ++c) channel(c, v00[c], v10[c], v01[c], v11[c], in[c]);
   } else {
     for (int c = 0; c < C; ++c) {
       const size_t base = ((size_t)b * C + c) * plane;
-      const float* xp = p.x + base;
-      const float a00 = (need_taps && p00) ? __ldg(xp + o00) : 0.0f, a10 = (need_taps && p10) ? __ldg(xp + o00 + 1) : 0.0f;
-      const float a01 = (need_taps && p01) ? __ldg(xp + o00 + W) : 0.0f, a11 = (need_taps && p11) ? __ldg(xp + o00 + W + 1) : 0.0f;
-      channel(c, a00, a10, a01, a11, FUSED_LOSS ? __ldcs(p.cur + base + o) : __ldcs(p.grad_out + base + o));
+      const FrameT* xp = frame_x + base;
+      const float a00 = (need_taps && p00) ? ld_gather(xp + o00) : 0.0f, a10 = (need_taps && p10) ? ld_gather(xp + o00 + 1) : 0.0f;
+      const float a01 = (need_taps && p01) ? ld_gather(xp + o00 + W) : 0.0f, a11 = (need_taps && p11) ? ld_gather(xp + o00 + W + 1) : 0.0f;
+      channel(c, a00, a10, a01, a11, ld_stream(frame_in + base + o));
     }
   }
   if (p.grad_f) {
     // d ix/d gx = W/2 (grid_sampler), d gx/d u = 2/(W-1) (flowtools.py:28)
     p.grad_f[(size_t)b * 2 * plane + o] = 2.0f * (g.Wf * 0.5f * gix) / g.dxf;
     p.grad_f[((size_t)b * 2 + 1) * plane + o] = 2.0f * (g.Hf * 0.5f * giy) / g.dyf;
+  }
+}
+
+// grad_x of bf16 frames: the fp32 accumulator the scatter-add left, rounded once (__float2bfloat16_rn, what torch's
+// .to(torch.bfloat16) does).  Launched behind warp_backward_kernel with programmatic dependent launch.  Four values per
+// lane: one 16-byte load, one 8-byte store (vec = the output is 8-byte aligned; the accumulator always is 16-byte aligned).
+__global__ void __launch_bounds__(kThreads) bwd_acc_to_bf16_kernel(const float* __restrict__ acc, __nv_bfloat16* __restrict__ out,
+                                                                   size_t n, int vec) {
+  asm volatile("griddepcontrol.wait;" ::: "memory");   // every red of the scatter has landed after this
+  const size_t i = ((size_t)blockIdx.x * kThreads + threadIdx.x) * 4;
+  if (i >= n) return;
+  if (vec && i + 4 <= n) {
+    const float4 v = __ldcs(reinterpret_cast<const float4*>(acc + i));
+    const __nv_bfloat162 lo = __floats2bfloat162_rn(v.x, v.y), hi = __floats2bfloat162_rn(v.z, v.w);
+    uint2 w;
+    w.x = *reinterpret_cast<const unsigned*>(&lo);
+    w.y = *reinterpret_cast<const unsigned*>(&hi);
+    __stcs(reinterpret_cast<uint2*>(out + i), w);
+  } else {
+    for (size_t k = i; k < n && k < i + 4; ++k) st_stream(out + k, __ldcs(acc + k));
   }
 }
 
@@ -2305,50 +2333,94 @@ extern "C" int tclb200_gradient_strided(const float* x, size_t x_batch_stride, f
   return run_gradient(x, x_batch_stride, out, B, H, W, reinterpret_cast<cudaStream_t>(stream));
 }
 
-static int run_backward(const BwdParams& p, bool fused, cudaStream_t s) {
+template <typename FrameT>
+static void launch_backward(const BwdParams& p, bool fused, dim3 grid, cudaStream_t s) {
+  if (fused) {
+    if (p.C == 3) warp_backward_kernel<true, 3, FrameT><<<grid, 256, 0, s>>>(p);
+    else warp_backward_kernel<true, 0, FrameT><<<grid, 256, 0, s>>>(p);
+  } else {
+    if (p.C == 3) warp_backward_kernel<false, 3, FrameT><<<grid, 256, 0, s>>>(p);
+    else if (p.C == 2) warp_backward_kernel<false, 2, FrameT><<<grid, 256, 0, s>>>(p);
+    else warp_backward_kernel<false, 0, FrameT><<<grid, 256, 0, s>>>(p);
+  }
+}
+
+// bf16 frames: p.grad_x is the fp32 accumulator and grad_x_bf16 the caller's output it is rounded into
+static int run_backward(const BwdParams& p, bool fused, int dtype, __nv_bfloat16* grad_x_bf16, cudaStream_t s) {
   const size_t n = (size_t)p.B * p.geo.H * p.geo.W;
+  if (dtype == TCLB200_BF16 && p.grad_x && n * p.C / (4 * kThreads) >= 0x7fffffffu)
+    return fail(TCLB200_ERR_UNSUPPORTED, "too many elements for one rounding launch");
   if (p.grad_x) CUDA_TRY(cudaMemsetAsync(p.grad_x, 0, n * p.C * sizeof(float), s));
   if (p.B > 65535) return fail(TCLB200_ERR_UNSUPPORTED, "batch too large for one backward launch");
   const dim3 grid((unsigned)cdiv(p.geo.W, 32), (unsigned)cdiv(p.geo.H, 8), (unsigned)p.B);
   if (grid.y > 65535) return fail(TCLB200_ERR_UNSUPPORTED, "image too tall for one backward launch");
-  if (fused) {
-    if (p.C == 3) warp_backward_kernel<true, 3><<<grid, 256, 0, s>>>(p);
-    else warp_backward_kernel<true, 0><<<grid, 256, 0, s>>>(p);
-  } else {
-    if (p.C == 3) warp_backward_kernel<false, 3><<<grid, 256, 0, s>>>(p);
-    else if (p.C == 2) warp_backward_kernel<false, 2><<<grid, 256, 0, s>>>(p);
-    else warp_backward_kernel<false, 0><<<grid, 256, 0, s>>>(p);
-  }
+  if (dtype == TCLB200_BF16) launch_backward<__nv_bfloat16>(p, fused, grid, s);
+  else launch_backward<float>(p, fused, grid, s);
   ++g_launches;
   CUDA_TRY(cudaGetLastError());
+  if (dtype == TCLB200_BF16 && p.grad_x) {
+    const size_t count = n * p.C;
+    cudaLaunchConfig_t cfg;
+    memset(&cfg, 0, sizeof(cfg));
+    cfg.gridDim = dim3((unsigned)((count + 4 * kThreads - 1) / (4 * kThreads))); cfg.blockDim = dim3(kThreads); cfg.stream = s;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr; cfg.numAttrs = 1;
+    const int vec = (reinterpret_cast<uintptr_t>(grad_x_bf16) & 7u) == 0;
+    ++g_launches;
+    CUDA_TRY(cudaLaunchKernelEx(&cfg, bwd_acc_to_bf16_kernel, (const float*)p.grad_x, grad_x_bf16, count, vec));
+  }
   return TCLB200_OK;
 }
 
-extern "C" int tclb200_warp_backward(const float* grad_out, const float* x, const float* f, float* grad_x, float* grad_f,
-                                     int B, int C, int H, int W, int flags, tclb200_stream_t stream) {
+extern "C" size_t tclb200_backward_workspace_bytes(int B, int C, int H, int W, int dtype) {
+  if (dtype != TCLB200_BF16 || B <= 0 || C <= 0 || H <= 0 || W <= 0) return 0;
+  return align_up((size_t)B * C * H * W * sizeof(float), 256);
+}
+
+// the frame dtype and, for bf16 frames with a grad_x / grad_prev, the accumulator workspace: p.grad_x is pointed at it
+static int backward_dtype_setup(BwdParams& p, int dtype, void* grad_x, void* workspace, size_t workspace_bytes, const char* what) {
+  if (dtype != TCLB200_F32 && dtype != TCLB200_BF16) return fail(TCLB200_ERR_INVALID, "unknown dtype");
+  if (dtype == TCLB200_F32 || grad_x == nullptr) {
+    p.grad_x = static_cast<float*>(grad_x);
+    return TCLB200_OK;
+  }
+  const size_t need = tclb200_backward_workspace_bytes(p.B, p.C, p.geo.H, p.geo.W, dtype);
+  if (workspace == nullptr || workspace_bytes < need) {
+    static thread_local char msg[192];
+    snprintf(msg, sizeof(msg), "%s of bf16 frames needs a workspace of tclb200_backward_workspace_bytes() = %zu bytes, got %zu",
+             what, need, workspace ? workspace_bytes : (size_t)0);
+    return fail(TCLB200_ERR_INVALID, "%s", msg);
+  }
+  if (!aligned16(workspace)) return fail(TCLB200_ERR_INVALID, "workspace must be 16-byte aligned");
+  p.grad_x = static_cast<float*>(workspace);
+  return TCLB200_OK;
+}
+
+extern "C" int tclb200_warp_backward_dt(const void* grad_out, const void* x, const float* f, void* grad_x, float* grad_f,
+                                        int B, int C, int H, int W, int dtype, int flags, void* workspace, size_t workspace_bytes,
+                                        tclb200_stream_t stream) {
   if (!grad_out || !x || !f) return fail(TCLB200_ERR_INVALID, "grad_out, x and f are required");
   if (B <= 0 || C <= 0 || H <= 0 || W <= 0) return fail(TCLB200_ERR_INVALID, "B, C, H, W must be positive");
   if ((size_t)H * W >= (1u << 30)) return fail(TCLB200_ERR_UNSUPPORTED, "H*W must be below 2^30");
   BwdParams p;
   memset(&p, 0, sizeof(p));
-  p.grad_out = grad_out; p.x = x; p.f = f; p.grad_x = grad_x; p.grad_f = grad_f;
+  p.grad_out = grad_out; p.x = x; p.f = f; p.grad_f = grad_f;
   p.geo = make_geo(H, W); p.B = B; p.C = C; p.flags = flags & TCLB200_VALIDITY;
-  return run_backward(p, false, reinterpret_cast<cudaStream_t>(stream));
+  const int rc = backward_dtype_setup(p, dtype, grad_x, workspace, workspace_bytes, "grad_x");
+  if (rc != TCLB200_OK) return rc;
+  return run_backward(p, false, dtype, static_cast<__nv_bfloat16*>(grad_x), reinterpret_cast<cudaStream_t>(stream));
 }
 
-extern "C" int tclb200_tcl_backward_scaled(const float* bf, const float* mask, const float* prev, const float* cur,
-                                           const float* grad_scale, float scale_mul, float* grad_prev, float* grad_cur, int B, int C,
-                                           int H, int W, int flags, int loss, tclb200_stream_t stream);
-
-extern "C" int tclb200_tcl_backward(const float* bf, const float* mask, const float* prev, const float* cur,
-                                    const float* grad_scale, float* grad_prev, float* grad_cur, int B, int C, int H, int W,
-                                    int flags, int loss, tclb200_stream_t stream) {
-  return tclb200_tcl_backward_scaled(bf, mask, prev, cur, grad_scale, 1.0f, grad_prev, grad_cur, B, C, H, W, flags, loss, stream);
+extern "C" int tclb200_warp_backward(const float* grad_out, const float* x, const float* f, float* grad_x, float* grad_f,
+                                     int B, int C, int H, int W, int flags, tclb200_stream_t stream) {
+  return tclb200_warp_backward_dt(grad_out, x, f, grad_x, grad_f, B, C, H, W, TCLB200_F32, flags, nullptr, 0, stream);
 }
 
-extern "C" int tclb200_tcl_backward_scaled(const float* bf, const float* mask, const float* prev, const float* cur,
-                                           const float* grad_scale, float scale_mul, float* grad_prev, float* grad_cur, int B, int C,
-                                           int H, int W, int flags, int loss, tclb200_stream_t stream) {
+extern "C" int tclb200_tcl_backward_dt(const float* bf, const float* mask, const void* prev, const void* cur, const float* grad_scale,
+                                       float scale_mul, void* grad_prev, void* grad_cur, int B, int C, int H, int W, int dtype,
+                                       int flags, int loss, void* workspace, size_t workspace_bytes, tclb200_stream_t stream) {
   if (!bf || !prev || !cur || !grad_scale) return fail(TCLB200_ERR_INVALID, "bf, prev, cur and grad_scale are required");
   if (B <= 0 || C <= 0 || H <= 0 || W <= 0) return fail(TCLB200_ERR_INVALID, "B, C, H, W must be positive");
   if (loss != TCLB200_L2 && loss != TCLB200_L1) return fail(TCLB200_ERR_INVALID, "unknown loss");
@@ -2356,9 +2428,24 @@ extern "C" int tclb200_tcl_backward_scaled(const float* bf, const float* mask, c
   BwdParams p;
   memset(&p, 0, sizeof(p));
   p.x = prev; p.f = bf; p.mask = mask; p.cur = cur; p.grad_scale = grad_scale; p.scale_mul = scale_mul;
-  p.grad_x = grad_prev; p.grad_cur = grad_cur;
+  p.grad_cur = grad_cur;
   p.geo = make_geo(H, W); p.B = B; p.C = C; p.flags = flags & TCLB200_VALIDITY; p.loss = loss;
-  return run_backward(p, true, reinterpret_cast<cudaStream_t>(stream));
+  const int rc = backward_dtype_setup(p, dtype, grad_prev, workspace, workspace_bytes, "grad_prev");
+  if (rc != TCLB200_OK) return rc;
+  return run_backward(p, true, dtype, static_cast<__nv_bfloat16*>(grad_prev), reinterpret_cast<cudaStream_t>(stream));
+}
+
+extern "C" int tclb200_tcl_backward_scaled(const float* bf, const float* mask, const float* prev, const float* cur,
+                                           const float* grad_scale, float scale_mul, float* grad_prev, float* grad_cur, int B, int C,
+                                           int H, int W, int flags, int loss, tclb200_stream_t stream) {
+  return tclb200_tcl_backward_dt(bf, mask, prev, cur, grad_scale, scale_mul, grad_prev, grad_cur, B, C, H, W, TCLB200_F32, flags, loss,
+                                 nullptr, 0, stream);
+}
+
+extern "C" int tclb200_tcl_backward(const float* bf, const float* mask, const float* prev, const float* cur,
+                                    const float* grad_scale, float* grad_prev, float* grad_cur, int B, int C, int H, int W,
+                                    int flags, int loss, tclb200_stream_t stream) {
+  return tclb200_tcl_backward_scaled(bf, mask, prev, cur, grad_scale, 1.0f, grad_prev, grad_cur, B, C, H, W, flags, loss, stream);
 }
 
 extern "C" int tclb200_hwc_split(const float* src, int N, int H, int W, int Cs, int n_out, float* const* dst, const int* c0,

@@ -135,21 +135,37 @@ class _WarpFn(torch.autograd.Function):
     @torch.autograd.function.once_differentiable
     def backward(ctx, grad_out):
         x, f = ctx.saved_tensors
-        if x.dtype != torch.float32:
-            raise RuntimeError("tcl_b200: warp backward is implemented for float32 frames")
-        B, C, H, W = x.shape
         gx, gf = _warp_backward_raw(grad_out, x, f, ctx.flags, ctx.needs_input_grad[0], ctx.needs_input_grad[1])
         return gx, gf, None
 
 
+def _backward_workspace(B, C, H, W, dtype, device):
+    """The fp32 accumulator a bf16 grad_x / grad_prev is scattered into, from torch's caching allocator: stream-ordered
+    reuse makes it safe to drop as soon as the launches are enqueued, and inside a CUDA graph capture it comes from the
+    graph's pool."""
+    nbytes = _cabi.lib().tclb200_backward_workspace_bytes(B, C, H, W, dtype)
+    return torch.empty(nbytes, dtype=torch.uint8, device=device), nbytes
+
+
 def _warp_backward_raw(grad_out, x, f, flags, need_x=True, need_f=True):
-    """Autograd of ``warp`` / ``fs_lib.warp`` on raw tensors (``tclb200_warp_backward``): (grad_x, grad_f)."""
+    """Autograd of ``warp`` / ``fs_lib.warp`` on raw tensors (``tclb200_warp_backward``): (grad_x, grad_f).
+
+    bf16 ``x``: ``grad_out`` is read in bf16 and ``grad_x`` comes back in bf16 (``tclb200_warp_backward_dt``): the fp32
+    gradients of the upcast frame, rounded once."""
     B, C, H, W = x.shape
     gx = torch.empty_like(x) if need_x else None
     gf = torch.empty_like(f) if need_f else None
-    go = grad_out.float().contiguous()
+    if x.dtype == torch.float32:
+        go = grad_out.float().contiguous()
+        with torch.cuda.device(x.device):
+            check(_cabi.lib().tclb200_warp_backward(_ptr(go), _ptr(x), _ptr(f), _ptr(gx), _ptr(gf), B, C, H, W, flags, _stream_handle()))
+        return gx, gf
+    dt = _frame_dtype(x)
+    go = grad_out.to(x.dtype).contiguous()
     with torch.cuda.device(x.device):
-        check(_cabi.lib().tclb200_warp_backward(_ptr(go), _ptr(x), _ptr(f), _ptr(gx), _ptr(gf), B, C, H, W, flags, _stream_handle()))
+        ws, nbytes = _backward_workspace(B, C, H, W, dt, x.device) if need_x else (None, 0)
+        check(_cabi.lib().tclb200_warp_backward_dt(_ptr(go), _ptr(x), _ptr(f), _ptr(gx), _ptr(gf), B, C, H, W, dt, flags, _ptr(ws),
+                                                   nbytes, _stream_handle()))
     return gx, gf
 
 
@@ -616,7 +632,7 @@ class _TemporalLossFn(torch.autograd.Function):
     def backward(ctx, grad_out):
         prev, cur, flow, mask = ctx.saved_tensors
         if prev.dtype != torch.float32:
-            raise RuntimeError("tcl_b200: temporal_loss backward is implemented for float32 frames")
+            return _loss_backward_bf16(ctx, grad_out, prev, cur, flow, mask)
         B, C, H, W = prev.shape
         need_prev, need_cur = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
         gp = torch.empty_like(prev) if need_prev else None
@@ -641,6 +657,23 @@ class _TemporalLossFn(torch.autograd.Function):
         return gp, gc, None, None, None, None
 
 
+def _loss_backward_bf16(ctx, grad_out, prev, cur, flow, mask):
+    """``_TemporalLossFn.backward`` for bf16 frames (``tclb200_tcl_backward_dt``): the fp32 gradients of the upcast frames,
+    each rounded once to bf16 -- what autograd gives the reference expression under ``torch.autocast(..., torch.bfloat16)``."""
+    B, C, H, W = prev.shape
+    dt = _frame_dtype(prev)
+    need_prev, need_cur = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
+    gp = torch.empty_like(prev) if need_prev else None
+    gc = torch.empty_like(cur) if need_cur else None
+    scale = grad_out if (grad_out.dtype == torch.float32 and grad_out.is_cuda) else grad_out.to(device=prev.device, dtype=torch.float32)
+    with torch.cuda.device(prev.device):
+        ws, nbytes = _backward_workspace(B, C, H, W, dt, prev.device) if need_prev else (None, 0)
+        check(_cabi.lib().tclb200_tcl_backward_dt(_ptr(flow), _ptr(mask), _ptr(prev), _ptr(cur), _ptr(scale), 1.0 / float(B * C * H * W),
+                                                  _ptr(gp), _ptr(gc), B, C, H, W, dt, ctx.flags, ctx.loss, _ptr(ws), nbytes,
+                                                  _stream_handle()))
+    return gp, gc, None, None, None, None
+
+
 def temporal_loss(mask, cur, prev, flow, loss="l2", validity=False):
     """Training temporal loss, differentiable w.r.t. ``cur`` and ``prev`` in one fused launch each way; a ``flow`` or ``mask``
     that requires grad gets its gradient too (composed from the differentiable ``warp``, like the reference expression).
@@ -648,6 +681,10 @@ def temporal_loss(mask, cur, prev, flow, loss="l2", validity=False):
     ``loss='l2'``: ((mask*(cur - warp(prev,flow)))**2).mean()      (solver.py:444, fs_ruder.py:97)
     ``loss='l1'``: (mask*abs(warp(prev,flow) - cur)).mean()         (MoGAN cycle_gan_model.py:280-281)
     ``validity`` selects fs_lib.warp for the learning-based trainers.
+
+    bf16 frames: the loss is evaluated in fp32 on the upcast frames and returned as an fp32 scalar; the frames' gradients
+    are the fp32 ones rounded to bf16 -- the reference expression under ``torch.autocast("cuda", torch.bfloat16)``, where
+    ``grid_sampler`` runs in fp32 and ``mask*(cur - w)`` promotes to fp32.
     """
     if not (cur.is_cuda and prev.is_cuda and flow.is_cuda and (mask is None or mask.is_cuda)):
         _require_cuda(mask, cur, prev, flow)
@@ -675,7 +712,11 @@ def temporal_loss(mask, cur, prev, flow, loss="l2", validity=False):
         if flow.requires_grad or mask.requires_grad:
             # a learnable flow (MoGAN's motion network: warp(fake_B, netM_A(bf)), cycle_gan_model.py:177-178,280) or a soft mask that
             # is being trained: the fused backward has no gradient for them, so the loss is composed like the reference expression
-            # from the differentiable warp (gradients to the frame and the flow, tclb200_warp_backward) and autograd's elementwise ops
+            # from the differentiable warp (gradients to the frame and the flow, tclb200_warp_backward) and autograd's elementwise ops.
+            # bf16 frames are upcast first, like autocast does for grid_sampler: the warp and the tail run in fp32 and the value is
+            # an fp32 scalar as on the fused path; autograd rounds the frames' gradients back to bf16
+            if prev.dtype != torch.float32:
+                prev, cur = prev.float(), cur.float()
             w = _warp(prev, flow, flags)
             return ((mask * (cur - w)) ** 2).mean() if code == L2 else (mask * torch.abs(w - cur)).mean()
         if prev.requires_grad or cur.requires_grad:

@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define TCLB200_ABI_VERSION 5
+#define TCLB200_ABI_VERSION 6
 
 #define TCLB200_OK 0
 #define TCLB200_ERR_INVALID 1     /* bad argument (null pointer, non-positive size, unknown enum) */
@@ -63,7 +63,7 @@ typedef void* tclb200_stream_t; /* cudaStream_t */
 
 int tclb200_abi_version(void);
 const char* tclb200_last_error(void);
-/* the compile-time configuration of this build of the library ("abi=5 th=32 bh=40 ... hot_only=0 diag=0 trace=0"): the
+/* the compile-time configuration of this build of the library ("abi=6 th=32 bh=40 ... hot_only=0 diag=0 trace=0"): the
  * wrappers refuse a library built with tuning macros (tools/sweep_build.py) unless it was asked for by name   (ABI v5) */
 const char* tclb200_build_info(void);
 
@@ -86,7 +86,7 @@ int tclb200_warp(const void* x, const float* f, void* out, int B, int C, int H, 
                  tclb200_stream_t stream);
 
 /* autograd of warp(): what F.grid_sample's backward + the grid normalisation give the reference
- * (solver.py:181 g_loss.backward()).  grad_out, x as in tclb200_warp (fp32 only); grad_x (B,C,H,W) fp32 is
+ * (solver.py:181 g_loss.backward()).  grad_out, x as in tclb200_warp (fp32; bf16: tclb200_warp_backward_dt); grad_x (B,C,H,W) fp32 is
  * OVERWRITTEN (zero-filled, then bilinear scatter-add); grad_f (B,2,H,W) fp32.  Either output may be NULL. */
 int tclb200_warp_backward(const float* grad_out, const float* x, const float* f, float* grad_x, float* grad_f, int B,
                           int C, int H, int W, int flags, tclb200_stream_t stream);
@@ -197,7 +197,7 @@ int tclb200_tcl_forward_host(const tclb200_host_args* args, tclb200_stream_t str
  *                                   or L = grad_scale * sum  m*|warp(prev,bf)-cur|      (L1)
  * (solver.py:444-446 + :181; fs_ruder.py:97-106; MoGAN .. :281,285).  grad_scale is a device scalar
  * (upstream gradient times 1/(B*C*H*W) times lambda).  grad_cur (B,C,H,W) fp32 is written; grad_prev
- * (B,C,H,W) fp32 is OVERWRITTEN with the bilinear scatter-add.  Either may be NULL.  fp32 frames only. */
+ * (B,C,H,W) fp32 is OVERWRITTEN with the bilinear scatter-add.  Either may be NULL.  fp32 frames (bf16: tclb200_tcl_backward_dt). */
 int tclb200_tcl_backward(const float* bf, const float* mask, const float* prev, const float* cur,
                          const float* grad_scale, float* grad_prev, float* grad_cur, int B, int C, int H, int W,
                          int flags, int loss, tclb200_stream_t stream);
@@ -207,6 +207,26 @@ int tclb200_tcl_backward(const float* bf, const float* mask, const float* prev, 
 int tclb200_tcl_backward_scaled(const float* bf, const float* mask, const float* prev, const float* cur,
                                 const float* grad_scale, float scale_mul, float* grad_prev, float* grad_cur, int B, int C,
                                 int H, int W, int flags, int loss, tclb200_stream_t stream);
+
+/* Backward of bf16 frames (ABI v6): the entries above with the frame dtype as an argument.  What they compute is the fp32
+ * backward of the upcast frames with each frame gradient rounded to bf16 once (__float2bfloat16_rn, torch's
+ * .to(torch.bfloat16)) -- what the reference gives under torch.autocast(..., torch.bfloat16), where grid_sampler runs in
+ * fp32 on the upcast frames and autograd casts each frame's gradient back.
+ *   x / prev, cur, grad_out, grad_x / grad_prev, grad_cur: `dtype` (TCLB200_F32 / TCLB200_BF16); flows, masks, grad_f and
+ *   grad_scale stay fp32.  grad_f and grad_cur are bit for bit the fp32 entries' results on the upcast frames (rounded
+ *   for grad_cur); grad_x / grad_prev is scattered into `workspace` as fp32, then rounded into the output by a second
+ *   kernel (a bf16 scatter-add would round on every add).
+ *   workspace: device memory, 16-byte aligned, >= tclb200_backward_workspace_bytes(B,C,H,W,dtype) bytes; only needed for
+ *   bf16 frames with grad_x / grad_prev requested (NULL / 0 otherwise; fp32 frames never use it).  Its contents are
+ *   irrelevant; it must stay untouched until the call's work on `stream` has completed.
+ *   TCLB200_ERR_INVALID for an unknown dtype or a missing / too small / misaligned workspace, before any CUDA call.
+ * With dtype = TCLB200_F32 they are tclb200_warp_backward / tclb200_tcl_backward_scaled. */
+size_t tclb200_backward_workspace_bytes(int B, int C, int H, int W, int dtype);  /* 0 for TCLB200_F32 */
+int tclb200_warp_backward_dt(const void* grad_out, const void* x, const float* f, void* grad_x, float* grad_f, int B, int C, int H,
+                             int W, int dtype, int flags, void* workspace, size_t workspace_bytes, tclb200_stream_t stream);
+int tclb200_tcl_backward_dt(const float* bf, const float* mask, const void* prev, const void* cur, const float* grad_scale,
+                            float scale_mul, void* grad_prev, void* grad_cur, int B, int C, int H, int W, int dtype, int flags,
+                            int loss, void* workspace, size_t workspace_bytes, tclb200_stream_t stream);
 
 /* Dataset ingest ("next" row of the scope table): HWC -> planar NCHW de-interleave on the GPU.
  *   - the 9-channel FlyingChairs2 / Hollywood2 blocks [img1 3 | img2 3 | mask 1 | flow 2]
