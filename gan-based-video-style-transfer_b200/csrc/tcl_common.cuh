@@ -84,7 +84,7 @@ struct FwdParams {
   const int* bf_index;     // flow field each pair reads as `bf` / `ff` (nullptr: its own)
   const int* ff_index;
   int pair_group;          // > 1: tiles of this many consecutive pairs are interleaved (window evaluations)
-  int cw_packed;           // host side only: launch the 8-consumer-warp variant (the tensor maps' boxes are sized for it)
+  int cw_packed;           // unused: a padding slot that keeps the offsets of the fields behind it
   int row_begin, row_end;  // rows of every pair this launch covers ([0, H) unless the frame is split into bands over several GPUs)
   void* warp_out;
   float* mask_out;

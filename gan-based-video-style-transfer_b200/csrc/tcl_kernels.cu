@@ -76,17 +76,8 @@
 #ifndef TCL_SCANNERS
 #define TCL_SCANNERS 2   // scanner warps (one warp needs about a tile period per tile and would pace the pipeline)
 #endif
-#ifndef TCL_PACKED
-#define TCL_PACKED 1  // interior staged tiles of the reducing hot configurations use packed fp32 arithmetic (lean_tile_packed)
-#endif
 #ifndef TCL_NS_MASK
 #define TCL_NS_MASK 3   // source-box stages of fbcCheckTorch on its own (two `ff` planes per stage)
-#endif
-#ifndef TCL_PACKED_MASK
-#define TCL_PACKED_MASK 1    // ... and for fbcCheckTorch on its own (mask_out only)
-#endif
-#ifndef TCL_PACKED_GIVEN
-#define TCL_PACKED_GIVEN 1   // ... also with a dataset mask (the training loss)
 #endif
 #ifndef TCL_DIAG
 #define TCL_DIAG 0    // tuning aids (tools/sweep_build.py): 1 = no source-box traffic, 3 = boxes at the tile's own position (no scan)
@@ -160,9 +151,18 @@ struct PairPtrs {
   FrameT* bout;
 };
 
+// Variants of the TMA kernel (its template parameter LEAN).  kVarGeneral reads every feature from FwdParams at run time;
+// the others fix a measured hot configuration at compile time (no validity mask, no near-threshold count) so the
+// per-pixel code carries no runtime feature checks.  Plain ints, not an enum: they are part of the kernels' mangled names.
+constexpr int kVarGeneral = 0;
+constexpr int kVarL2 = 1;        // both mask tests or a dataset mask, L2 error, no per-pixel outputs; also fbcCheckTorch on
+                                 // its own (CT == 0: mask_out only) and warp() on its own (MASK_NONE: warp_out only)
+constexpr int kVarL1 = 2;        // as kVarL2 with the L1 error
+constexpr int kVarMobOnly = 3;   // the mask alone with the motion-boundary test alone (fbcCheckTorch_mob)
+constexpr int kVarOutputs = 4;   // as kVarL2 plus the per-pixel outputs (warp_out / mask_out / blend_out, whichever are set)
+
 // everything that happens to one pixel once its taps and motion-boundary verdict are known.
-// LEAN fixes the hot configuration at compile time (both mask tests, L2 error, no optional outputs, no
-// near-threshold count) so the per-pixel code carries no runtime feature checks.
+// LEAN (any variant but kVarGeneral) fixes the hot configuration at compile time.
 // `cv` = this pixel's prefetched `cur` values (CT of them) or nullptr to load them here.
 template <typename FrameT, int MASK, bool REDUCE, int CT, int LEAN, typename FlowSrc, typename FrameSrc>
 __device__ __forceinline__ void finish_pixel(const FwdParams& p, const PixTaps& s, float u, float v, float nb, float keep,
@@ -188,7 +188,7 @@ __device__ __forceinline__ void finish_pixel(const FwdParams& p, const PixTaps& 
     if ((LEAN && MASK != MASK_NONE) || (!LEAN && io.cur)) {
       const float x = cv ? cv[c] : ld_stream(io.cur + (size_t)c * plane + o);
       if (REDUCE) {
-        if (LEAN == 1 || (!LEAN && p.loss == TCLB200_L2)) {   // LEAN: 1 = L2, 2 = L1 fixed at compile time
+        if (LEAN == kVarL2 || (!LEAN && p.loss == TCLB200_L2)) {
           const float md = __fmul_rn(keep, __fsub_rn(x, w));     // mask*(cur - warp)   sintel_eval.py:110
           err = __fmaf_rn(md, md, err);
         } else {
@@ -394,13 +394,11 @@ __device__ __forceinline__ unsigned long long gtime() { unsigned long long t; as
 #else
 #define TCL_STAMP(k, slot) do { } while (0)
 #endif
-// consumer warps per CTA: 8 (eight pixels per lane and tile) for the packed-arithmetic configuration, 16 (four pixels
-// per lane) for everything else -- measured per configuration (DESIGN.md); TCL_CWARPS forces one value (tuning builds)
-#ifdef TCL_CWARPS
-constexpr int kCWarpsPacked = TCL_CWARPS, kCWarpsOther = TCL_CWARPS;
-#else
-constexpr int kCWarpsPacked = 8, kCWarpsOther = 16;
-#endif
+// interior / edge / mixed staged tiles of these variants use packed fp32 arithmetic (lean_tile_packed): the reducing hot
+// configurations and fbcCheckTorch on its own
+__host__ __device__ constexpr bool uses_packed(int mask, bool reduce, int ct, int var) {
+  return ((var == kVarL2 || var == kVarL1) && ct == 3 && mask != MASK_NONE) || (var == kVarL2 && ct == 0 && mask == MASK_COMPUTED && !reduce);
+}
 
 // Lane -> pixel mapping of the consumer warps.  A warp owns a 16-column x kRows-row block of the 64 x TH tile (4 column
 // blocks x CW/4 row blocks); lane = 16 * h + c works on column c and on rows h, h + 2, h + 4, ... of the block.  One
@@ -1301,11 +1299,7 @@ __global__ void __launch_bounds__(Cfg::kThreads, 1) fused_forward_ws_kernel(cons
                                                                          const __grid_constant__ CUtensorMap tm_cur) {
   constexpr int NB = Cfg::NB, NS = Cfg::NS, P = Cfg::kPPL;
   constexpr int kCWarps = Cfg::CW;
-  constexpr int kLoss = LEAN == 2 ? TCLB200_L1 : TCLB200_L2;
-  // interior / edge / mixed staged tiles of the reducing hot configurations: packed fp32 arithmetic (lean_tile_packed)
-  // ... and fbcCheckTorch on its own (mask_out only)
-  constexpr bool kPacked = TCL_PACKED && (((LEAN == 1 || LEAN == 2) && CT == 3 && (MASK == MASK_COMPUTED || (MASK == MASK_GIVEN && TCL_PACKED_GIVEN))) ||
-                                          (TCL_PACKED_MASK && LEAN == 1 && CT == 0 && MASK == MASK_COMPUTED && !REDUCE));
+  constexpr int kLoss = LEAN == kVarL1 ? TCLB200_L1 : TCLB200_L2;
   using Ctl = WsCtl<NB, NS, kCWarps>;
   static_assert(sizeof(Ctl) <= Cfg::kCtlBytes, "control block too large");
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -1316,9 +1310,7 @@ __global__ void __launch_bounds__(Cfg::kThreads, 1) fused_forward_ws_kernel(cons
   auto prev_stage = [&](int s) { return reinterpret_cast<FrameT*>(smem + Cfg::kSrcOff + (size_t)s * Cfg::kSrcStage + Cfg::kFfStage); };
 
   const int total_tiles = p.B * p.tiles_per_pair;
-  // LEAN: 1 = both mask tests / L2, 2 = both mask tests / L1, 3 = mask-only with the motion-boundary test alone,
-  //       4 = as 1 plus the optional per-pixel outputs (warp_out / mask_out / blend_out, whichever are set)
-  const bool want_occ = MASK == MASK_COMPUTED && (LEAN ? LEAN != 3 : (p.flags & TCLB200_OCC) != 0);
+  const bool want_occ = MASK == MASK_COMPUTED && (LEAN ? LEAN != kVarMobOnly : (p.flags & TCLB200_OCC) != 0);
   const bool want_frames = CT > 0 && (LEAN || p.prev != nullptr);
   const bool want_scan = want_occ || want_frames;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -1543,21 +1535,21 @@ __global__ void __launch_bounds__(Cfg::kThreads, 1) fused_forward_ws_kernel(cons
 #else
     const int mode = ctl->meta[ss][2];
 #endif
-    if (LEAN == 3) {   // nothing staged, nothing sampled: the flow tile alone decides
+    if (LEAN == kVarMobOnly) {   // nothing staged, nothing sampled: the flow tile alone decides
       if (t_edge) lean_tile<FrameT, MASK, CT, TCLB200_L2, Cfg, true, false, false>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
       else lean_tile<FrameT, MASK, CT, TCLB200_L2, Cfg, false, false, false>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
     } else if (LEAN && mode == 1) {
-      if constexpr (kPacked) {
+      if constexpr (uses_packed(MASK, REDUCE, CT, LEAN)) {
         if (t_edge) err = lean_tile_packed<FrameT, MASK, kLoss, Cfg, true, false, CT>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
         else err = lean_tile_packed<FrameT, MASK, kLoss, Cfg, false, false, CT>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
       } else {
-        if (t_edge) err = lean_tile<FrameT, MASK, CT, kLoss, Cfg, true, false, true, LEAN == 4>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
-        else err = lean_tile<FrameT, MASK, CT, kLoss, Cfg, false, false, true, LEAN == 4>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
+        if (t_edge) err = lean_tile<FrameT, MASK, CT, kLoss, Cfg, true, false, true, LEAN == kVarOutputs>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
+        else err = lean_tile<FrameT, MASK, CT, kLoss, Cfg, false, false, true, LEAN == kVarOutputs>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
       }
-    } else if (LEAN == 4) {   // outputs wanted and the tile is mixed / unstaged: the feature-complete exact path
-      err = full_tile<FrameT, MASK, REDUCE, CT, 0, Cfg, true>(p, bf_stage(sb), ff_stage(ss), prev_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk, have_cur, near);
+    } else if (LEAN == kVarOutputs) {   // outputs wanted and the tile is mixed / unstaged: the feature-complete exact path
+      err = full_tile<FrameT, MASK, REDUCE, CT, kVarGeneral, Cfg, true>(p, bf_stage(sb), ff_stage(ss), prev_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk, have_cur, near);
     } else if (LEAN && mode == 2) {
-      if constexpr (kPacked) err = lean_tile_packed<FrameT, MASK, kLoss, Cfg, true, true, CT>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
+      if constexpr (uses_packed(MASK, REDUCE, CT, LEAN)) err = lean_tile_packed<FrameT, MASK, kLoss, Cfg, true, true, CT>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
       else err = lean_tile<FrameT, MASK, CT, kLoss, Cfg, true, true>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
     } else if (LEAN || t_edge) {
       err = full_tile<FrameT, MASK, REDUCE, CT, LEAN, Cfg, true>(p, bf_stage(sb), ff_stage(ss), prev_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk, have_cur, near);
@@ -1957,16 +1949,31 @@ extern "C" const char* tclb200_last_error(void) { return g_err; }
 #endif
 extern "C" const char* tclb200_build_info(void) {
   return "abi=" TCL_STR(TCLB200_ABI_VERSION) " th=" TCL_STR(TCL_TH) " bh=" TCL_STR(TCL_BH) "/" TCL_STR(TCL_BH8) " bw=" TCL_STR(TCL_BW) " bw16=" TCL_STR(TCL_BW16)
-         " ns=" TCL_STR(TCL_NS) "/" TCL_STR(TCL_NS_NOFF) " nb=" TCL_STR(TCL_NB) " cwarps=" TCL_CWARPS_S " scanners=" TCL_STR(TCL_SCANNERS) " packed=" TCL_STR(TCL_PACKED)
-         " packed_given=" TCL_STR(TCL_PACKED_GIVEN) " hot_only=" TCL_STR(TCL_HOT_ONLY_V) " diag=" TCL_STR(TCL_DIAG) " trace=" TCL_STR(TCL_TRACE_V);
+         " ns=" TCL_STR(TCL_NS) "/" TCL_STR(TCL_NS_NOFF) " nb=" TCL_STR(TCL_NB) " cwarps=" TCL_CWARPS_S " scanners=" TCL_STR(TCL_SCANNERS)
+         " hot_only=" TCL_STR(TCL_HOT_ONLY_V) " diag=" TCL_STR(TCL_DIAG) " trace=" TCL_STR(TCL_TRACE_V);
 }
 
 // tile shape of the TMA kernel: 64 x TH pixels per tile, 80 x BH source boxes: after rounding the box origin down
 // to a 16-byte boundary the taps may still spread >= 8 px in x and BH-TH-1 px in y beyond the tile's own extent
 // before the tile falls back to global gathers
 constexpr int kTW = 64, kTH = TCL_TH;
-constexpr int box_height(int cw, int esize) { return esize == 2 ? TCL_BH16 : (cw == 8 ? TCL_BH8 : TCL_BH); }
-template <typename FrameT> constexpr int box_width() { return sizeof(FrameT) == 4 ? TCL_BW : TCL_BW16; }
+
+// Geometry of one instantiation of the TMA kernel: consumer warps, source-box and flow-tile stages, source-box size, and
+// whether `ff` planes are staged.  WsCfg takes its template arguments from it and the plan sizes the tensor maps' boxes
+// from it, so the two cannot disagree.  `cw` is the consumer-warp count the plan asks for (8 or 16); TCL_CWARPS forces
+// one value for every configuration (tuning builds).
+struct WsGeo { int cw, ns, nb, bw, bh; bool ff; };
+constexpr WsGeo ws_geo(int esize, int mask, int ct, int var, int cw) {
+#ifdef TCL_CWARPS
+  cw = TCL_CWARPS;
+#endif
+  const bool ff = mask == MASK_COMPUTED;
+  const bool mask_only = ff && ct == 0 && var == kVarL2;   // fbcCheckTorch on its own: no frame planes, a third stage fits
+  const int ns = !ff ? TCL_NS_NOFF : mask_only ? TCL_NS_MASK : TCL_NS;
+  const int nb = !ff ? TCL_NS_NOFF + 2 : mask_only ? TCL_NS_MASK + 2 : TCL_NB;
+  const int bh = !ff ? TCL_BH_NOFF : esize == 2 ? TCL_BH16 : cw == 8 ? TCL_BH8 : TCL_BH;
+  return {cw, ns, nb, esize == 2 ? TCL_BW16 : TCL_BW, bh, ff};
+}
 
 static inline int cdiv(int a, int b) { return (a + b - 1) / b; }
 // scratch is sized for the finest tiling any kernel uses (32 x 8 generic tiles)
@@ -2019,52 +2026,6 @@ static int sm_count() {   // of the current device, cached per device index (a p
   return v;
 }
 
-static cudaError_t launch_fold(const FwdParams& p, cudaStream_t s);
-
-template <typename FrameT, int MASK, bool REDUCE, int CT, int LEAN, int CW>
-static cudaError_t launch_tma_cw(const FwdParams& p, const CUtensorMap& tb, const CUtensorMap& tf, const CUtensorMap& tp, const CUtensorMap& tc,
-                                 cudaStream_t s) {
-  constexpr bool has_ff = MASK == MASK_COMPUTED;
-  // (mask-only launches stage no frame planes: a third source stage fits beside the flow ring)
-  constexpr int NS = has_ff ? (CT == 0 && LEAN == 1 ? TCL_NS_MASK : TCL_NS) : TCL_NS_NOFF, NB = has_ff ? (CT == 0 && LEAN == 1 ? TCL_NS_MASK + 2 : TCL_NB) : TCL_NS_NOFF + 2;
-  using Cfg = WsCfg<FrameT, CT, kTW, kTH, box_width<FrameT>(), (has_ff ? box_height(CW, (int)sizeof(FrameT)) : TCL_BH_NOFF), NB, NS, CW, has_ff>;
-  auto kern = fused_forward_ws_kernel<FrameT, MASK, REDUCE, CT, LEAN, Cfg>;
-  static bool configured[64] = {};  // per instantiation and device (the attribute is a per-device property of the function)
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) dev = 63;   // (an uncached slot: set the attribute every time)
-  if (!configured[dev] || dev == 63) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmemBytes);
-    if (e != cudaSuccess) return e;
-    configured[dev] = true;
-  }
-  // persistent: one CTA per SM (or fewer when there are fewer tiles)
-  const size_t tiles = (size_t)p.B * p.tiles_per_pair;
-  const size_t slots = (size_t)sm_count();
-  const unsigned grid = (unsigned)(tiles < slots ? tiles : slots);
-  kern<<<grid, Cfg::kThreads, Cfg::kSmemBytes, s>>>(p, tb, tf, tp, tc);
-  ++g_launches;
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess || !REDUCE) return e;
-  return launch_fold(p, s);
-}
-
-// Consumer warps per CTA.  The packed-arithmetic configuration on fp32 frames (computeTCL: both mask tests, C == 3) runs
-// best with 8 warps x 8 pixels per lane on large frames (Sintel shape: 130 vs 124 Gpix/s); small frames, where a larger
-// share of the tiles straddles a motion boundary and waits for global gathers (256 x 256 training crops: 87 vs 97), bf16
-// frames (98 vs 123) and every other configuration run best with 16 warps x 4 pixels.
-template <typename FrameT, int MASK, bool REDUCE, int CT, int LEAN>
-static cudaError_t launch_tma(const FwdParams& p, const CUtensorMap& tb, const CUtensorMap& tf, const CUtensorMap& tp, const CUtensorMap& tc,
-                              cudaStream_t s) {
-  // (decided by run_fused, which sized the tensor maps' boxes for it: wants_packed8)
-  constexpr bool packed8 = TCL_PACKED && MASK == MASK_COMPUTED && sizeof(FrameT) == 4 &&
-                           (((LEAN == 1 || LEAN == 2) && CT == 3) || (TCL_PACKED_MASK && LEAN == 1 && CT == 0 && !REDUCE));
-  if constexpr (packed8 && kCWarpsPacked != kCWarpsOther) {
-    if (p.cw_packed) return launch_tma_cw<FrameT, MASK, REDUCE, CT, LEAN, kCWarpsPacked>(p, tb, tf, tp, tc, s);
-  }
-  if (p.cw_packed && kCWarpsPacked != kCWarpsOther) return cudaErrorInvalidConfiguration;   // (tensor maps sized for the other variant)
-  return launch_tma_cw<FrameT, MASK, REDUCE, CT, LEAN, kCWarpsOther>(p, tb, tf, tp, tc, s);
-}
-
 static cudaError_t launch_fold(const FwdParams& p, cudaStream_t s) {   // behind a kernel that stored one fp64 partial per tile
   ++g_launches;
   cudaLaunchConfig_t cfg;
@@ -2076,74 +2037,6 @@ static cudaError_t launch_fold(const FwdParams& p, cudaStream_t s) {   // behind
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr; cfg.numAttrs = 1;
   return small ? cudaLaunchKernelEx(&cfg, fold_partials_small_kernel, p) : cudaLaunchKernelEx(&cfg, fold_partials_kernel, p);
-}
-
-template <typename FrameT>
-static cudaError_t launch_direct(const FwdParams& p, cudaStream_t s) {
-  auto kern = p.loss == TCLB200_L1 ? fused_forward_direct_kernel<FrameT, TCLB200_L1> : fused_forward_direct_kernel<FrameT, TCLB200_L2>;
-  kern<<<(unsigned)((size_t)p.B * p.tiles_per_pair), kDirectThreads, 0, s>>>(p);
-  ++g_launches;
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return e;
-  return launch_fold(p, s);
-}
-
-template <typename FrameT, int MASK, bool REDUCE>
-static cudaError_t launch_generic(const FwdParams& p, cudaStream_t s) {
-  const unsigned grid = (unsigned)((size_t)p.B * p.tiles_per_pair);
-  if (p.C == 3) fused_forward_generic_kernel<FrameT, MASK, REDUCE, 3><<<grid, kThreads, 0, s>>>(p);
-  else fused_forward_generic_kernel<FrameT, MASK, REDUCE, 0><<<grid, kThreads, 0, s>>>(p);
-  ++g_launches;
-  return cudaGetLastError();
-}
-
-template <typename FrameT>
-static cudaError_t dispatch(const FwdParams& p, int mask_kind, bool reduce, bool tma, const CUtensorMap& tb, const CUtensorMap& tf,
-                            const CUtensorMap& tp, const CUtensorMap& tc, cudaStream_t s) {
-#ifdef TCL_HOT_ONLY   // tuning builds (tools/sweep_build.py): only the fp32 (1) or bf16 (2) computeTCL configuration, compiles in seconds
-  if (sizeof(FrameT) == (TCL_HOT_ONLY == 2 ? 2 : 4) && mask_kind == MASK_COMPUTED && reduce && tma && p.C == 3 && p.prev && p.cur && !p.warp_out && !p.mask_out &&
-      !p.blend_out && !p.near_threshold && p.loss == TCLB200_L2)
-    return launch_tma<typename std::conditional<TCL_HOT_ONLY == 2, __nv_bfloat16, float>::type, MASK_COMPUTED, true, 3, 1>(p, tb, tf, tp, tc, s);
-  if (mask_kind == MASK_COMPUTED && !reduce && !p.prev) return launch_generic<float, MASK_COMPUTED, false>(p, s);
-  return cudaErrorNotSupported;
-#else
-#define TCL_CASE(MK, RD)                                                                       \
-  if (mask_kind == MK && reduce == RD) {                                                       \
-    if (!tma) return launch_generic<FrameT, MK, RD>(p, s);                                     \
-    if (p.C == 3 && lean_out && MK != MASK_NONE) return launch_tma<FrameT, (MK == MASK_NONE ? MASK_GIVEN : MK), RD, 3, 4>(p, tb, tf, tp, tc, s); \
-    if (p.C == 3 && lean && RD) return p.loss == TCLB200_L1 ? launch_tma<FrameT, MK, true, 3, 2>(p, tb, tf, tp, tc, s)   \
-                                                            : launch_tma<FrameT, MK, true, 3, 1>(p, tb, tf, tp, tc, s);  \
-    if (MK == MASK_COMPUTED && !RD && lean_mask) return launch_tma<float, MASK_COMPUTED, false, 0, 1>(p, tb, tf, tp, tc, s); \
-    if (MK == MASK_COMPUTED && !RD && lean_mob) return launch_tma<float, MASK_COMPUTED, false, 0, 3>(p, tb, tf, tp, tc, s); \
-    if (MK == MASK_NONE && !RD && lean_warp) return launch_tma<FrameT, MASK_NONE, false, 3, 1>(p, tb, tf, tp, tc, s); \
-    return p.C == 3 ? launch_tma<FrameT, MK, RD, 3, 0>(p, tb, tf, tp, tc, s) : launch_tma<FrameT, MK, RD, 0, 0>(p, tb, tf, tp, tc, s); \
-  }
-  // LEAN = the measured hot configurations, fixed at compile time: computeTCL / training loss with C == 3
-  const bool lean = reduce && p.prev && p.cur && !p.warp_out && !p.mask_out && !p.blend_out && !p.near_threshold &&
-                    !(p.flags & TCLB200_VALIDITY) && mask_kind != MASK_NONE &&
-                    (mask_kind != MASK_COMPUTED || (p.flags & (TCLB200_OCC | TCLB200_MOB)) == (TCLB200_OCC | TCLB200_MOB));
-  // ... the same with per-pixel outputs (warp / mask / blend), with or without the reduction
-  const bool lean_out = p.prev && p.cur && (p.warp_out || p.blend_out || (p.mask_out && mask_kind == MASK_COMPUTED)) &&
-                        !(p.mask_out && mask_kind == MASK_GIVEN) && !p.near_threshold && !(p.flags & TCLB200_VALIDITY) &&
-                        p.loss == TCLB200_L2 && mask_kind != MASK_NONE &&
-                        (mask_kind != MASK_COMPUTED || (p.flags & (TCLB200_OCC | TCLB200_MOB)) == (TCLB200_OCC | TCLB200_MOB));
-  // ... and fbcCheckTorch on its own: both tests, mask_out only
-  const bool lean_mask = !reduce && !p.prev && p.mask_out && !p.near_threshold && mask_kind == MASK_COMPUTED &&
-                         (p.flags & (TCLB200_OCC | TCLB200_MOB)) == (TCLB200_OCC | TCLB200_MOB);
-  // ... and its optimisation-based variant: the motion-boundary test alone
-  const bool lean_mob = !reduce && !p.prev && p.mask_out && !p.near_threshold && mask_kind == MASK_COMPUTED &&
-                        (p.flags & (TCLB200_OCC | TCLB200_MOB)) == TCLB200_MOB;
-  // ... and warp() on its own (C == 3, no validity mask): warp_out only
-  const bool lean_warp = !reduce && p.prev && p.C == 3 && !p.cur && p.warp_out && !p.mask_out && !p.blend_out && mask_kind == MASK_NONE;
-  TCL_CASE(MASK_COMPUTED, true)
-  TCL_CASE(MASK_COMPUTED, false)
-  TCL_CASE(MASK_GIVEN, true)
-  TCL_CASE(MASK_GIVEN, false)
-  TCL_CASE(MASK_NONE, true)
-  TCL_CASE(MASK_NONE, false)
-#undef TCL_CASE
-  return cudaErrorInvalidValue;
-#endif
 }
 
 extern "C" int tclb200_debug_tile_stats(unsigned long long* out2, int reset) {
@@ -2176,6 +2069,190 @@ extern "C" void tclb200_debug_force_generic(int on) { g_force_generic = on; }
 #define TCL_DIRECT_MAX_PX (2u << 20)
 #endif
 
+// ---- forward plan --------------------------------------------------------------------------------
+// Which forward kernel a call runs, decided from its validated arguments alone (no CUDA calls): the path, the template
+// arguments of the instantiation, and for the TMA kernel its geometry (the boxes of the tensor maps) and consumer warps.
+enum : int { kPathGeneric = 0, kPathDirect = 1, kPathTma = 2 };
+struct FwdPlan {
+  int path;
+  int esize;               // frame type of the instantiation: 4 = fp32, 2 = bf16
+  int mask_kind;
+  bool reduce;
+  int ct, var, cw;         // CT; variant (kVar*; the direct kernel's loss); consumer warps (TMA kernel: 8 or 16, else 0)
+  WsGeo geo;               // TMA kernel: ws_geo(esize, mask_kind, ct, var, cw)
+  int tiles_x, tiles_per_pair;
+};
+
+// tma_ok: the flows' plane / pair strides are multiples of 16 bytes (false: the tensor maps did not encode)
+static FwdPlan plan_forward(const tclb200_tcl_args* a, bool tma_ok) {
+  FwdPlan q;
+  memset(&q, 0, sizeof(q));
+  q.esize = a->dtype == TCLB200_BF16 ? 2 : 4;
+  q.mask_kind = a->ff ? MASK_COMPUTED : (a->mask_in ? MASK_GIVEN : MASK_NONE);
+  q.reduce = a->cur && (a->pair_sums || a->total_sums || a->pair_vals || a->total_val);
+  q.ct = a->prev && a->C == 3 ? 3 : 0;
+  const int rows = a->row_begin != 0 || a->row_end != 0 ? a->row_end - a->row_begin : a->H;
+  // TMA needs 16-byte aligned bases and row strides; frames need C == 3 (the compiled box depth)
+  const bool tma = tma_ok && g_force_generic != 1 && (a->W % 4 == 0) && ((a->W * q.esize) % 16 == 0) && aligned16(a->bf) &&
+                   aligned16(a->ff) && aligned16(a->prev) && aligned16(a->cur) && (!a->prev || a->C == 3) && a->B <= 65535 * 16 &&
+                   a->H <= 16384 && a->W <= 16384;   // (box addresses are evaluated in fp32, see lean_tile)
+  // short launches of the training loss (dataset mask, reduction only): the direct kernel, no tensor maps needed
+  const bool direct = tma && g_force_generic != 2 && q.mask_kind == MASK_GIVEN && q.reduce && a->C == 3 && !a->warp_out && !a->mask_out &&
+                      !a->blend_out && !a->near_threshold && !(a->flags & (TCLB200_VALIDITY | TCLB200_THROUGHPUT)) && aligned16(a->mask_in) &&
+                      ((size_t)a->B * (size_t)rows * a->W <= TCL_DIRECT_MAX_PX || g_force_generic == 3);
+  if (!tma) {
+    q.path = kPathGeneric;
+    q.tiles_x = cdiv(a->W, 32);
+    q.tiles_per_pair = q.tiles_x * cdiv(rows, kWarps);
+    return q;
+  }
+  if (direct) {
+    q.path = kPathDirect;
+    q.var = a->loss == TCLB200_L1 ? kVarL1 : kVarL2;
+    q.tiles_per_pair = (int)(((size_t)rows * a->W + kDirectChunk - 1) / kDirectChunk);
+    return q;
+  }
+  q.path = kPathTma;
+  q.tiles_x = cdiv(a->W, kTW);
+  q.tiles_per_pair = q.tiles_x * cdiv(rows, kTH);
+  const int tests = a->flags & (TCLB200_OCC | TCLB200_MOB);
+  const bool outputs = a->warp_out || a->mask_out || a->blend_out;
+  // the measured hot configurations, fixed at compile time: computeTCL / the training loss (C == 3, both tests when the
+  // mask is computed, no validity mask, no near-threshold count) ...
+  const bool hot = a->prev && a->cur && q.mask_kind != MASK_NONE && (q.mask_kind != MASK_COMPUTED || tests == (TCLB200_OCC | TCLB200_MOB)) &&
+                   !a->near_threshold && !(a->flags & TCLB200_VALIDITY);
+  if (hot && q.reduce && !outputs) {
+    q.var = a->loss == TCLB200_L1 ? kVarL1 : kVarL2;
+  } else if (hot && outputs && a->loss == TCLB200_L2 && !(a->mask_out && q.mask_kind == MASK_GIVEN)) {
+    q.var = kVarOutputs;   // ... the same with per-pixel outputs, with or without the reduction
+  } else if (!a->prev && q.mask_kind == MASK_COMPUTED && !a->near_threshold &&
+             (tests == (TCLB200_OCC | TCLB200_MOB) || tests == TCLB200_MOB)) {
+    q.var = tests == TCLB200_MOB ? kVarMobOnly : kVarL2;   // ... fbcCheckTorch on its own (mask_out is set, no reduction)
+    q.esize = 4;                                           //     (it reads no frames)
+  } else if (q.mask_kind == MASK_NONE && a->prev && !a->cur && a->warp_out && !a->mask_out && !a->blend_out) {
+    q.var = kVarL2;        // ... and warp() on its own: warp_out only
+  } else {
+    q.var = kVarGeneral;
+  }
+  // Consumer warps per CTA.  The packed-arithmetic configurations with a computed mask on fp32 frames run best with
+  // 8 warps x 8 pixels per lane on large frames (Sintel shape: 130 vs 124 Gpix/s); small frames, where a larger share of
+  // the tiles straddles a motion boundary and waits for global gathers (256 x 256 training crops: 87 vs 97), bf16 frames
+  // (98 vs 123) and every other configuration run best with 16 warps x 4 pixels.
+  q.cw = uses_packed(q.mask_kind, q.reduce, q.ct, q.var) && q.mask_kind == MASK_COMPUTED && a->dtype == TCLB200_F32 &&
+                 (size_t)a->H * a->W >= (size_t)384 * 384 ? 8 : 16;
+  q.geo = ws_geo(q.esize, q.mask_kind, q.ct, q.var, q.cw);
+  return q;
+}
+
+// ---- launch table --------------------------------------------------------------------------------
+template <int PATH, typename FrameT, int MASK, bool REDUCE, int CT, int VAR, int CW>
+static cudaError_t launch_forward(const FwdParams& p, const CUtensorMap* tm, cudaStream_t s) {
+  const size_t tiles = (size_t)p.B * p.tiles_per_pair;
+  if constexpr (PATH == kPathGeneric) {
+    fused_forward_generic_kernel<FrameT, MASK, REDUCE, CT><<<(unsigned)tiles, kThreads, 0, s>>>(p);
+  } else if constexpr (PATH == kPathDirect) {
+    fused_forward_direct_kernel<FrameT, VAR == kVarL1 ? TCLB200_L1 : TCLB200_L2><<<(unsigned)tiles, kDirectThreads, 0, s>>>(p);
+  } else {
+    constexpr WsGeo G = ws_geo((int)sizeof(FrameT), MASK, CT, VAR, CW);
+    using Cfg = WsCfg<FrameT, CT, kTW, kTH, G.bw, G.bh, G.nb, G.ns, G.cw, G.ff>;
+    auto kern = fused_forward_ws_kernel<FrameT, MASK, REDUCE, CT, VAR, Cfg>;
+    static bool configured[64] = {};  // per instantiation and device (the attribute is a per-device property of the function)
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) dev = 63;   // (an uncached slot: set the attribute every time)
+    if (!configured[dev] || dev == 63) {
+      const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmemBytes);
+      if (e != cudaSuccess) return e;
+      configured[dev] = true;
+    }
+    // persistent: one CTA per SM (or fewer when there are fewer tiles)
+    const size_t slots = (size_t)sm_count();
+    kern<<<(unsigned)(tiles < slots ? tiles : slots), Cfg::kThreads, Cfg::kSmemBytes, s>>>(p, tm[0], tm[1], tm[2], tm[3]);
+  }
+  ++g_launches;
+  const cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess || !REDUCE || PATH == kPathGeneric) return e;   // (the generic kernel folds its own partials)
+  return launch_fold(p, s);
+}
+
+struct FwdRow {
+  int path, esize, mask;
+  bool reduce;
+  int ct, var, cw;
+  cudaError_t (*launch)(const FwdParams&, const CUtensorMap*, cudaStream_t);   // nullptr: not compiled into this build
+};
+
+// Tuning builds with TCL_HOT_ONLY (tools/sweep_build.py) compile computeTCL's rows alone, on fp32 (1) or bf16 (2) frames:
+// they build in seconds, and every other call finds no row.
+constexpr bool row_compiled(int path, int esize, int mask, bool reduce, int ct, int var) {
+#ifdef TCL_HOT_ONLY
+  return path == kPathTma && esize == (TCL_HOT_ONLY == 2 ? 2 : 4) && mask == MASK_COMPUTED && reduce && ct == 3 && var == kVarL2;
+#else
+  return true;
+#endif
+}
+
+template <int PATH, typename FrameT, int MASK, bool REDUCE, int CT, int VAR, int CW = 0>
+constexpr FwdRow row() {
+  constexpr int E = (int)sizeof(FrameT);
+  if constexpr (row_compiled(PATH, E, MASK, REDUCE, CT, VAR)) return {PATH, E, MASK, REDUCE, CT, VAR, CW, launch_forward<PATH, FrameT, MASK, REDUCE, CT, VAR, CW>};
+  else return {PATH, E, MASK, REDUCE, CT, VAR, CW, nullptr};
+}
+
+using bf16 = __nv_bfloat16;
+// Every forward kernel instantiation there is, each once: the only place that names one.  TMA rows with CT == 0 do not
+// reduce (a reduction needs `cur`, `cur` needs `prev`, and the TMA kernel needs C == 3 with `prev`), and the variants
+// fixed at compile time have the masks plan_forward gives them.
+static constexpr FwdRow kFwdRows[] = {
+    // generic kernel: shapes TMA cannot describe (CT == 0: any C, read at run time)
+    row<kPathGeneric, float, MASK_COMPUTED, true, 3, kVarGeneral>(),  row<kPathGeneric, float, MASK_COMPUTED, true, 0, kVarGeneral>(),
+    row<kPathGeneric, float, MASK_COMPUTED, false, 3, kVarGeneral>(), row<kPathGeneric, float, MASK_COMPUTED, false, 0, kVarGeneral>(),
+    row<kPathGeneric, float, MASK_GIVEN, true, 3, kVarGeneral>(),     row<kPathGeneric, float, MASK_GIVEN, true, 0, kVarGeneral>(),
+    row<kPathGeneric, float, MASK_GIVEN, false, 3, kVarGeneral>(),    row<kPathGeneric, float, MASK_GIVEN, false, 0, kVarGeneral>(),
+    row<kPathGeneric, float, MASK_NONE, true, 3, kVarGeneral>(),      row<kPathGeneric, float, MASK_NONE, true, 0, kVarGeneral>(),
+    row<kPathGeneric, float, MASK_NONE, false, 3, kVarGeneral>(),     row<kPathGeneric, float, MASK_NONE, false, 0, kVarGeneral>(),
+    row<kPathGeneric, bf16, MASK_COMPUTED, true, 3, kVarGeneral>(),   row<kPathGeneric, bf16, MASK_COMPUTED, true, 0, kVarGeneral>(),
+    row<kPathGeneric, bf16, MASK_COMPUTED, false, 3, kVarGeneral>(),  row<kPathGeneric, bf16, MASK_COMPUTED, false, 0, kVarGeneral>(),
+    row<kPathGeneric, bf16, MASK_GIVEN, true, 3, kVarGeneral>(),      row<kPathGeneric, bf16, MASK_GIVEN, true, 0, kVarGeneral>(),
+    row<kPathGeneric, bf16, MASK_GIVEN, false, 3, kVarGeneral>(),     row<kPathGeneric, bf16, MASK_GIVEN, false, 0, kVarGeneral>(),
+    row<kPathGeneric, bf16, MASK_NONE, true, 3, kVarGeneral>(),       row<kPathGeneric, bf16, MASK_NONE, true, 0, kVarGeneral>(),
+    row<kPathGeneric, bf16, MASK_NONE, false, 3, kVarGeneral>(),      row<kPathGeneric, bf16, MASK_NONE, false, 0, kVarGeneral>(),
+    // direct kernel: short launches of the training loss
+    row<kPathDirect, float, MASK_GIVEN, true, 3, kVarL2>(), row<kPathDirect, float, MASK_GIVEN, true, 3, kVarL1>(),
+    row<kPathDirect, bf16, MASK_GIVEN, true, 3, kVarL2>(),  row<kPathDirect, bf16, MASK_GIVEN, true, 3, kVarL1>(),
+    // TMA kernel, computed mask
+    row<kPathTma, float, MASK_COMPUTED, true, 3, kVarL2, 8>(),        row<kPathTma, float, MASK_COMPUTED, true, 3, kVarL2, 16>(),
+    row<kPathTma, float, MASK_COMPUTED, true, 3, kVarL1, 8>(),        row<kPathTma, float, MASK_COMPUTED, true, 3, kVarL1, 16>(),
+    row<kPathTma, float, MASK_COMPUTED, true, 3, kVarOutputs, 16>(),  row<kPathTma, float, MASK_COMPUTED, true, 3, kVarGeneral, 16>(),
+    row<kPathTma, float, MASK_COMPUTED, false, 3, kVarOutputs, 16>(), row<kPathTma, float, MASK_COMPUTED, false, 3, kVarGeneral, 16>(),
+    row<kPathTma, float, MASK_COMPUTED, false, 0, kVarL2, 8>(),       row<kPathTma, float, MASK_COMPUTED, false, 0, kVarL2, 16>(),
+    row<kPathTma, float, MASK_COMPUTED, false, 0, kVarMobOnly, 16>(), row<kPathTma, float, MASK_COMPUTED, false, 0, kVarGeneral, 16>(),
+    row<kPathTma, bf16, MASK_COMPUTED, true, 3, kVarL2, 16>(),        row<kPathTma, bf16, MASK_COMPUTED, true, 3, kVarL1, 16>(),
+    row<kPathTma, bf16, MASK_COMPUTED, true, 3, kVarOutputs, 16>(),   row<kPathTma, bf16, MASK_COMPUTED, true, 3, kVarGeneral, 16>(),
+    row<kPathTma, bf16, MASK_COMPUTED, false, 3, kVarOutputs, 16>(),  row<kPathTma, bf16, MASK_COMPUTED, false, 3, kVarGeneral, 16>(),
+    row<kPathTma, bf16, MASK_COMPUTED, false, 0, kVarGeneral, 16>(),
+    // TMA kernel, dataset mask
+    row<kPathTma, float, MASK_GIVEN, true, 3, kVarL2, 16>(),          row<kPathTma, float, MASK_GIVEN, true, 3, kVarL1, 16>(),
+    row<kPathTma, float, MASK_GIVEN, true, 3, kVarOutputs, 16>(),     row<kPathTma, float, MASK_GIVEN, true, 3, kVarGeneral, 16>(),
+    row<kPathTma, float, MASK_GIVEN, false, 3, kVarOutputs, 16>(),    row<kPathTma, float, MASK_GIVEN, false, 3, kVarGeneral, 16>(),
+    row<kPathTma, float, MASK_GIVEN, false, 0, kVarGeneral, 16>(),
+    row<kPathTma, bf16, MASK_GIVEN, true, 3, kVarL2, 16>(),           row<kPathTma, bf16, MASK_GIVEN, true, 3, kVarL1, 16>(),
+    row<kPathTma, bf16, MASK_GIVEN, true, 3, kVarOutputs, 16>(),      row<kPathTma, bf16, MASK_GIVEN, true, 3, kVarGeneral, 16>(),
+    row<kPathTma, bf16, MASK_GIVEN, false, 3, kVarOutputs, 16>(),     row<kPathTma, bf16, MASK_GIVEN, false, 3, kVarGeneral, 16>(),
+    row<kPathTma, bf16, MASK_GIVEN, false, 0, kVarGeneral, 16>(),
+    // TMA kernel, no mask
+    row<kPathTma, float, MASK_NONE, true, 3, kVarGeneral, 16>(),      row<kPathTma, float, MASK_NONE, false, 3, kVarGeneral, 16>(),
+    row<kPathTma, float, MASK_NONE, false, 3, kVarL2, 16>(),          row<kPathTma, float, MASK_NONE, false, 0, kVarGeneral, 16>(),
+    row<kPathTma, bf16, MASK_NONE, true, 3, kVarGeneral, 16>(),       row<kPathTma, bf16, MASK_NONE, false, 3, kVarGeneral, 16>(),
+    row<kPathTma, bf16, MASK_NONE, false, 3, kVarL2, 16>(),           row<kPathTma, bf16, MASK_NONE, false, 0, kVarGeneral, 16>(),
+};
+
+static const FwdRow* find_row(const FwdPlan& q) {
+  for (const FwdRow& r : kFwdRows)
+    if (r.path == q.path && r.esize == q.esize && r.mask == q.mask_kind && r.reduce == q.reduce && r.ct == q.ct && r.var == q.var && r.cw == q.cw)
+      return r.launch ? &r : nullptr;
+  return nullptr;
+}
+
 static int run_fused(const tclb200_tcl_args* a, cudaStream_t s) {
   if (!a) return fail(TCLB200_ERR_INVALID, "args is NULL");
   if (a->B <= 0 || a->H <= 0 || a->W <= 0) return fail(TCLB200_ERR_INVALID, "B, H, W must be positive");
@@ -2196,13 +2273,10 @@ static int run_fused(const tclb200_tcl_args* a, cudaStream_t s) {
     return fail(TCLB200_ERR_INVALID, "band mode needs 0 <= row_begin < row_end <= H");
   if (band && (a->pair_vals || a->total_val)) return fail(TCLB200_ERR_INVALID, "band mode returns sums only (pair_sums / total_sums): a band's mean is not the frame's");
   if ((size_t)a->H * a->W >= (1u << 30)) return fail(TCLB200_ERR_UNSUPPORTED, "H*W must be below 2^30");
-  const bool reduce = a->cur && (a->pair_sums || a->total_sums || a->pair_vals || a->total_val);
-  const int mask_kind = a->ff ? MASK_COMPUTED : (a->mask_in ? MASK_GIVEN : MASK_NONE);
-  if (mask_kind == MASK_COMPUTED && !(a->flags & (TCLB200_OCC | TCLB200_MOB)))
+  if (a->ff && !(a->flags & (TCLB200_OCC | TCLB200_MOB)))
     return fail(TCLB200_ERR_INVALID, "ff given but neither TCLB200_OCC nor TCLB200_MOB requested");
   if (!a->prev && !a->mask_out) return fail(TCLB200_ERR_INVALID, "nothing to compute: no frames and no mask_out");
 
-  const int esz = a->dtype == TCLB200_BF16 ? 2 : 4;
   // flows may be row-dense views with their own plane / pair strides (RAFT's padded output cropped by
   // InputPadder.unpad or flow_up[:,:,:H,:]); 0 = dense
   const size_t hw = (size_t)a->H * a->W;
@@ -2211,33 +2285,17 @@ static int run_fused(const tclb200_tcl_args* a, cudaStream_t s) {
   if (bf_plane < hw || ff_plane < hw || (a->B > 1 && (bf_batch < hw || ff_batch < hw)))
     return fail(TCLB200_ERR_INVALID, "flow plane / pair strides must be at least H*W");
   const bool strides16 = bf_plane % 4 == 0 && bf_batch % 4 == 0 && ff_plane % 4 == 0 && ff_batch % 4 == 0;   // TMA: 16-byte strides
-  // TMA needs 16-byte aligned bases and row strides; frames need C == 3 (the compiled box depth)
-  bool tma = g_force_generic != 1 && (a->W % 4 == 0) && ((a->W * esz) % 16 == 0) && aligned16(a->bf) && aligned16(a->ff) &&
-             aligned16(a->prev) && aligned16(a->cur) && (!a->prev || a->C == 3) && a->B <= 65535 * 16 && strides16 &&
-             a->H <= 16384 && a->W <= 16384;   // (box addresses are evaluated in fp32, see lean_tile)
-  // the packed-arithmetic configuration on large fp32 frames runs with 8 consumer warps and taller boxes (launch_tma): the
-  // same conditions as dispatch()'s `lean` for the computed-mask reductions
-  const bool cw_hot = reduce && a->prev && a->cur && a->C == 3 && !a->warp_out && !a->mask_out && !a->blend_out;
-  const bool cw_mask = TCL_PACKED_MASK && !reduce && !a->prev && a->mask_out;   // (dispatch()'s `lean_mask`: fbcCheckTorch on its own)
-  const bool cw_packed = TCL_PACKED && kCWarpsPacked != kCWarpsOther && tma && a->dtype == TCLB200_F32 && mask_kind == MASK_COMPUTED &&
-                         (cw_hot || cw_mask) && !a->near_threshold &&
-                         !(a->flags & TCLB200_VALIDITY) && (a->flags & (TCLB200_OCC | TCLB200_MOB)) == (TCLB200_OCC | TCLB200_MOB) &&
-                         (size_t)a->H * a->W >= (size_t)384 * 384;
-  // short launches of the training loss (dataset mask, reduction only): the direct kernel, no tensor maps needed
-  const size_t launch_px = (size_t)a->B * (size_t)((band ? a->row_end - a->row_begin : a->H)) * a->W;
-  const bool direct = tma && g_force_generic != 2 && mask_kind == MASK_GIVEN && reduce && a->C == 3 && !a->warp_out && !a->mask_out &&
-                      !a->blend_out && !a->near_threshold && !(a->flags & (TCLB200_VALIDITY | TCLB200_THROUGHPUT)) && aligned16(a->mask_in) &&
-                      (launch_px <= TCL_DIRECT_MAX_PX || g_force_generic == 3);
-  CUtensorMap tb, tf, tp, tc;
-  memset(&tb, 0, sizeof(tb)); memset(&tf, 0, sizeof(tf)); memset(&tp, 0, sizeof(tp)); memset(&tc, 0, sizeof(tc));
-  if (tma && !direct) {
-    const int bw = a->dtype == TCLB200_BF16 ? box_width<__nv_bfloat16>() : box_width<float>();
-    const int kBH = mask_kind == MASK_COMPUTED ? box_height(cw_packed ? kCWarpsPacked : kCWarpsOther, esz) : TCL_BH_NOFF;
-    tma = make_map(&tb, a->bf, 4, a->W, a->H, 2, a->bf_index ? a->n_bf_fields : a->B, kTW + 16, kTH + 2, 2, bf_plane, bf_batch);
-    if (tma && mask_kind == MASK_COMPUTED && (a->flags & TCLB200_OCC))
-      tma = make_map(&tf, a->ff, 4, a->W, a->H, 2, a->ff_index ? a->n_ff_fields : a->B, bw, kBH, 2, ff_plane, ff_batch);
-    if (tma && a->prev) tma = make_map(&tp, a->prev, esz, a->W, a->H, 3, a->prev_index ? a->n_prev_frames : a->B, bw, kBH, 3);
-    if (tma && a->prev && a->cur) tma = make_map(&tc, a->cur, esz, a->W, a->H, 3, a->cur_index ? a->n_cur_frames : a->B, kTW, kTH, 3);
+  FwdPlan plan = plan_forward(a, strides16);
+  CUtensorMap tm[4];   // bf, ff, prev, cur
+  memset(tm, 0, sizeof(tm));
+  if (plan.path == kPathTma) {
+    const WsGeo& g = plan.geo;
+    bool ok = make_map(&tm[0], a->bf, 4, a->W, a->H, 2, a->bf_index ? a->n_bf_fields : a->B, kTW + 16, kTH + 2, 2, bf_plane, bf_batch);
+    if (ok && plan.mask_kind == MASK_COMPUTED && (a->flags & TCLB200_OCC))
+      ok = make_map(&tm[1], a->ff, 4, a->W, a->H, 2, a->ff_index ? a->n_ff_fields : a->B, g.bw, g.bh, 2, ff_plane, ff_batch);
+    if (ok && a->prev) ok = make_map(&tm[2], a->prev, plan.esize, a->W, a->H, 3, a->prev_index ? a->n_prev_frames : a->B, g.bw, g.bh, 3);
+    if (ok && a->prev && a->cur) ok = make_map(&tm[3], a->cur, plan.esize, a->W, a->H, 3, a->cur_index ? a->n_cur_frames : a->B, kTW, kTH, 3);
+    if (!ok) plan = plan_forward(a, false);   // a tensor map that does not encode: the generic kernel
   }
 
   FwdParams p;
@@ -2247,7 +2305,6 @@ static int run_fused(const tclb200_tcl_args* a, cudaStream_t s) {
   p.prev_index = a->prev ? a->prev_index : nullptr; p.cur_index = a->cur ? a->cur_index : nullptr;
   p.bf_index = a->bf_index; p.ff_index = a->ff ? a->ff_index : nullptr;
   p.pair_group = a->pair_group > 1 ? a->pair_group : 1;
-  p.cw_packed = cw_packed ? 1 : 0;
   p.warp_out = a->warp_out; p.mask_out = a->mask_out; p.blend_out = a->blend_out;
   p.pair_sums = a->pair_sums; p.total_sums = a->total_sums; p.pair_vals = a->pair_vals; p.total_val = a->total_val;
   p.near_threshold = a->near_threshold;
@@ -2255,13 +2312,12 @@ static int run_fused(const tclb200_tcl_args* a, cudaStream_t s) {
   p.B = a->B; p.C = a->prev ? a->C : 0;
   p.row_begin = band ? a->row_begin : 0;
   p.row_end = band ? a->row_end : a->H;
-  p.tiles_x = tma ? cdiv(a->W, kTW) : cdiv(a->W, 32);
-  p.tiles_per_pair = p.tiles_x * (tma ? cdiv(p.row_end - p.row_begin, kTH) : cdiv(p.row_end - p.row_begin, kWarps));
-  if (direct) { p.tiles_x = 0; p.tiles_per_pair = (int)(((size_t)(p.row_end - p.row_begin) * a->W + kDirectChunk - 1) / kDirectChunk); }
+  p.tiles_x = plan.tiles_x;
+  p.tiles_per_pair = plan.tiles_per_pair;
   p.flags = a->flags; p.loss = a->loss; p.finalize = a->finalize;
   p.inv_count = a->prev ? 1.0 / ((double)a->C * a->H * a->W) : 0.0;
   if ((size_t)p.B * p.tiles_per_pair >= 0x7fffffffu) return fail(TCLB200_ERR_UNSUPPORTED, "too many tiles for one launch");
-  if (reduce) {
+  if (plan.reduce) {
     if (!a->scratch || a->scratch_bytes < tclb200_scratch_bytes(a->B, a->H, a->W))
       return fail(TCLB200_ERR_INVALID, "scratch missing or smaller than tclb200_scratch_bytes(B,H,W)");
     char* base = reinterpret_cast<char*>(a->scratch);
@@ -2271,16 +2327,13 @@ static int run_fused(const tclb200_tcl_args* a, cudaStream_t s) {
     p.scratch.batch_ticket = p.scratch.pair_ticket + a->B;
     // long launches of the TMA kernel hand out tiles through a counter (two words behind the tickets)
     const size_t tiles = (size_t)p.B * p.tiles_per_pair;
-    p.scratch.tile_ctr = (tma && !direct && tiles > 16 * (size_t)sm_count()) ? p.scratch.batch_ticket + 1 : nullptr;
+    p.scratch.tile_ctr = (plan.path == kPathTma && tiles > 16 * (size_t)sm_count()) ? p.scratch.batch_ticket + 1 : nullptr;
   }
-  if (direct) {
-    const cudaError_t e = a->dtype == TCLB200_BF16 ? launch_direct<__nv_bfloat16>(p, s) : launch_direct<float>(p, s);
-    if (e != cudaSuccess) return fail(TCLB200_ERR_CUDA, "fused forward (direct) launch: %s", cudaGetErrorString(e));
-    return TCLB200_OK;
-  }
-  const cudaError_t e = a->dtype == TCLB200_BF16 ? dispatch<__nv_bfloat16>(p, mask_kind, reduce, tma, tb, tf, tp, tc, s)
-                                                 : dispatch<float>(p, mask_kind, reduce, tma, tb, tf, tp, tc, s);
-  if (e != cudaSuccess) return fail(TCLB200_ERR_CUDA, "fused forward launch: %s", cudaGetErrorString(e));
+  const FwdRow* row = find_row(plan);
+  if (!row) return fail(TCLB200_ERR_UNSUPPORTED, "no forward kernel is compiled for this configuration (build: %s)", tclb200_build_info());
+  const cudaError_t e = row->launch(p, tm, s);
+  if (e != cudaSuccess)
+    return fail(TCLB200_ERR_CUDA, plan.path == kPathDirect ? "fused forward (direct) launch: %s" : "fused forward launch: %s", cudaGetErrorString(e));
   return TCLB200_OK;
 }
 

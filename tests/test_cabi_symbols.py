@@ -99,12 +99,13 @@ def test_host_entry_validation_without_gpu(tcl):
     assert b"workspace" in lib.tclb200_last_error()
 
 
-def test_build_info_names_the_configuration_and_tuning_builds_are_refused(tcl, monkeypatch):
+def test_build_info_names_the_tile_configuration_and_tuning_builds_are_refused(tcl, monkeypatch):
     info = tcl._cabi.lib().tclb200_build_info().decode()
     assert tcl._cabi._is_product_build(info), info
-    for key in ("abi=%d" % tcl._cabi.ABI_VERSION, "th=", "bh=", "bw=", "ns=", "nb=", "packed=", "hot_only=0", "diag=0", "trace=0"):
+    for key in ("abi=%d" % tcl._cabi.ABI_VERSION, "th=", "bh=", "bw=", "ns=", "nb=", "cwarps=", "hot_only=0", "diag=0", "trace=0"):
         assert key in info
     assert not tcl._cabi._is_product_build(info.replace("hot_only=0", "hot_only=1"))
+    assert not tcl._cabi._is_product_build(info.replace("diag=0", "diag=1"))
     assert not tcl._cabi._is_product_build(info.replace("abi=%d" % tcl._cabi.ABI_VERSION, "abi=4"))
     a = tcl._cabi.HostArgs()      # a clip without pairs is not an error (and needs no GPU)
     a.P, a.F = 0, 1

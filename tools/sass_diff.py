@@ -5,6 +5,8 @@ compared by their instruction text alone (opcode and operands; addresses and enc
 
   python tools/sass_diff.py OLD.so|.o NEW.so|.o [--match warp_backward_kernel]
       prints one line per matched kernel: identical / DIFFERENT (+ the first differing instruction); exit code 1 on any difference
+  python tools/sass_diff.py --exact OLD.so|.o NEW.so|.o [--match ""]
+      the same over every matched kernel, bf16 ones included, keyed by its full demangled name (no fp32 key folding)
   python tools/sass_diff.py --digest LIB [--match ...]
       prints a SHA-256 of each matched kernel's instruction text (what tests/test_bf16_backward_cpu.py pins)
 """
@@ -48,14 +50,18 @@ def main():
     ap.add_argument("new")
     ap.add_argument("--match", default="warp_backward_kernel")
     ap.add_argument("--digest", action="store_true")
+    ap.add_argument("--exact", action="store_true", help="key every kernel by its full demangled name")
     args = ap.parse_args()
     if args.digest:
         for name, instrs in sorted(kernels(args.new, args.match).items()):
             if "__nv_bfloat16" not in name:
                 print(f"{fp32_key(name)}  {len(instrs)}  {digest(instrs)}")
         return 0
-    old = {fp32_key(k): v for k, v in kernels(args.old, args.match).items()}
-    new = {fp32_key(k): v for k, v in kernels(args.new, args.match).items() if "__nv_bfloat16" not in k}
+    if args.exact:
+        old, new = kernels(args.old, args.match), kernels(args.new, args.match)
+    else:
+        old = {fp32_key(k): v for k, v in kernels(args.old, args.match).items()}
+        new = {fp32_key(k): v for k, v in kernels(args.new, args.match).items() if "__nv_bfloat16" not in k}
     bad = 0
     for key in sorted(set(old) | set(new)):
         if key not in old or key not in new:

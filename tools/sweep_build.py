@@ -14,8 +14,6 @@ VARIANTS = {
     "hot_s1": {"TCL_HOT_ONLY": 1, "TCL_CWARPS": 8, "TCL_SCANNERS": 1},
     "hot_s3": {"TCL_HOT_ONLY": 1, "TCL_CWARPS": 8, "TCL_SCANNERS": 3},
     "hot_w8": {"TCL_HOT_ONLY": 1, "TCL_CWARPS": 8},
-    "hot_w16_scalar": {"TCL_HOT_ONLY": 1, "TCL_CWARPS": 16, "TCL_PACKED": 0},
-    "hot_scalar": {"TCL_HOT_ONLY": 1, "TCL_PACKED": 0},
     "hot_bw76": {"TCL_HOT_ONLY": 1, "TCL_BW": 76},
     "hot_w16_bw76": {"TCL_HOT_ONLY": 1, "TCL_CWARPS": 16, "TCL_BW": 76},
     "hot_w12": {"TCL_HOT_ONLY": 1, "TCL_CWARPS": 12, "TCL_TH": 24, "TCL_BH": 32},
@@ -27,13 +25,10 @@ VARIANTS = {
     "w8_th16_ns3": {"TCL_HOT_ONLY": 1, "TCL_CWARPS": 8, "TCL_NS": 3, "TCL_NB": 5, "TCL_BH": 22, "TCL_BW": 76, "TCL_TH": 16},
     "w8_th16_ns4": {"TCL_HOT_ONLY": 1, "TCL_CWARPS": 8, "TCL_NS": 4, "TCL_NB": 6, "TCL_BH": 22, "TCL_BW": 76, "TCL_TH": 16},
     "w8_th16_ns2": {"TCL_HOT_ONLY": 1, "TCL_CWARPS": 8, "TCL_NS": 2, "TCL_NB": 4, "TCL_BH": 22, "TCL_BW": 76, "TCL_TH": 16},
-    "full_pg0": {"TCL_PACKED_GIVEN": 0},
     "full_w16": {"TCL_CWARPS": 16},
     "full_w8": {"TCL_CWARPS": 8},
     "hot_s1": {"TCL_HOT_ONLY": 1, "TCL_SCANNERS": 1},
-    "hot_sleep200": {"TCL_HOT_ONLY": 1, "TCL_IDLE_SLEEP_NS": 200},
     "hot_hint1000": {"TCL_HOT_ONLY": 1, "TCL_CONS_HINT_NS": 1000},
-    "hot_hint1000_sleep200": {"TCL_HOT_ONLY": 1, "TCL_CONS_HINT_NS": 1000, "TCL_IDLE_SLEEP_NS": 200},
     "hot_s3x": {"TCL_HOT_ONLY": 1, "TCL_SCANNERS": 3},
     "hot_s4x": {"TCL_HOT_ONLY": 1, "TCL_SCANNERS": 4},
     "hot_bh42": {"TCL_HOT_ONLY": 1, "TCL_BH": 42},
@@ -67,6 +62,7 @@ if __name__ == "__main__":
     for n, pr in procs:
         out = pr.communicate()[0]
         lines = out.splitlines()
-        hot = [i for i, l in enumerate(lines) if ("ws_kernelIfLi2ELb1ELi3ELb1" in l or "ws_kernelI13__nv_bfloat16Li2ELb1ELi3" in l) and "Compiling" in l]
+        # ptxas -v report of computeTCL's kernel: fused_forward_ws_kernel<float or bf16, MASK_COMPUTED, true, 3, kVarL2, ...>
+        hot = [i for i, l in enumerate(lines) if ("ws_kernelIfLi2ELb1ELi3ELi1E" in l or "ws_kernelI13__nv_bfloat16Li2ELb1ELi3ELi1E" in l) and "Compiling" in l]
         info = " | ".join(l.strip() for l in lines[hot[0] + 1:hot[0] + 4]) if hot else "?"
         print(n, "rc", pr.returncode, info[:230])
