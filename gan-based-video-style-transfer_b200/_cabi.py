@@ -12,10 +12,10 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 LIB_PATH = os.environ.get("TCL_B200_LIB") or os.path.join(CSRC, "libtcl_b200.so")  # env override: tuning sweeps only
 HEADER = os.path.join(os.path.dirname(_HERE), "include", "tcl_b200.h")
-ABI_VERSION = 6
+ABI_VERSION = 7
 
 # enums mirrored from include/tcl_b200.h
-F32, BF16 = 0, 1
+F32, BF16, U8 = 0, 1, 3
 OCC, MOB, VALIDITY = 1, 2, 4
 L2, L1 = 0, 1
 FIN_MEAN, FIN_RMSE = 0, 1
@@ -45,6 +45,7 @@ class TclArgs(ctypes.Structure):
         ("bf_index", ctypes.c_void_p), ("ff_index", ctypes.c_void_p),
         ("n_bf_fields", ctypes.c_int), ("n_ff_fields", ctypes.c_int), ("pair_group", ctypes.c_int),
         ("row_begin", ctypes.c_int), ("row_end", ctypes.c_int),
+        ("u8_scale", ctypes.c_float * 3), ("u8_offset", ctypes.c_float * 3),
     ]
 
 
@@ -58,6 +59,7 @@ class HostArgs(ctypes.Structure):
         ("P", ctypes.c_int), ("F", ctypes.c_int), ("C", ctypes.c_int), ("H", ctypes.c_int), ("W", ctypes.c_int),
         ("dtype", ctypes.c_int), ("flags", ctypes.c_int), ("loss", ctypes.c_int), ("finalize", ctypes.c_int),
         ("chunk_pairs", ctypes.c_int), ("frame_slots", ctypes.c_int),
+        ("u8_scale", ctypes.c_float * 3), ("u8_offset", ctypes.c_float * 3),
     ]
 
 

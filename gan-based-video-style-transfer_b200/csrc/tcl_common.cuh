@@ -31,6 +31,9 @@ __device__ __forceinline__ float ld_stream(const __nv_bfloat16* p) {
 // read-only gather through the non-coherent cache (bilinear taps that neighbouring lanes re-read)
 __device__ __forceinline__ float ld_gather(const float* p) { return __ldg(p); }
 __device__ __forceinline__ float ld_gather(const __nv_bfloat16* p) { return __bfloat162float(__ldg(p)); }
+// uint8 frames (TCLB200_U8): the raw byte as an exact fp32 integer; u8_value() then applies the normalisation
+__device__ __forceinline__ float ld_stream(const uint8_t* p) { return (float)__ldcs(reinterpret_cast<const unsigned char*>(p)); }
+__device__ __forceinline__ float ld_gather(const uint8_t* p) { return (float)__ldg(reinterpret_cast<const unsigned char*>(p)); }
 __device__ __forceinline__ void st_stream(float* p, float v) { __stcs(p, v); }
 __device__ __forceinline__ void st_stream(__nv_bfloat16* p, float v) {
   __stcs(reinterpret_cast<unsigned short*>(p), __bfloat16_as_ushort(__float2bfloat16_rn(v)));
@@ -72,6 +75,14 @@ struct Scratch {
   unsigned* tile_ctr;      // [2] tile counter / finished-CTA counter of the dynamic tile schedule (nullptr: static); zero between launches
 };
 
+// Normalisation of uint8 frames: v = u * scale[c] + offset[c], one rounded product and one rounded sum (torch's
+// u.float().mul(scale).add(offset)).  Scalar __fmul_rn / __fadd_rn on purpose: ptxas 12.9 contracts a packed
+// mul.rn.f32x2 + add.rn.f32x2 into one FFMA2 (one rounding instead of two, DESIGN.md section 4.1); it leaves these alone.
+struct FrameNorm {
+  float scale[3], offset[3];
+};
+__device__ __forceinline__ float u8_value(float u, const FrameNorm& n, int c) { return __fadd_rn(__fmul_rn(u, n.scale[c]), n.offset[c]); }
+
 struct FwdParams {
   const float* ff;
   const float* bf;
@@ -101,6 +112,16 @@ struct FwdParams {
   int flags, loss, finalize;
   double inv_count;  // 1/(C*H*W)
 };
+// the parameter block of the uint8-frame kernels: FwdParams followed by the normalisation (the kernels of the other frame
+// types keep FwdParams as it is, so their parameter offsets -- and instructions -- do not move).  Device code that holds
+// `const FwdParams&` reaches the normalisation through u8_norm() when FrameT is uint8_t.  That is sound because frame-type
+// code is only ever entered through the two kernel bodies (fused_forward_generic, fused_forward_ws), which take their
+// parameter type as a template argument and static_assert that uint8 frames come with FwdParamsU8 and no other frame type
+// does: a uint8 instantiation reached from a kernel that takes plain FwdParams does not compile.
+struct FwdParamsU8 : FwdParams {
+  FrameNorm norm;
+};
+__device__ __forceinline__ const FrameNorm& u8_norm(const FwdParams& p) { return static_cast<const FwdParamsU8&>(p).norm; }
 
 __device__ __forceinline__ float finalise_value(double mean, int finalize) {
   return (float)(finalize == TCLB200_FIN_RMSE ? sqrt(mean) : mean);

@@ -9,7 +9,7 @@
 //   copy streams    chunk k (on copy stream k % 2: two streams keep the link busy across the gaps between one stream's
 //                   copies -- with eight ranks sharing one host memory system those gaps are bandwidth nobody else can use):
 //                   the frames its pairs need that are not on the device yet (each frame crosses PCIe ONCE: 28 B/px per
-//                   pair instead of 40 for a clip), then the two flows of its pairs into ring slot k % 3
+//                   pair instead of 40 for a clip of fp32 frames; 19 with uint8 frames), then the two flows of its pairs into ring slot k % 3
 //   caller's stream chunk k: one fused launch (tclb200_tcl_forward in clip mode) on that slot, results into the
 //                   device result array; after the last chunk one D2H copy of the per-pair results
 //
@@ -26,6 +26,7 @@
 // events costs more than a small job).  On any failure the function drains both streams before it returns, so the
 // caller may free or reuse its host buffers as soon as it sees the error.
 #include <cuda_runtime.h>
+#include <math.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <string.h>
@@ -65,7 +66,7 @@ Layout make_layout(int P, int F, int C, int H, int W, int dtype, int chunk_pairs
     L.chunk = by_bytes < 1 ? 1 : (by_bytes > (size_t)kMaxDefaultChunk ? kMaxDefaultChunk : (int)by_bytes);
   }
   if (L.chunk > P) L.chunk = P;
-  L.frame_bytes = px * C * (dtype == TCLB200_BF16 ? 2 : 4);
+  L.frame_bytes = px * C * (dtype == TCLB200_U8 ? 1 : dtype == TCLB200_BF16 ? 2 : 4);
   L.flow_bytes = px * 2 * sizeof(float);
   L.mask_bytes = px * sizeof(float);
   size_t o = 0;
@@ -164,7 +165,12 @@ extern "C" int tclb200_tcl_forward_host(const tclb200_host_args* a, tclb200_stre
   if (a->F <= 0 || a->C <= 0 || a->H <= 0 || a->W <= 0) return hfail(TCLB200_ERR_INVALID, "F, C, H, W must be positive");
   if (!a->bf || !a->frames || !a->prev_index || !a->cur_index) return hfail(TCLB200_ERR_INVALID, "bf, frames, prev_index and cur_index are required");
   if (!a->pair_vals && !a->pair_sums) return hfail(TCLB200_ERR_INVALID, "nothing to return: pair_vals and pair_sums are both NULL");
-  if (a->dtype != TCLB200_F32 && a->dtype != TCLB200_BF16) return hfail(TCLB200_ERR_INVALID, "unknown dtype");
+  if (a->dtype != TCLB200_F32 && a->dtype != TCLB200_BF16 && a->dtype != TCLB200_U8) return hfail(TCLB200_ERR_INVALID, "unknown dtype");
+  if (a->dtype == TCLB200_U8) {   // (the fused launches check the same; here nothing has been enqueued yet)
+    if (a->C != 3) return hfail(TCLB200_ERR_INVALID, "uint8 frames must have C == 3");
+    for (int c = 0; c < 3; ++c)
+      if (!isfinite(a->u8_scale[c]) || !isfinite(a->u8_offset[c])) return hfail(TCLB200_ERR_INVALID, "uint8 frames: u8_scale / u8_offset must be finite");
+  }
   if (a->frame_slots < 0) return hfail(TCLB200_ERR_INVALID, "frame_slots must not be negative");
   for (int p = 0; p < a->P; ++p)
     if (a->prev_index[p] < 0 || a->prev_index[p] >= a->F || a->cur_index[p] < 0 || a->cur_index[p] >= a->F)
@@ -271,6 +277,7 @@ extern "C" int tclb200_tcl_forward_host(const tclb200_host_args* a, tclb200_stre
     t.scratch = ws + L.scratch; t.scratch_bytes = tclb200_scratch_bytes(L.chunk, a->H, a->W);
     t.B = n; t.C = a->C; t.H = a->H; t.W = a->W;
     t.dtype = a->dtype; t.flags = a->flags | TCLB200_THROUGHPUT; t.loss = a->loss; t.finalize = a->finalize;
+    memcpy(t.u8_scale, a->u8_scale, sizeof(t.u8_scale)); memcpy(t.u8_offset, a->u8_offset, sizeof(t.u8_offset));
     const int rc = tclb200_tcl_forward(&t, stream);
     if (rc != TCLB200_OK) return bail(rc);   // tclb200_last_error() already holds the message
     HOST_TRY(cudaEventRecord(pipe->done[slot], comp));

@@ -5,7 +5,7 @@
 // methods/learning-based/fs_lib.py:5-39, utils/sintel_eval.py:104-110, utils/metrics/eval.py:137-138,
 // methods/GAN-based/StarGANv2AdvCon/core/solver.py:427-446 of the upstream repository.
 //
-// Data layout in HBM: planar NCHW, fp32 flows/masks, fp32 or bf16 frames.
+// Data layout in HBM: planar NCHW, fp32 flows/masks, fp32 or bf16 frames (and uint8 frames for the evaluation's reductions).
 //
 // fused_forward_ws_kernel (the hot kernel, details at its definition): persistent, warp-specialised, one CTA per SM.
 //   producer warp    TMA pipeline: flow tiles of `bf` (+1 px halo, zero-filled outside the image = the zero padding of
@@ -23,6 +23,8 @@
 //   reduction        lane -> warp butterfly -> fp64 per tile (plain store) -> fold_partials_kernel (programmatic
 //                    dependent launch) sums tiles per pair, pairs per batch in index order: deterministic.
 // fused_forward_generic_kernel covers shapes TMA cannot describe (W % 4 != 0, unaligned views, C != 3).
+// uint8 frames (evaluation only): fused_forward_ws_u8_kernel / fused_forward_generic_u8_kernel are the same two kernels with
+// the frames normalised per channel as they are loaded (W % 16 == 0 for the TMA one: uint8 box rows are multiples of 16 bytes).
 // warp_backward_kernel: autograd of warp / fused backward of the training loss.  gradient_kernel.  hwc_split_kernel
 // (dataset ingest) and upsample_flow_kernel (RAFT's convex upsampling) are the steps either side of the path.
 // HBM-bound fp32 streaming + gather: no tensor cores, nothing here is a contraction.
@@ -30,6 +32,7 @@
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <limits.h>
+#include <math.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <string.h>
@@ -128,6 +131,36 @@ struct GlobalSrc {
   }
 };
 
+// uint8 frames: each tap inside the image is normalised (u8_value) before it is weighted; a tap outside contributes 0, as
+// grid_sample's zero padding of the normalised frame does -- not the normalisation's offset
+template <>
+struct GlobalSrc<uint8_t> {
+  const uint8_t* base;
+  size_t plane;
+  Geo g;
+  FrameNorm n;
+  __device__ __forceinline__ float sample(int c, const PixTaps& s) const {
+    const Taps t = full_taps(s, g);
+    const uint8_t* q = base + (size_t)c * plane + t.o00;
+    const float v00 = t.p00 ? u8_value(ld_gather(q), n, c) : 0.0f;
+    const float v10 = t.p10 ? u8_value(ld_gather(q + 1), n, c) : 0.0f;
+    const float v01 = t.p01 ? u8_value(ld_gather(q + g.W), n, c) : 0.0f;
+    const float v11 = t.p11 ? u8_value(ld_gather(q + g.W + 1), n, c) : 0.0f;
+    return combine(v00, v10, v01, v11, t, kV);
+  }
+};
+template <typename FrameT>
+__device__ __forceinline__ GlobalSrc<FrameT> frame_src(const FwdParams& p, const FrameT* base, size_t plane) {
+  if constexpr (std::is_same<FrameT, uint8_t>::value) return GlobalSrc<FrameT>{base, plane, p.geo, u8_norm(p)};
+  else return GlobalSrc<FrameT>{base, plane, p.geo};
+}
+// a value of `cur` as loaded (ld_stream) -> the value the error uses: uint8 frames are normalised, the others are as they are
+template <typename FrameT>
+__device__ __forceinline__ float frame_value(const FwdParams& p, float raw, int c) {
+  if constexpr (std::is_same<FrameT, uint8_t>::value) return u8_value(raw, u8_norm(p), c);
+  else return raw;
+}
+
 // source box in shared memory, origin (ox,oy), zero-filled outside the image: all four taps are plain reads.
 // fma(0, w, acc) == acc for the finite weights of an in-box pixel, so this equals the predicated form.
 template <typename T, int PITCH, int CH_STRIDE>
@@ -143,6 +176,30 @@ struct SmemSrc {
     return acc;
   }
 };
+
+// uint8 frames: normalised per tap; a tap outside the image contributes 0 (the box holds byte 0 there, i.e. the offset)
+template <int PITCH, int CH_STRIDE>
+struct SmemSrc<uint8_t, PITCH, CH_STRIDE> {
+  const uint8_t* base;
+  int ox, oy;
+  int W, H;
+  FrameNorm n;
+  __device__ __forceinline__ float sample(int c, const PixTaps& s) const {
+    const uint8_t* q = base + c * CH_STRIDE + (s.y0 - oy) * PITCH + (s.x0 - ox);
+    const bool xin0 = (unsigned)s.x0 < (unsigned)W, xin1 = (unsigned)(s.x0 + 1) < (unsigned)W;
+    const bool yin0 = (unsigned)s.y0 < (unsigned)H, yin1 = (unsigned)(s.y0 + 1) < (unsigned)H;
+    float acc = __fmul_rn(xin0 && yin0 ? u8_value((float)q[0], n, c) : 0.0f, s.nw);
+    acc = __fmaf_rn(xin1 && yin0 ? u8_value((float)q[1], n, c) : 0.0f, s.ne, acc);
+    acc = __fmaf_rn(xin0 && yin1 ? u8_value((float)q[PITCH], n, c) : 0.0f, s.sw, acc);
+    acc = __fmaf_rn(xin1 && yin1 ? u8_value((float)q[PITCH + 1], n, c) : 0.0f, s.se, acc);
+    return acc;
+  }
+};
+template <typename FrameT, int PITCH, int CH_STRIDE>
+__device__ __forceinline__ SmemSrc<FrameT, PITCH, CH_STRIDE> smem_src(const FwdParams& p, const FrameT* base, int ox, int oy) {
+  if constexpr (std::is_same<FrameT, uint8_t>::value) return SmemSrc<FrameT, PITCH, CH_STRIDE>{base, ox, oy, p.geo.W, p.geo.H, u8_norm(p)};
+  else return SmemSrc<FrameT, PITCH, CH_STRIDE>{base, ox, oy};
+}
 
 template <typename FrameT>
 struct PairPtrs {
@@ -180,13 +237,15 @@ __device__ __forceinline__ void finish_pixel(const FwdParams& p, const PixTaps& 
   float valid = 1.0f;
   if (validity) valid = binarise_validity(ones_sample(full_taps(s, p.geo), kV));
   const int C = CT > 0 ? CT : p.C;
+  constexpr bool kOuts = !std::is_same<FrameT, uint8_t>::value;   // (uint8 frames are scored, never written: no warp_out / blend_out)
 #pragma unroll
   for (int c = 0; c < C; ++c) {
     float w = psrc.sample(c, s);
     if (validity) w = __fmul_rn(w, valid);
-    if ((!LEAN || MASK == MASK_NONE) && io.wout) st_stream(io.wout + (size_t)c * plane + o, w);   // (LEAN + MASK_NONE = warp only)
+    if constexpr (kOuts)
+      if ((!LEAN || MASK == MASK_NONE) && io.wout) st_stream(io.wout + (size_t)c * plane + o, w);   // (LEAN + MASK_NONE = warp only)
     if ((LEAN && MASK != MASK_NONE) || (!LEAN && io.cur)) {
-      const float x = cv ? cv[c] : ld_stream(io.cur + (size_t)c * plane + o);
+      const float x = cv ? cv[c] : frame_value<FrameT>(p, ld_stream(io.cur + (size_t)c * plane + o), c);
       if (REDUCE) {
         if (LEAN == kVarL2 || (!LEAN && p.loss == TCLB200_L2)) {
           const float md = __fmul_rn(keep, __fsub_rn(x, w));     // mask*(cur - warp)   sintel_eval.py:110
@@ -195,8 +254,9 @@ __device__ __forceinline__ void finish_pixel(const FwdParams& p, const PixTaps& 
           err += __fmul_rn(keep, fabsf(__fsub_rn(w, x)));        // mask*|warp - cur|   MoGAN cycle_gan_model.py:281
         }
       }
-      if (!LEAN && io.bout)                                      // m*warp + (1-m)*img   obst_eval.py:500
-        st_stream(io.bout + (size_t)c * plane + o, __fadd_rn(__fmul_rn(keep, w), __fmul_rn(__fsub_rn(1.0f, keep), x)));
+      if constexpr (kOuts)
+        if (!LEAN && io.bout)                                    // m*warp + (1-m)*img   obst_eval.py:500
+          st_stream(io.bout + (size_t)c * plane + o, __fadd_rn(__fmul_rn(keep, w), __fmul_rn(__fsub_rn(1.0f, keep), x)));
     }
   }
 }
@@ -222,8 +282,10 @@ __device__ __forceinline__ PairPtrs<FrameT> pair_ptrs(const FwdParams& p, int pa
 // ---------------------------------------------------------------------------------------------
 // generic forward kernel: one pixel per lane, everything straight from global memory
 // ---------------------------------------------------------------------------------------------
-template <typename FrameT, int MASK, bool REDUCE, int CT>
-__global__ void __launch_bounds__(kThreads) fused_forward_generic_kernel(const FwdParams p) {
+template <typename FrameT, int MASK, bool REDUCE, int CT, typename Params>
+__device__ __forceinline__ void fused_forward_generic(const Params& p) {
+  static_assert(std::is_same<FrameT, uint8_t>::value == std::is_same<Params, FwdParamsU8>::value,
+                "uint8 frames come with their normalisation (FwdParamsU8), the other frame types without it");
   const Geo& g = p.geo;
   const int W = g.W, H = g.H;
   const size_t plane = (size_t)H * W;
@@ -254,12 +316,21 @@ __global__ void __launch_bounds__(kThreads) fused_forward_generic_kernel(const F
     }
     const PixTaps s = pix_taps(u, v, x, y, g);
     GlobalSrc<float> fsrc{p.ff ? p.ff + (size_t)ff_field(p, pair) * p.ff_batch : nullptr, p.ff_plane, g};
-    GlobalSrc<FrameT> psrc{p.prev ? reinterpret_cast<const FrameT*>(p.prev) + (size_t)prev_frame(p, pair) * C * plane : nullptr, plane, g};
+    const GlobalSrc<FrameT> psrc = frame_src<FrameT>(p, p.prev ? reinterpret_cast<const FrameT*>(p.prev) + (size_t)prev_frame(p, pair) * C * plane : nullptr, plane);
     finish_pixel<FrameT, MASK, REDUCE, CT, false>(p, s, u, v, nb, keep, o, plane, pair, fsrc, psrc,
                                                   pair_ptrs<FrameT>(p, pair, cur_frame(p, pair), C, plane), nullptr, err, near);
   }
   count_near(near, p.near_threshold);
   if (REDUCE) reduce_and_finalise(err, p, pair, tile);
+}
+template <typename FrameT, int MASK, bool REDUCE, int CT>
+__global__ void __launch_bounds__(kThreads) fused_forward_generic_kernel(const FwdParams p) {
+  fused_forward_generic<FrameT, MASK, REDUCE, CT>(p);
+}
+// uint8 frames (C == 3, reductions only): the same kernel with the normalisation behind the parameters
+template <int MASK>
+__global__ void __launch_bounds__(kThreads) fused_forward_generic_u8_kernel(const FwdParamsU8 p) {
+  fused_forward_generic<uint8_t, MASK, true, 3>(p);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -671,9 +742,9 @@ __device__ __forceinline__ float full_tile(const FwdParams& p, const float* s_bu
   const PairPtrs<FrameT> io = pair_ptrs<FrameT>(p, t.pair, t.cf, CT > 0 ? CT : p.C, plane);
   const int ox = meta[0], oy = meta[1], mode = meta[2];   // mode 0: nothing staged, 1: every tap in the boxes, 2: mixed
   const SmemSrc<float, Cfg::BW, Cfg::BH * Cfg::BW> fs{s_ff, ox, oy};
-  const SmemSrc<FrameT, Cfg::BW, Cfg::BH * Cfg::BW> ps{s_prev, ox, oy};
+  const SmemSrc<FrameT, Cfg::BW, Cfg::BH * Cfg::BW> ps = smem_src<FrameT, Cfg::BW, Cfg::BH * Cfg::BW>(p, s_prev, ox, oy);
   const GlobalSrc<float> fg{p.ff ? p.ff + (size_t)t.ffi * p.ff_batch : nullptr, p.ff_plane, g};
-  const GlobalSrc<FrameT> pg{p.prev ? reinterpret_cast<const FrameT*>(p.prev) + (size_t)t.pf * (CT > 0 ? CT : p.C) * plane : nullptr, plane, g};
+  const GlobalSrc<FrameT> pg = frame_src<FrameT>(p, p.prev ? reinterpret_cast<const FrameT*>(p.prev) + (size_t)t.pf * (CT > 0 ? CT : p.C) * plane : nullptr, plane);
   float err = 0.0f;
 #pragma unroll
   for (int k = 0; k < Cfg::kPPL; ++k) {   // fully unrolled: cur[k] / mk[k] must stay in registers
@@ -806,6 +877,23 @@ __device__ __forceinline__ float lds_tap(uint32_t a, __nv_bfloat16) {
   asm volatile("ld.shared.u16 %0, [%1+%2];" : "=r"(h) : "r"(a), "n"(OFF));
   return __uint_as_float(h << 16);
 }
+template <int OFF>
+__device__ __forceinline__ float lds_tap(uint32_t a, uint8_t) {
+  unsigned h;   // (zero-extended into the 32-bit register)
+  asm volatile("ld.shared.u8 %0, [%1+%2];" : "=r"(h) : "r"(a), "n"(OFF));
+  return (float)h;
+}
+// uint8 frames: one plane of a staged box, normalised per tap; taps outside the image (q.. false: only on tiles whose box
+// crosses the border) contribute 0 -- the box holds byte 0 there, which would normalise to the offset
+template <int OFF, int PITCH>
+__device__ __forceinline__ float staged_tap4_u8(uint32_t a, const LeanTaps& tp, const FrameNorm& n, int c, bool q00, bool q10, bool q01,
+                                                bool q11) {
+  float w = __fmul_rn(q00 ? u8_value(lds_tap<OFF>(a, uint8_t()), n, c) : 0.0f, tp.nw);
+  w = __fmaf_rn(q10 ? u8_value(lds_tap<OFF + 1>(a, uint8_t()), n, c) : 0.0f, tp.ne, w);
+  w = __fmaf_rn(q01 ? u8_value(lds_tap<OFF + PITCH>(a, uint8_t()), n, c) : 0.0f, tp.sw, w);
+  w = __fmaf_rn(q11 ? u8_value(lds_tap<OFF + PITCH + 1>(a, uint8_t()), n, c) : 0.0f, tp.se, w);
+  return w;
+}
 // one plane of a staged box, grid_sampler_2d's accumulation order (zero-filled outside the image: all four taps are plain reads)
 template <typename T, int OFF, int PITCH>
 __device__ __forceinline__ float staged_tap4(uint32_t a, const LeanTaps& tp) {
@@ -845,6 +933,8 @@ __device__ __forceinline__ float lean_tile(const FwdParams& p, const float* s_bu
   const int c0 = (ly0 + 1) * BFW + lx0 + Cfg::kHaloL;
   const bool xin = !EDGE || t.x0 + lx0 < g.W;
   const bool validity = MASK == MASK_NONE && (p.flags & TCLB200_VALIDITY);
+  // uint8 frames: does this tile's source box cross the image border (then its staged taps need in-image predicates)?
+  const bool box_border = FE == 1 && (box_x < 0 || box_y < 0 || box_x + BW > g.W || box_y + Cfg::BH > g.H);
   // staged tiles: byte address of a pixel's top-left tap = base + 4 * ((fyf - box_y) * BW + (fxf - box_x)), evaluated with two
   // fmas on exact small integers (the placement keeps |box| < 2^15, so every intermediate is an integer below 2^24)
   const uint32_t ff_base = smem_u32(s_ff), prev_base = smem_u32(s_prev);
@@ -907,7 +997,23 @@ __device__ __forceinline__ float lean_tile(const FwdParams& p, const float* s_bu
           a = staged_tap4<float, 0, BW>(fa, tp);
           b = staged_tap4<float, PL * 4, BW>(fa, tp);
         }
-        if (CT == 3) {
+        if constexpr (FE == 1) {
+          if (CT == 3) {
+            uint32_t pa = (uint32_t)__float2int_rn(__fmaf_rn(tp.fyf, (float)BW, __fmaf_rn(tp.fxf, 1.0f, prev_k)));
+            if (EDGE && !inside) pa = prev_base;
+            bool q00 = true, q10 = true, q01 = true, q11 = true;
+            if (box_border) {   // (exact small integers: the placement keeps the box within |2^15|)
+              const int gx = (int)tp.fxf, gy = (int)tp.fyf;
+              const bool xin0 = (unsigned)gx < (unsigned)g.W, xin1 = (unsigned)(gx + 1) < (unsigned)g.W;
+              const bool yin0 = (unsigned)gy < (unsigned)g.H, yin1 = (unsigned)(gy + 1) < (unsigned)g.H;
+              q00 = xin0 && yin0; q10 = xin1 && yin0; q01 = xin0 && yin1; q11 = xin1 && yin1;
+            }
+            const FrameNorm& nrm = u8_norm(p);
+            w3[0] = staged_tap4_u8<0, BW>(pa, tp, nrm, 0, q00, q10, q01, q11);
+            w3[1] = staged_tap4_u8<PL, BW>(pa, tp, nrm, 1, q00, q10, q01, q11);
+            w3[2] = staged_tap4_u8<2 * PL, BW>(pa, tp, nrm, 2, q00, q10, q01, q11);
+          }
+        } else if (CT == 3) {
           if (FE == 4) {   // fp32 frames: the prev planes sit behind the ff planes, the same address register serves them
             w3[0] = staged_tap4<FrameT, (int)Cfg::kFfStage, BW>(fa, tp);
             w3[1] = staged_tap4<FrameT, (int)Cfg::kFfStage + PL * FE, BW>(fa, tp);
@@ -947,8 +1053,26 @@ __device__ __forceinline__ float lean_tile(const FwdParams& p, const float* s_bu
           return w;
         };
         if (MASK == MASK_COMPUTED && OCC) { a = tap4(pf); b = tap4(pf + psf); }
+        if constexpr (FE == 1) {
+          // uint8 frames: in-image predicates for the staged taps too (the box's fill is byte 0), then the normalisation
+          const int gx = (int)tp.fxf, gy = (int)tp.fyf;
+          const bool xin0 = (unsigned)gx < (unsigned)g.W, xin1 = (unsigned)(gx + 1) < (unsigned)g.W;
+          const bool yin0 = (unsigned)gy < (unsigned)g.H, yin1 = (unsigned)(gy + 1) < (unsigned)g.H;
+          const bool r00 = xin0 && yin0, r10 = xin1 && yin0, r01 = xin0 && yin1, r11 = xin1 && yin1;
+          const FrameNorm& nrm = u8_norm(p);
 #pragma unroll
-        for (int ch = 0; ch < CT; ++ch) w3[ch] = tap4(pp + ch * ps);
+          for (int ch = 0; ch < CT; ++ch) {
+            const FrameT* bp = pp + ch * ps;
+            float w = __fmul_rn(r00 ? u8_value((float)bp[0], nrm, ch) : 0.0f, tp.nw);
+            w = __fmaf_rn(r10 ? u8_value((float)bp[1], nrm, ch) : 0.0f, tp.ne, w);
+            w = __fmaf_rn(r01 ? u8_value((float)bp[rs], nrm, ch) : 0.0f, tp.sw, w);
+            w = __fmaf_rn(r11 ? u8_value((float)bp[rs + 1], nrm, ch) : 0.0f, tp.se, w);
+            w3[ch] = w;
+          }
+        } else {
+#pragma unroll
+          for (int ch = 0; ch < CT; ++ch) w3[ch] = tap4(pp + ch * ps);
+        }
       }
       if (MASK == MASK_COMPUTED && OCC) {
         // occlusion: |wf+bf|^2  vs  0.01*(|wf|^2+|bf|^2) + 0.5
@@ -975,8 +1099,9 @@ __device__ __forceinline__ float lean_tile(const FwdParams& p, const float* s_bu
       for (int ch = 0; ch < CT; ++ch) {
         const float w = w3[ch];
         if (MASK == MASK_NONE) {   // warp() on its own: store the warped frame (two coalesced row segments per warp instruction)
-          if (inside)
-            st_stream(reinterpret_cast<FrameT*>(p.warp_out) + ((size_t)t.pair * 3 + ch) * gplane + (size_t)(t.y0 + ly0 + dyk) * g.W + (t.x0 + lx0),
+          if constexpr (FE != 1)
+            if (inside)
+              st_stream(reinterpret_cast<FrameT*>(p.warp_out) + ((size_t)t.pair * 3 + ch) * gplane + (size_t)(t.y0 + ly0 + dyk) * g.W + (t.x0 + lx0),
                       validity ? __fmul_rn(w, valid) : w);
           continue;
         }
@@ -1006,12 +1131,13 @@ __device__ __forceinline__ float lean_tile(const FwdParams& p, const float* s_bu
 #pragma unroll
     for (int k = 0; k < P; ++k)
       if ((outbits >> k) & 1u) {
-        if (CT == 3) {
+        if constexpr (CT == 3 && FE != 1) {
           e[k] = pixel_global<FrameT, MASK, false, LOSS>(p.bf + (size_t)t.bfi * p.bf_batch, p.bf_plane, p.ff + (size_t)t.ffi * p.ff_batch, p.ff_plane,
                                                    reinterpret_cast<const FrameT*>(p.prev) + (size_t)t.pf * 3 * plane, g, t.x0 + lx0,
                                                    t.y0 + ly0 + pix_dy(k), cur[k][0], cur[k][1], cur[k][2], mk[k]);
           keepbits |= 1u << k;   // the verdict is already applied
-        } else {
+        } else {   // (mask-only; and uint8 frames: the loop's error is exact already -- the taps came from global memory with the
+                   // predicates -- only the verdict that was too close to call is redone)
           const float kp = pixel_global<FrameT, MASK, true, LOSS>(p.bf + (size_t)t.bfi * p.bf_batch, p.bf_plane, p.ff + (size_t)t.ffi * p.ff_batch, p.ff_plane, nullptr, g,
                                                             t.x0 + lx0, t.y0 + ly0 + pix_dy(k), 0.0f, 0.0f, 0.0f, 0.0f);
           keepbits = (keepbits & ~(1u << k)) | ((kp != 0.0f ? 1u : 0u) << k);
@@ -1032,9 +1158,11 @@ __device__ __forceinline__ float lean_tile(const FwdParams& p, const float* s_bu
       if (mo) __stcs(mo + off, keepf);
 #pragma unroll
       for (int ch = 0; ch < 3; ++ch) {
-        if (wo) st_stream(wo + ch * gplane + off, wv[k][ch]);
-        if (bo)   // m*warp + (1-m)*img   obst_eval.py:500
-          st_stream(bo + ch * gplane + off, __fadd_rn(__fmul_rn(keepf, wv[k][ch]), __fmul_rn(__fsub_rn(1.0f, keepf), cur[k][ch])));
+        if constexpr (FE != 1) {   // (uint8 frames: mask_out only)
+          if (wo) st_stream(wo + ch * gplane + off, wv[k][ch]);
+          if (bo)   // m*warp + (1-m)*img   obst_eval.py:500
+            st_stream(bo + ch * gplane + off, __fadd_rn(__fmul_rn(keepf, wv[k][ch]), __fmul_rn(__fsub_rn(1.0f, keepf), cur[k][ch])));
+        }
       }
     }
   }
@@ -1292,11 +1420,11 @@ __device__ __forceinline__ float lean_tile_packed(const FwdParams& p, const floa
 //   consumer warps  one pass per pixel: flow + 4 neighbours from the flow tile (vertical strips, see WsCfg),
 //                   motion-boundary test, sampling position, 4 x (2 + C) taps from the source boxes, occlusion test,
 //                   masked error against `cur` (coalesced global loads issued before the wait for the boxes).
-template <typename FrameT, int MASK, bool REDUCE, int CT, int LEAN, typename Cfg>
-__global__ void __launch_bounds__(Cfg::kThreads, 1) fused_forward_ws_kernel(const FwdParams p, const __grid_constant__ CUtensorMap tm_bf,
-                                                                         const __grid_constant__ CUtensorMap tm_ff,
-                                                                         const __grid_constant__ CUtensorMap tm_prev,
-                                                                         const __grid_constant__ CUtensorMap tm_cur) {
+template <typename FrameT, int MASK, bool REDUCE, int CT, int LEAN, typename Cfg, typename Params>
+__device__ __forceinline__ void fused_forward_ws(const Params& p, const CUtensorMap& tm_bf, const CUtensorMap& tm_ff,
+                                                 const CUtensorMap& tm_prev, const CUtensorMap& tm_cur) {
+  static_assert(std::is_same<FrameT, uint8_t>::value == std::is_same<Params, FwdParamsU8>::value,
+                "uint8 frames come with their normalisation (FwdParamsU8), the other frame types without it");
   constexpr int NB = Cfg::NB, NS = Cfg::NS, P = Cfg::kPPL;
   constexpr int kCWarps = Cfg::CW;
   constexpr int kLoss = LEAN == kVarL1 ? TCLB200_L1 : TCLB200_L2;
@@ -1503,7 +1631,7 @@ __global__ void __launch_bounds__(Cfg::kThreads, 1) fused_forward_ws_kernel(cons
         for (int c = 0; c < Cfg::kC; ++c) {
           const FrameT* pc = cb + (size_t)c * plane;
 #pragma unroll
-          for (int i = 0; i < P; ++i) cur[i][c] = have_cur ? to_f32(__ldg(pc + (ptrdiff_t)pix_dy(i) * g.W)) : 0.0f;
+          for (int i = 0; i < P; ++i) cur[i][c] = have_cur ? frame_value<FrameT>(p, to_f32(__ldg(pc + (ptrdiff_t)pix_dy(i) * g.W)), c) : 0.0f;
         }
 #pragma unroll
         for (int i = 0; i < P; ++i) mk[i] = MASK == MASK_GIVEN ? __ldcs(mb + (ptrdiff_t)pix_dy(i) * g.W) : 0.0f;
@@ -1512,7 +1640,7 @@ __global__ void __launch_bounds__(Cfg::kThreads, 1) fused_forward_ws_kernel(cons
         for (int c = 0; c < Cfg::kC; ++c) {
           const FrameT* pc = cb + (size_t)c * plane;
 #pragma unroll
-          for (int i = 0; i < P; ++i) cur[i][c] = have_cur ? ld_stream(pc + (ptrdiff_t)pix_dy(i) * g.W) : 0.0f;
+          for (int i = 0; i < P; ++i) cur[i][c] = have_cur ? frame_value<FrameT>(p, ld_stream(pc + (ptrdiff_t)pix_dy(i) * g.W), c) : 0.0f;
         }
 #pragma unroll
         for (int i = 0; i < P; ++i) mk[i] = MASK == MASK_GIVEN ? __ldcs(mb + (ptrdiff_t)pix_dy(i) * g.W) : 0.0f;
@@ -1522,7 +1650,7 @@ __global__ void __launch_bounds__(Cfg::kThreads, 1) fused_forward_ws_kernel(cons
           const bool inside = t.x0 + lx0 < g.W && t.y0 + ly0 + pix_dy(i) < p.row_end;
           const ptrdiff_t off = (ptrdiff_t)pix_dy(i) * g.W;
 #pragma unroll
-          for (int c = 0; c < Cfg::kC; ++c) cur[i][c] = (have_cur && inside) ? ld_stream(cb + off + (size_t)c * plane) : 0.0f;
+          for (int c = 0; c < Cfg::kC; ++c) cur[i][c] = (have_cur && inside) ? frame_value<FrameT>(p, ld_stream(cb + off + (size_t)c * plane), c) : 0.0f;
           mk[i] = (MASK == MASK_GIVEN && inside) ? __ldcs(mb + off) : 0.0f;
         }
       }
@@ -1539,7 +1667,7 @@ __global__ void __launch_bounds__(Cfg::kThreads, 1) fused_forward_ws_kernel(cons
       if (t_edge) lean_tile<FrameT, MASK, CT, TCLB200_L2, Cfg, true, false, false>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
       else lean_tile<FrameT, MASK, CT, TCLB200_L2, Cfg, false, false, false>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
     } else if (LEAN && mode == 1) {
-      if constexpr (uses_packed(MASK, REDUCE, CT, LEAN)) {
+      if constexpr (uses_packed(MASK, REDUCE, CT, LEAN) && sizeof(FrameT) != 1) {
         if (t_edge) err = lean_tile_packed<FrameT, MASK, kLoss, Cfg, true, false, CT>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
         else err = lean_tile_packed<FrameT, MASK, kLoss, Cfg, false, false, CT>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
       } else {
@@ -1549,7 +1677,7 @@ __global__ void __launch_bounds__(Cfg::kThreads, 1) fused_forward_ws_kernel(cons
     } else if (LEAN == kVarOutputs) {   // outputs wanted and the tile is mixed / unstaged: the feature-complete exact path
       err = full_tile<FrameT, MASK, REDUCE, CT, kVarGeneral, Cfg, true>(p, bf_stage(sb), ff_stage(ss), prev_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk, have_cur, near);
     } else if (LEAN && mode == 2) {
-      if constexpr (uses_packed(MASK, REDUCE, CT, LEAN)) err = lean_tile_packed<FrameT, MASK, kLoss, Cfg, true, true, CT>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
+      if constexpr (uses_packed(MASK, REDUCE, CT, LEAN) && sizeof(FrameT) != 1) err = lean_tile_packed<FrameT, MASK, kLoss, Cfg, true, true, CT>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
       else err = lean_tile<FrameT, MASK, CT, kLoss, Cfg, true, true>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
     } else if (LEAN || t_edge) {
       err = full_tile<FrameT, MASK, REDUCE, CT, LEAN, Cfg, true>(p, bf_stage(sb), ff_stage(ss), prev_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk, have_cur, near);
@@ -1563,6 +1691,23 @@ __global__ void __launch_bounds__(Cfg::kThreads, 1) fused_forward_ws_kernel(cons
     if (threadIdx.x == 0) TCL_STAMP(k, 3);
   }
   if (!LEAN) count_near(near, p.near_threshold);
+}
+template <typename FrameT, int MASK, bool REDUCE, int CT, int LEAN, typename Cfg>
+__global__ void __launch_bounds__(Cfg::kThreads, 1) fused_forward_ws_kernel(const FwdParams p, const __grid_constant__ CUtensorMap tm_bf,
+                                                                         const __grid_constant__ CUtensorMap tm_ff,
+                                                                         const __grid_constant__ CUtensorMap tm_prev,
+                                                                         const __grid_constant__ CUtensorMap tm_cur) {
+  fused_forward_ws<FrameT, MASK, REDUCE, CT, LEAN, Cfg>(p, tm_bf, tm_ff, tm_prev, tm_cur);
+}
+// uint8 frames (C == 3, reductions only): the same kernel with the normalisation behind the parameters.  The staged taps of
+// tiles whose source box crosses the image border carry per-tap predicates (the box's out-of-image fill is byte 0, which would
+// normalise to the offset, not to grid_sample's 0), and the tiles never take the packed-arithmetic path (lean_tile only).
+template <int MASK, bool REDUCE, int CT, int LEAN, typename Cfg>
+__global__ void __launch_bounds__(Cfg::kThreads, 1) fused_forward_ws_u8_kernel(const FwdParamsU8 p, const __grid_constant__ CUtensorMap tm_bf,
+                                                                            const __grid_constant__ CUtensorMap tm_ff,
+                                                                            const __grid_constant__ CUtensorMap tm_prev,
+                                                                            const __grid_constant__ CUtensorMap tm_cur) {
+  fused_forward_ws<uint8_t, MASK, REDUCE, CT, LEAN, Cfg>(p, tm_bf, tm_ff, tm_prev, tm_cur);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1971,8 +2116,9 @@ constexpr WsGeo ws_geo(int esize, int mask, int ct, int var, int cw) {
   const bool mask_only = ff && ct == 0 && var == kVarL2;   // fbcCheckTorch on its own: no frame planes, a third stage fits
   const int ns = !ff ? TCL_NS_NOFF : mask_only ? TCL_NS_MASK : TCL_NS;
   const int nb = !ff ? TCL_NS_NOFF + 2 : mask_only ? TCL_NS_MASK + 2 : TCL_NB;
-  const int bh = !ff ? TCL_BH_NOFF : esize == 2 ? TCL_BH16 : cw == 8 ? TCL_BH8 : TCL_BH;
-  return {cw, ns, nb, esize == 2 ? TCL_BW16 : TCL_BW, bh, ff};
+  // (uint8 frames take bf16's geometry: smaller boxes than fp32's, retuned only with a measurement that shows a gain)
+  const int bh = !ff ? TCL_BH_NOFF : esize != 4 ? TCL_BH16 : cw == 8 ? TCL_BH8 : TCL_BH;
+  return {cw, ns, nb, esize != 4 ? TCL_BW16 : TCL_BW, bh, ff};
 }
 
 static inline int cdiv(int a, int b) { return (a + b - 1) / b; }
@@ -2010,7 +2156,8 @@ static bool make_map(CUtensorMap* m, const void* base, int esize, int W, int H, 
   const cuuint64_t strides[3] = {(cuuint64_t)W * esize, (cuuint64_t)plane_stride * esize, (cuuint64_t)batch_stride * esize};
   const cuuint32_t box[4] = {(cuuint32_t)bw, (cuuint32_t)bh, (cuuint32_t)bp, 1u};
   const cuuint32_t estr[4] = {1u, 1u, 1u, 1u};
-  const CUtensorMapDataType dt = esize == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
+  const CUtensorMapDataType dt = esize == 1 ? CU_TENSOR_MAP_DATA_TYPE_UINT8
+                                 : esize == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
   return fn(m, dt, 4, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
             CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
@@ -2075,7 +2222,7 @@ extern "C" void tclb200_debug_force_generic(int on) { g_force_generic = on; }
 enum : int { kPathGeneric = 0, kPathDirect = 1, kPathTma = 2 };
 struct FwdPlan {
   int path;
-  int esize;               // frame type of the instantiation: 4 = fp32, 2 = bf16
+  int esize;               // frame type of the instantiation: 4 = fp32, 2 = bf16, 1 = uint8
   int mask_kind;
   bool reduce;
   int ct, var, cw;         // CT; variant (kVar*; the direct kernel's loss); consumer warps (TMA kernel: 8 or 16, else 0)
@@ -2087,7 +2234,8 @@ struct FwdPlan {
 static FwdPlan plan_forward(const tclb200_tcl_args* a, bool tma_ok) {
   FwdPlan q;
   memset(&q, 0, sizeof(q));
-  q.esize = a->dtype == TCLB200_BF16 ? 2 : 4;
+  // (uint8 frames: frame-less calls -- fbcCheckTorch on its own, a dataset mask copied out -- read no frames and take the fp32 rows)
+  q.esize = a->dtype == TCLB200_BF16 ? 2 : (a->dtype == TCLB200_U8 && a->prev) ? 1 : 4;
   q.mask_kind = a->ff ? MASK_COMPUTED : (a->mask_in ? MASK_GIVEN : MASK_NONE);
   q.reduce = a->cur && (a->pair_sums || a->total_sums || a->pair_vals || a->total_val);
   q.ct = a->prev && a->C == 3 ? 3 : 0;
@@ -2097,7 +2245,8 @@ static FwdPlan plan_forward(const tclb200_tcl_args* a, bool tma_ok) {
                    aligned16(a->ff) && aligned16(a->prev) && aligned16(a->cur) && (!a->prev || a->C == 3) && a->B <= 65535 * 16 &&
                    a->H <= 16384 && a->W <= 16384;   // (box addresses are evaluated in fp32, see lean_tile)
   // short launches of the training loss (dataset mask, reduction only): the direct kernel, no tensor maps needed
-  const bool direct = tma && g_force_generic != 2 && q.mask_kind == MASK_GIVEN && q.reduce && a->C == 3 && !a->warp_out && !a->mask_out &&
+  // (uint8 frames have no direct rows: a uint8 frame is a decoded video frame to be scored, not a training batch)
+  const bool direct = tma && g_force_generic != 2 && q.esize != 1 && q.mask_kind == MASK_GIVEN && q.reduce && a->C == 3 && !a->warp_out && !a->mask_out &&
                       !a->blend_out && !a->near_threshold && !(a->flags & (TCLB200_VALIDITY | TCLB200_THROUGHPUT)) && aligned16(a->mask_in) &&
                       ((size_t)a->B * (size_t)rows * a->W <= TCL_DIRECT_MAX_PX || g_force_generic == 3);
   if (!tma) {
@@ -2148,25 +2297,39 @@ static FwdPlan plan_forward(const tclb200_tcl_args* a, bool tma_ok) {
 template <int PATH, typename FrameT, int MASK, bool REDUCE, int CT, int VAR, int CW>
 static cudaError_t launch_forward(const FwdParams& p, const CUtensorMap* tm, cudaStream_t s) {
   const size_t tiles = (size_t)p.B * p.tiles_per_pair;
-  if constexpr (PATH == kPathGeneric) {
+  if constexpr (PATH == kPathGeneric && std::is_same<FrameT, uint8_t>::value) {
+    static_assert(REDUCE && CT == 3, "uint8 frames: C == 3, reductions only");
+    fused_forward_generic_u8_kernel<MASK><<<(unsigned)tiles, kThreads, 0, s>>>(static_cast<const FwdParamsU8&>(p));
+  } else if constexpr (PATH == kPathGeneric) {
     fused_forward_generic_kernel<FrameT, MASK, REDUCE, CT><<<(unsigned)tiles, kThreads, 0, s>>>(p);
   } else if constexpr (PATH == kPathDirect) {
     fused_forward_direct_kernel<FrameT, VAR == kVarL1 ? TCLB200_L1 : TCLB200_L2><<<(unsigned)tiles, kDirectThreads, 0, s>>>(p);
   } else {
     constexpr WsGeo G = ws_geo((int)sizeof(FrameT), MASK, CT, VAR, CW);
     using Cfg = WsCfg<FrameT, CT, kTW, kTH, G.bw, G.bh, G.nb, G.ns, G.cw, G.ff>;
-    auto kern = fused_forward_ws_kernel<FrameT, MASK, REDUCE, CT, VAR, Cfg>;
-    static bool configured[64] = {};  // per instantiation and device (the attribute is a per-device property of the function)
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) dev = 63;   // (an uncached slot: set the attribute every time)
-    if (!configured[dev] || dev == 63) {
-      const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmemBytes);
-      if (e != cudaSuccess) return e;
-      configured[dev] = true;
+    // (uint8 frames: the entry that takes FwdParamsU8, i.e. the parameters followed by the normalisation)
+    auto launch = [&](auto kern, const auto& params) -> cudaError_t {
+      static bool configured[64] = {};  // per instantiation and device (the attribute is a per-device property of the function)
+      int dev = 0;
+      if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) dev = 63;   // (an uncached slot: set the attribute every time)
+      if (!configured[dev] || dev == 63) {
+        const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmemBytes);
+        if (e != cudaSuccess) return e;
+        configured[dev] = true;
+      }
+      // persistent: one CTA per SM (or fewer when there are fewer tiles)
+      const size_t slots = (size_t)sm_count();
+      kern<<<(unsigned)(tiles < slots ? tiles : slots), Cfg::kThreads, Cfg::kSmemBytes, s>>>(params, tm[0], tm[1], tm[2], tm[3]);
+      return cudaSuccess;
+    };
+    cudaError_t e0;
+    if constexpr (std::is_same<FrameT, uint8_t>::value) {
+      static_assert(REDUCE && CT == 3, "uint8 frames: C == 3, reductions only");
+      e0 = launch(fused_forward_ws_u8_kernel<MASK, REDUCE, CT, VAR, Cfg>, static_cast<const FwdParamsU8&>(p));
+    } else {
+      e0 = launch(fused_forward_ws_kernel<FrameT, MASK, REDUCE, CT, VAR, Cfg>, p);
     }
-    // persistent: one CTA per SM (or fewer when there are fewer tiles)
-    const size_t slots = (size_t)sm_count();
-    kern<<<(unsigned)(tiles < slots ? tiles : slots), Cfg::kThreads, Cfg::kSmemBytes, s>>>(p, tm[0], tm[1], tm[2], tm[3]);
+    if (e0 != cudaSuccess) return e0;
   }
   ++g_launches;
   const cudaError_t e = cudaGetLastError();
@@ -2216,6 +2379,9 @@ static constexpr FwdRow kFwdRows[] = {
     row<kPathGeneric, bf16, MASK_GIVEN, false, 3, kVarGeneral>(),     row<kPathGeneric, bf16, MASK_GIVEN, false, 0, kVarGeneral>(),
     row<kPathGeneric, bf16, MASK_NONE, true, 3, kVarGeneral>(),       row<kPathGeneric, bf16, MASK_NONE, true, 0, kVarGeneral>(),
     row<kPathGeneric, bf16, MASK_NONE, false, 3, kVarGeneral>(),      row<kPathGeneric, bf16, MASK_NONE, false, 0, kVarGeneral>(),
+    // ... and uint8 frames (C == 3, reductions only; `p` is the FwdParamsU8 of run_fused) on shapes TMA cannot describe
+    row<kPathGeneric, uint8_t, MASK_COMPUTED, true, 3, kVarGeneral>(), row<kPathGeneric, uint8_t, MASK_GIVEN, true, 3, kVarGeneral>(),
+    row<kPathGeneric, uint8_t, MASK_NONE, true, 3, kVarGeneral>(),
     // direct kernel: short launches of the training loss
     row<kPathDirect, float, MASK_GIVEN, true, 3, kVarL2>(), row<kPathDirect, float, MASK_GIVEN, true, 3, kVarL1>(),
     row<kPathDirect, bf16, MASK_GIVEN, true, 3, kVarL2>(),  row<kPathDirect, bf16, MASK_GIVEN, true, 3, kVarL1>(),
@@ -2230,6 +2396,8 @@ static constexpr FwdRow kFwdRows[] = {
     row<kPathTma, bf16, MASK_COMPUTED, true, 3, kVarOutputs, 16>(),   row<kPathTma, bf16, MASK_COMPUTED, true, 3, kVarGeneral, 16>(),
     row<kPathTma, bf16, MASK_COMPUTED, false, 3, kVarOutputs, 16>(),  row<kPathTma, bf16, MASK_COMPUTED, false, 3, kVarGeneral, 16>(),
     row<kPathTma, bf16, MASK_COMPUTED, false, 0, kVarGeneral, 16>(),
+    row<kPathTma, uint8_t, MASK_COMPUTED, true, 3, kVarL2, 16>(),     row<kPathTma, uint8_t, MASK_COMPUTED, true, 3, kVarL1, 16>(),
+    row<kPathTma, uint8_t, MASK_COMPUTED, true, 3, kVarOutputs, 16>(), row<kPathTma, uint8_t, MASK_COMPUTED, true, 3, kVarGeneral, 16>(),
     // TMA kernel, dataset mask
     row<kPathTma, float, MASK_GIVEN, true, 3, kVarL2, 16>(),          row<kPathTma, float, MASK_GIVEN, true, 3, kVarL1, 16>(),
     row<kPathTma, float, MASK_GIVEN, true, 3, kVarOutputs, 16>(),     row<kPathTma, float, MASK_GIVEN, true, 3, kVarGeneral, 16>(),
@@ -2239,11 +2407,14 @@ static constexpr FwdRow kFwdRows[] = {
     row<kPathTma, bf16, MASK_GIVEN, true, 3, kVarOutputs, 16>(),      row<kPathTma, bf16, MASK_GIVEN, true, 3, kVarGeneral, 16>(),
     row<kPathTma, bf16, MASK_GIVEN, false, 3, kVarOutputs, 16>(),     row<kPathTma, bf16, MASK_GIVEN, false, 3, kVarGeneral, 16>(),
     row<kPathTma, bf16, MASK_GIVEN, false, 0, kVarGeneral, 16>(),
+    row<kPathTma, uint8_t, MASK_GIVEN, true, 3, kVarL2, 16>(),        row<kPathTma, uint8_t, MASK_GIVEN, true, 3, kVarL1, 16>(),
+    row<kPathTma, uint8_t, MASK_GIVEN, true, 3, kVarGeneral, 16>(),
     // TMA kernel, no mask
     row<kPathTma, float, MASK_NONE, true, 3, kVarGeneral, 16>(),      row<kPathTma, float, MASK_NONE, false, 3, kVarGeneral, 16>(),
     row<kPathTma, float, MASK_NONE, false, 3, kVarL2, 16>(),          row<kPathTma, float, MASK_NONE, false, 0, kVarGeneral, 16>(),
     row<kPathTma, bf16, MASK_NONE, true, 3, kVarGeneral, 16>(),       row<kPathTma, bf16, MASK_NONE, false, 3, kVarGeneral, 16>(),
     row<kPathTma, bf16, MASK_NONE, false, 3, kVarL2, 16>(),           row<kPathTma, bf16, MASK_NONE, false, 0, kVarGeneral, 16>(),
+    row<kPathTma, uint8_t, MASK_NONE, true, 3, kVarGeneral, 16>(),
 };
 
 static const FwdRow* find_row(const FwdPlan& q) {
@@ -2257,7 +2428,15 @@ static int run_fused(const tclb200_tcl_args* a, cudaStream_t s) {
   if (!a) return fail(TCLB200_ERR_INVALID, "args is NULL");
   if (a->B <= 0 || a->H <= 0 || a->W <= 0) return fail(TCLB200_ERR_INVALID, "B, H, W must be positive");
   if (!a->bf) return fail(TCLB200_ERR_INVALID, "bf (the flow the warp samples with) is required");
-  if (a->dtype != TCLB200_F32 && a->dtype != TCLB200_BF16) return fail(TCLB200_ERR_INVALID, "unknown dtype");
+  if (a->dtype != TCLB200_F32 && a->dtype != TCLB200_BF16 && a->dtype != TCLB200_U8) return fail(TCLB200_ERR_INVALID, "unknown dtype");
+  if (a->dtype == TCLB200_U8 && a->prev) {   // uint8 frames are scored, never written: C == 3, a reduction, a finite normalisation
+    if (a->warp_out || a->blend_out) return fail(TCLB200_ERR_UNSUPPORTED, "uint8 frames: warp_out / blend_out are not supported (reductions only)");
+    if (a->C != 3) return fail(TCLB200_ERR_INVALID, "uint8 frames must have C == 3");
+    if (!a->cur || !(a->pair_sums || a->total_sums || a->pair_vals || a->total_val))
+      return fail(TCLB200_ERR_INVALID, "uint8 frames need cur and a reduction (pair_sums / total_sums / pair_vals / total_val)");
+    for (int c = 0; c < 3; ++c)
+      if (!isfinite(a->u8_scale[c]) || !isfinite(a->u8_offset[c])) return fail(TCLB200_ERR_INVALID, "uint8 frames: u8_scale / u8_offset must be finite");
+  }
   if (a->loss != TCLB200_L2 && a->loss != TCLB200_L1) return fail(TCLB200_ERR_INVALID, "unknown loss");
   if (a->finalize != TCLB200_FIN_MEAN && a->finalize != TCLB200_FIN_RMSE) return fail(TCLB200_ERR_INVALID, "unknown finalize");
   if (a->prev && a->C <= 0) return fail(TCLB200_ERR_INVALID, "C must be positive when frames are given");
@@ -2298,8 +2477,11 @@ static int run_fused(const tclb200_tcl_args* a, cudaStream_t s) {
     if (!ok) plan = plan_forward(a, false);   // a tensor map that does not encode: the generic kernel
   }
 
-  FwdParams p;
-  memset(&p, 0, sizeof(p));
+  FwdParamsU8 pu8;   // FwdParams + the normalisation of uint8 frames (only the uint8 kernels take the latter)
+  memset(&pu8, 0, sizeof(pu8));
+  if (plan.esize == 1)
+    for (int c = 0; c < 3; ++c) { pu8.norm.scale[c] = a->u8_scale[c]; pu8.norm.offset[c] = a->u8_offset[c]; }
+  FwdParams& p = pu8;
   p.ff = a->ff; p.bf = a->bf; p.mask_in = a->mask_in; p.prev = a->prev; p.cur = a->cur;
   p.ff_plane = ff_plane; p.ff_batch = ff_batch; p.bf_plane = bf_plane; p.bf_batch = bf_batch;
   p.prev_index = a->prev ? a->prev_index : nullptr; p.cur_index = a->cur ? a->cur_index : nullptr;
@@ -2344,6 +2526,7 @@ extern "C" int tclb200_tcl_forward(const tclb200_tcl_args* args, tclb200_stream_
 extern "C" int tclb200_warp(const void* x, const float* f, void* out, int B, int C, int H, int W, int dtype, int flags,
                             tclb200_stream_t stream) {
   if (!x || !f || !out) return fail(TCLB200_ERR_INVALID, "x, f and out are required");
+  if (dtype == TCLB200_U8) return fail(TCLB200_ERR_INVALID, "warp: uint8 frames are not a dtype of warped outputs (float32 / bfloat16)");
   tclb200_tcl_args a;
   memset(&a, 0, sizeof(a));
   a.bf = f; a.prev = x; a.warp_out = out;
@@ -2434,6 +2617,7 @@ extern "C" size_t tclb200_backward_workspace_bytes(int B, int C, int H, int W, i
 
 // the frame dtype and, for bf16 frames with a grad_x / grad_prev, the accumulator workspace: p.grad_x is pointed at it
 static int backward_dtype_setup(BwdParams& p, int dtype, void* grad_x, void* workspace, size_t workspace_bytes, const char* what) {
+  if (dtype == TCLB200_U8) return fail(TCLB200_ERR_INVALID, "uint8 frames have no backward (dtype TCLB200_U8 is scored, never differentiated)");
   if (dtype != TCLB200_F32 && dtype != TCLB200_BF16) return fail(TCLB200_ERR_INVALID, "unknown dtype");
   if (dtype == TCLB200_F32 || grad_x == nullptr) {
     p.grad_x = static_cast<float*>(grad_x);

@@ -24,7 +24,7 @@ import ctypes
 import torch
 
 from . import _cabi
-from ._cabi import BF16, F32, FIN_MEAN, FIN_RMSE, L1, L2, MOB, OCC, VALIDITY, HostArgs, TclArgs, check
+from ._cabi import BF16, F32, FIN_MEAN, FIN_RMSE, L1, L2, MOB, OCC, U8, VALIDITY, HostArgs, TclArgs, check
 
 _scratch_cache = {}
 
@@ -73,6 +73,38 @@ def _frame_dtype(t):
     if t.dtype == torch.bfloat16:
         return BF16
     raise RuntimeError(f"tcl_b200: frames must be float32 or bfloat16, got {t.dtype}")
+
+
+U8_SCALE = float(torch.tensor(1.0 / 255.0, dtype=torch.float32))   # the default normalisation of uint8 frames: [0, 1]
+
+
+def _eval_frame_dtype(t):
+    """The frame dtype of an evaluation entry: float32, bfloat16, or uint8 (stored video, scored only)."""
+    return U8 if t.dtype == torch.uint8 else _frame_dtype(t)
+
+
+def _u8_norm(dt, u8_scale, u8_offset, C):
+    """-> ((scale x3), (offset x3)) as fp32 values.  ``u8_scale`` / ``u8_offset``: a float or 3 floats (per channel); None =
+    1/255 and 0.  Non-default values with frames that are not uint8 raise instead of being ignored."""
+    if dt != U8:
+        if u8_scale is not None or u8_offset is not None:
+            raise RuntimeError("tcl_b200: u8_scale / u8_offset apply to uint8 frames only")
+        return (0.0,) * 3, (0.0,) * 3
+    if C != 3:
+        raise RuntimeError(f"tcl_b200: uint8 frames must have 3 channels, got {C}")
+
+    def three(v, default, name):
+        v = default if v is None else v
+        v = [float(x) for x in (v.flatten().tolist() if torch.is_tensor(v) else (v if isinstance(v, (list, tuple)) else [v]))]
+        if len(v) == 1:
+            v = v * 3
+        if len(v) != 3:
+            raise RuntimeError(f"tcl_b200: {name} must be a float or 3 floats, got {len(v)}")
+        v = torch.tensor(v, dtype=torch.float32)   # (the values the kernels use: rounded to fp32 once)
+        if not bool(torch.isfinite(v).all()):
+            raise RuntimeError(f"tcl_b200: {name} must be finite")
+        return tuple(float(x) for x in v)
+    return three(u8_scale, U8_SCALE, "u8_scale"), three(u8_offset, 0.0, "u8_offset")
 
 
 def _scratch(B, H, W, device):
@@ -287,7 +319,8 @@ def _index(idx, B, n_frames, name, validate=True):
 
 def fused_forward(bf, prev, cur, ff=None, mask=None, loss=L2, finalize=FIN_RMSE, flags=OCC | MOB,
                   want_warp=False, want_mask=False, want_blend=False, want_near=False, want_sums=True,
-                  prev_index=None, cur_index=None, validate_index=True, bf_index=None, ff_index=None, pair_group=0, rows=None):
+                  prev_index=None, cur_index=None, validate_index=True, bf_index=None, ff_index=None, pair_group=0, rows=None,
+                  u8_scale=None, u8_offset=None):
     """One launch: warp ``prev`` by ``bf``, build or read the mask, reduce the masked error against ``cur``.
 
     ``ff`` given -> the mask is computed (fbcCheckTorch semantics, tests per ``flags``);
@@ -303,6 +336,10 @@ def fused_forward(bf, prev, cur, ff=None, mask=None, loss=L2, finalize=FIN_RMSE,
 
     Band mode: ``rows=(r0, r1)`` evaluates target rows [r0, r1) of every pair only (inputs stay whole frames); the result
     carries ``pair_sums`` / ``total_sums`` but no means (see ``sharding.evaluate_banded``).
+
+    uint8 frames (B,3,H,W) -- stored video: PNGs, decoded clips -- are scored as ``u.float() * u8_scale + u8_offset`` (per
+    channel; a float or 3 floats; default 1/255 and 0, i.e. [0, 1]); the result is the fp32 path's on the normalised frames.
+    Reductions only: ``want_warp`` / ``want_blend`` raise, ``want_sums`` must stay on.
     """
     _require_cuda(bf, prev, cur, ff, mask, bf_index, ff_index)
     bf, bf_plane, bf_batch = _flow_view(bf, "bf")
@@ -324,9 +361,10 @@ def fused_forward(bf, prev, cur, ff=None, mask=None, loss=L2, finalize=FIN_RMSE,
         out_like = torch.empty((B,) + tuple(prev.shape[1:]), dtype=prev.dtype, device=prev.device)
     else:
         out_like = None
-    dt = _frame_dtype(prev)
+    dt = _eval_frame_dtype(prev)
     prev, cur = prev.contiguous(), cur.contiguous()
     C = prev.shape[1]
+    norm = _u8_norm(dt, u8_scale, u8_offset, C)
     dev = bf.device
     if mask is not None and ff is None:
         if mask.shape != (B, 1, H, W):
@@ -373,21 +411,23 @@ def fused_forward(bf, prev, cur, ff=None, mask=None, loss=L2, finalize=FIN_RMSE,
         a.pair_group = int(pair_group)
         if rows is not None:
             a.row_begin, a.row_end = r0, r1
+        a.u8_scale[:], a.u8_offset[:] = norm
         check(_cabi.lib().tclb200_tcl_forward(ctypes.byref(a), _stream_handle()))
     return res
 
 
-def temporal_error(ff, bf, prev, cur):
-    """``computeTCL`` minus RAFT and the generator: sqrt(mean((mask*(cur - warp(prev,bf)))**2)), 0-dim tensor."""
-    return fused_forward(bf, prev, cur, ff=ff, finalize=FIN_RMSE).total_val
+def temporal_error(ff, bf, prev, cur, u8_scale=None, u8_offset=None):
+    """``computeTCL`` minus RAFT and the generator: sqrt(mean((mask*(cur - warp(prev,bf)))**2)), 0-dim tensor.
+    (uint8 frames: see ``fused_forward`` for ``u8_scale`` / ``u8_offset``; the same holds for the functions below.)"""
+    return fused_forward(bf, prev, cur, ff=ff, finalize=FIN_RMSE, u8_scale=u8_scale, u8_offset=u8_offset).total_val
 
 
-def temporal_error_per_pair(ff, bf, prev, cur):
+def temporal_error_per_pair(ff, bf, prev, cur, u8_scale=None, u8_offset=None):
     """Per-pair RMSE (B,) with the mask computed from (ff,bf) -- the batched form of ``computeTCL``."""
-    return fused_forward(bf, prev, cur, ff=ff, finalize=FIN_RMSE).pair_vals
+    return fused_forward(bf, prev, cur, ff=ff, finalize=FIN_RMSE, u8_scale=u8_scale, u8_offset=u8_offset).pair_vals
 
 
-def temporal_error_clip(frames, ff, bf):
+def temporal_error_clip(frames, ff, bf, u8_scale=None, u8_offset=None):
     """Per-pair RMSE (T-1,) over a clip of T stylised frames stored ONCE: pair i warps ``frames[i]`` by ``bf[i]`` and
     compares with ``frames[i+1]`` under the mask of (``ff[i]``, ``bf[i]``) -- the evaluation loop of
     utils/sintel_eval.py:206-222 for a deterministic generator.  Every frame is read from HBM once (28 instead of
@@ -397,7 +437,7 @@ def temporal_error_clip(frames, ff, bf):
         raise RuntimeError(f"tcl_b200: a clip of {T} frames has {T - 1} consecutive pairs, got {bf.shape[0]} flows")
     idx = torch.arange(T, dtype=torch.int32, device=frames.device)
     return fused_forward(bf, frames, frames, ff=ff, finalize=FIN_RMSE, prev_index=idx[:-1], cur_index=idx[1:],
-                         validate_index=False).pair_vals
+                         validate_index=False, u8_scale=u8_scale, u8_offset=u8_offset).pair_vals
 
 
 def window_evaluations(n_frames, window=4):
@@ -429,9 +469,9 @@ def window_evaluations(n_frames, window=4):
             "group": 2 * (window - 1), "n_complete": len(full)}
 
 
-def temporal_error_window(frames, flow_bank, window=4, index=None, finalize=FIN_RMSE):
+def temporal_error_window(frames, flow_bank, window=4, index=None, finalize=FIN_RMSE, u8_scale=None, u8_offset=None):
     """Temporal error of every directed evaluation of a clip's temporal windows in ONE launch, everything stored once:
-    ``frames`` (T,C,H,W) fp32/bf16, ``flow_bank`` (2*J,2,H,W) in the layout of ``window_evaluations`` (``index`` = its
+    ``frames`` (T,C,H,W) fp32/bf16/uint8, ``flow_bank`` (2*J,2,H,W) in the layout of ``window_evaluations`` (``index`` = its
     result, computed when omitted).  Each frame is the ``cur`` of up to window-1 evaluations and the ``prev`` of as many,
     each flow field the ``bf`` of one and the ``ff`` of the opposite one; the tiles of a target frame's evaluations are
     interleaved (``pair_group``), so the re-reads are L2 hits: 4 frames + 6 fields per complete window of 6 evaluations
@@ -442,7 +482,8 @@ def temporal_error_window(frames, flow_bank, window=4, index=None, finalize=FIN_
     dev = frames.device
     to = lambda k: index[k].to(dev)
     res = fused_forward(flow_bank, frames, frames, ff=flow_bank, finalize=finalize, prev_index=to("prev_index"), cur_index=to("cur_index"),
-                        bf_index=to("bf_index"), ff_index=to("ff_index"), pair_group=index["group"])
+                        bf_index=to("bf_index"), ff_index=to("ff_index"), pair_group=index["group"], u8_scale=u8_scale,
+                        u8_offset=u8_offset)
     return res.pair_vals
 
 
@@ -469,10 +510,12 @@ def _host_tensor(t, name, dtype=None):
 
 
 def temporal_error_host(frames, ff, bf, prev_index=None, cur_index=None, mask=None, loss=L2, finalize=FIN_RMSE,
-                        flags=OCC | MOB, chunk_pairs=0, device=None, sync=True, return_sums=False, max_device_frames=None):
+                        flags=OCC | MOB, chunk_pairs=0, device=None, sync=True, return_sums=False, max_device_frames=None,
+                        u8_scale=None, u8_offset=None):
     """The evaluation loop of utils/sintel_eval.py:206-222 (and solver.py:336-347) on HOST tensors.
 
-    ``frames`` (F,C,H,W) fp32/bf16: the stylised frames of one or more clips, each stored once; ``ff`` / ``bf``
+    ``frames`` (F,C,H,W) fp32/bf16, or (F,3,H,W) uint8 with ``u8_scale`` / ``u8_offset`` as in ``fused_forward`` (a third of
+    the bf16 bytes on the link): the stylised frames of one or more clips, each stored once; ``ff`` / ``bf``
     (P,2,H,W) fp32; pair p warps ``frames[prev_index[p]]`` by ``bf[p]`` and compares with ``frames[cur_index[p]]``
     under the mask of (``ff[p]``, ``bf[p]``) -- or under ``mask[p]`` (P,1,H,W) when ``ff`` is None
     (utils/metrics/eval.py:137-138).  Default indices: the consecutive pairs of ONE clip (P = F-1).
@@ -488,7 +531,7 @@ def temporal_error_host(frames, ff, bf, prev_index=None, cur_index=None, mask=No
     if not torch.cuda.is_available():
         raise RuntimeError("tcl_b200: temporal_error_host needs a CUDA device; this path has no CPU implementation")
     frames = _host_tensor(frames, "frames")
-    dt = _frame_dtype(frames)
+    dt = _eval_frame_dtype(frames)
     bf = _host_tensor(bf, "bf", torch.float32)
     ff = _host_tensor(ff, "ff", torch.float32)
     mask = _host_tensor(mask, "mask", torch.float32) if ff is None else None
@@ -496,6 +539,7 @@ def temporal_error_host(frames, ff, bf, prev_index=None, cur_index=None, mask=No
         raise RuntimeError(f"tcl_b200: frames {tuple(frames.shape)} / bf {tuple(bf.shape)} must be (F,C,H,W) / (P,2,H,W)")
     F_, C, H, W = frames.shape
     P = bf.shape[0]
+    norm = _u8_norm(dt, u8_scale, u8_offset, C)
     if ff is not None and ff.shape != bf.shape:
         raise RuntimeError(f"tcl_b200: ff {tuple(ff.shape)} and bf {tuple(bf.shape)} do not match")
     if mask is not None and tuple(mask.shape) != (P, 1, H, W):
@@ -541,6 +585,7 @@ def temporal_error_host(frames, ff, bf, prev_index=None, cur_index=None, mask=No
     a.P, a.F, a.C, a.H, a.W = P, F_, C, H, W
     a.dtype, a.flags, a.loss, a.finalize, a.chunk_pairs = dt, flags, loss, finalize, chunk_pairs
     a.frame_slots = 0 if slots >= F_ else slots
+    a.u8_scale[:], a.u8_offset[:] = norm
     with torch.cuda.device(dev):
         stream = torch.cuda.current_stream()
         check(lib.tclb200_tcl_forward_host(ctypes.byref(a), ctypes.c_void_p(stream.cuda_stream)))
@@ -551,13 +596,14 @@ def temporal_error_host(frames, ff, bf, prev_index=None, cur_index=None, mask=No
     return (out, sums) if return_sums else out
 
 
-def temporal_rmse_per_sample(mask, cur, prev, flow):
+def temporal_rmse_per_sample(mask, cur, prev, flow, u8_scale=None, u8_offset=None):
     """FC2 metric: ((mask*(cur - warp(prev,flow)))**2).mean(dim=(1,2,3))**0.5 -> (N,)."""
-    return fused_forward(flow, prev, cur, mask=mask, finalize=FIN_RMSE).pair_vals
+    return fused_forward(flow, prev, cur, mask=mask, finalize=FIN_RMSE, u8_scale=u8_scale, u8_offset=u8_offset).pair_vals
 
 
 def warp_blend(mask, prev, flow, img):
     """mask*warp(prev,flow) + (1-mask)*img in one pass (obst_eval.py:500)."""
+    _frame_dtype(prev)   # (a warped output: float32 / bfloat16 frames only)
     return fused_forward(flow, prev, img, mask=mask, want_blend=True, want_sums=False).blend
 
 

@@ -118,12 +118,14 @@ def unpack(packed: torch.Tensor, n_seq: int) -> dict:
 
 
 def evaluate_sharded(ff, bf, prev, cur, seq_of_pair: torch.Tensor, n_seq: int,
-                     group: Optional[dist.ProcessGroup] = None, chunk: Optional[int] = None, kernel_events=None) -> dict:
+                     group: Optional[dist.ProcessGroup] = None, chunk: Optional[int] = None, kernel_events=None,
+                     u8_scale=None, u8_offset=None) -> dict:
     """Temporal error of this rank's shard of pairs (already resident on its GPU) + the one all-reduce.
 
     ``chunk`` bounds the pairs per launch (None = one launch for the shard).  Returns ``unpack``'s dict.
     ``kernel_events``: optional list; a (start, end) pair of CUDA timing events recorded around every fused launch is
     appended to it (bench.py times the dominant kernel inside its timed region this way).
+    uint8 frames: ``u8_scale`` / ``u8_offset`` as in ``ops.fused_forward`` (here and in the two functions below).
     """
     from . import ops
     n = bf.shape[0]
@@ -138,7 +140,8 @@ def evaluate_sharded(ff, bf, prev, cur, seq_of_pair: torch.Tensor, n_seq: int,
             if kernel_events is not None:
                 ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
                 ev[0].record()
-            res = ops.fused_forward(bf[s:e], prev[s:e], cur[s:e], ff=ff[s:e], finalize=ops.FIN_RMSE)
+            res = ops.fused_forward(bf[s:e], prev[s:e], cur[s:e], ff=ff[s:e], finalize=ops.FIN_RMSE, u8_scale=u8_scale,
+                                    u8_offset=u8_offset)
             if kernel_events is not None:
                 ev[1].record()
                 kernel_events.append(ev)
@@ -158,7 +161,7 @@ def band_rows(H: int, world: int, rank: int, align: int = 32):
 
 
 def evaluate_banded(ff, bf, prev, cur, group: Optional[dist.ProcessGroup] = None, rank: Optional[int] = None,
-                    world: Optional[int] = None) -> dict:
+                    world: Optional[int] = None, u8_scale=None, u8_offset=None) -> dict:
     """Fewer pairs than GPUs (one 4K pair on eight GPUs, BASELINE config 5; SURVEY.md section 8e): every rank holds the same
     whole pairs, evaluates one horizontal band of target rows of each (the flow gradient and the bilinear taps read beyond
     the band: the inputs are replicated, nothing is exchanged), and the bands' fp64 sums of squares are added with the path's
@@ -172,7 +175,7 @@ def evaluate_banded(ff, bf, prev, cur, group: Optional[dist.ProcessGroup] = None
     C = prev.shape[1]
     r0, r1 = band_rows(H, world, rank)
     if r1 > r0:
-        sums = ops.fused_forward(bf, prev, cur, ff=ff, rows=(r0, r1)).pair_sums.clone()
+        sums = ops.fused_forward(bf, prev, cur, ff=ff, rows=(r0, r1), u8_scale=u8_scale, u8_offset=u8_offset).pair_sums.clone()
     else:
         sums = torch.zeros(B, dtype=torch.float64, device=bf.device)
     sums = allreduce_sums(sums, group)
@@ -180,7 +183,8 @@ def evaluate_banded(ff, bf, prev, cur, group: Optional[dist.ProcessGroup] = None
 
 
 def evaluate_sharded_host(frames, ff, bf, prev_index, cur_index, seq_of_pair, n_seq: int,
-                          group: Optional[dist.ProcessGroup] = None, device=None, chunk_pairs: int = 0) -> dict:
+                          group: Optional[dist.ProcessGroup] = None, device=None, chunk_pairs: int = 0, u8_scale=None,
+                          u8_offset=None) -> dict:
     """The same evaluation with this rank's shard in HOST memory (``ops.temporal_error_host``: frames of the rank's clips
     stored once, pairs index them) + the one all-reduce.  ``seq_of_pair``: sequence id of each local pair (CPU or CUDA
     long tensor).  Returns ``unpack``'s dict of device tensors."""
@@ -192,7 +196,7 @@ def evaluate_sharded_host(frames, ff, bf, prev_index, cur_index, seq_of_pair, n_
         packed = torch.zeros(2 * n_seq + 2, dtype=torch.float64, device=dev)
     else:
         vals, sums = ops.temporal_error_host(frames, ff, bf, prev_index, cur_index, chunk_pairs=chunk_pairs, device=dev,
-                                             return_sums=True)
+                                             return_sums=True, u8_scale=u8_scale, u8_offset=u8_offset)
         packed = pack_local(vals.to(dev, non_blocking=True), sums.to(dev, non_blocking=True).sum(),
                             torch.as_tensor(seq_of_pair).to(dev), n_seq, C * H * W)
     return unpack(allreduce_sums(packed, group), n_seq)

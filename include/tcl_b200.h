@@ -12,7 +12,9 @@
  *
  * Conventions
  *   - all tensors NCHW contiguous; flows are (B,2,H,W) fp32 in pixels, channel 0 = u (x), 1 = v (y);
- *     frames are (B,C,H,W) fp32 or bf16 (TCLB200_F32 / TCLB200_BF16); masks are (B,1,H,W) fp32 in {0,1}
+ *     frames are (B,C,H,W) fp32 or bf16 (TCLB200_F32 / TCLB200_BF16); masks are (B,1,H,W) fp32 in {0,1};
+ *     the evaluation entries (reductions of tclb200_tcl_forward, tclb200_tcl_forward_host) also score stored 8-bit video:
+ *     (B,3,H,W) uint8 frames (TCLB200_U8) with a per-channel normalisation, see tclb200_tcl_args.u8_scale
  *   - every function returns 0 on success, a TCLB200_ERR_* code otherwise, never throws or aborts;
  *     tclb200_last_error() returns a thread-local message for the last failing call
  *   - no hidden global state: accumulators and scratch are passed in; calls are asynchronous on
@@ -29,7 +31,7 @@
 extern "C" {
 #endif
 
-#define TCLB200_ABI_VERSION 6
+#define TCLB200_ABI_VERSION 7
 
 #define TCLB200_OK 0
 #define TCLB200_ERR_INVALID 1     /* bad argument (null pointer, non-positive size, unknown enum) */
@@ -39,6 +41,8 @@ extern "C" {
 /* frame dtype */
 #define TCLB200_F32 0
 #define TCLB200_BF16 1
+/* (2 is not assigned) */
+#define TCLB200_U8 3   /* planar uint8, C == 3, reductions only: frames that are scored, never written or differentiated  (ABI v7) */
 
 /* mask tests of fbcCheckTorch (utils/flowtools.py:45,53); the optimisation-based variant
  * (methods/optimization-based/flowtools.py:34-58) is TCLB200_MOB alone */
@@ -81,7 +85,7 @@ int tclb200_gradient_strided(const float* x, size_t x_batch_stride, float* out, 
 /* warp(x, f)  utils/flowtools.py:18-32 (copies: utils/metrics/eval.py:43-57, StarGAN/solver.py:42-56;
  * inline: StarGANv2AdvCon/core/solver.py:427-443, CycleGANCon/models/cycle_gan_model.py:191-203)
  * flags & TCLB200_VALIDITY selects fs_lib.warp (methods/learning-based/fs_lib.py:5-39).
- * x, out (B,C,H,W) of `dtype`; f (B,2,H,W) fp32. */
+ * x, out (B,C,H,W) of `dtype` (TCLB200_F32 / TCLB200_BF16; TCLB200_U8 is TCLB200_ERR_INVALID); f (B,2,H,W) fp32. */
 int tclb200_warp(const void* x, const float* f, void* out, int B, int C, int H, int W, int dtype, int flags,
                  tclb200_stream_t stream);
 
@@ -124,7 +128,7 @@ typedef struct tclb200_tcl_args {
   void* scratch;        /* >= tclb200_scratch_bytes(B,H,W), zero-filled at allocation */
   size_t scratch_bytes;
   int B, C, H, W;
-  int dtype;            /* TCLB200_F32 / TCLB200_BF16 (frames only; flows and masks are fp32) */
+  int dtype;            /* TCLB200_F32 / TCLB200_BF16 / TCLB200_U8 (frames only; flows and masks are fp32) */
   int flags;            /* TCLB200_OCC | TCLB200_MOB tests when ff is given; TCLB200_VALIDITY */
   int loss;             /* TCLB200_L2 / TCLB200_L1 */
   int finalize;         /* TCLB200_FIN_MEAN / TCLB200_FIN_RMSE */
@@ -157,6 +161,16 @@ typedef struct tclb200_tcl_args {
    * BASELINE config 5) splits every frame into horizontal bands, one per GPU, and adds the bands' pair_sums with the path's
    * one all-reduce.  pair_vals / total_val are refused in this mode (a band's mean is not the frame's). */
   int row_begin, row_end;
+  /* uint8 frames (dtype TCLB200_U8, ABI v7; read for that dtype only): every frame value the kernels use is
+   *     v = float(u) * u8_scale[c] + u8_offset[c]      (one rounded fp32 product, then one rounded fp32 sum)
+   * -- bit for bit torch's u.float().mul(scale).add(offset) with fp32 (1,3,1,1) scale / offset.  The reference's value ranges:
+   * scale 1/255, offset 0 for [0,1]; scale 2/255, offset -1 for [-1,1] (Normalize(0.5, 0.5)); scale 1, offset -mean_c for
+   * 0..255 with the mean subtracted.  grid_sample's zero padding applies to the normalised frame: a tap outside the image
+   * contributes 0, not u8_offset[c].  With u8 frames C must be 3, a reduction must be requested and scale / offset must be
+   * finite (TCLB200_ERR_INVALID otherwise); warp_out / blend_out are TCLB200_ERR_UNSUPPORTED.  mask_out and near_threshold
+   * work as for fp32 frames, and the result is the fp32 path's on the normalised frames. */
+  float u8_scale[3];
+  float u8_offset[3];
 } tclb200_tcl_args;
 
 int tclb200_tcl_forward(const tclb200_tcl_args* args, tclb200_stream_t stream);
@@ -187,9 +201,13 @@ typedef struct tclb200_host_args {
   int frame_slots;       /* device frame slots the workspace provides: 0 (or >= F) = the whole bank stays resident; fewer =
                           * a ring -- a slot is reused once every chunk that reads its frame has completed; a window of
                           * (3 + 1) chunks of pairs must fit (TCLB200_ERR_INVALID otherwise)          (ABI v5) */
+  /* dtype TCLB200_U8 (ABI v7): as in tclb200_tcl_args.  Each frame crosses PCIe once at 3 B/px instead of 12 (fp32) */
+  float u8_scale[3];
+  float u8_offset[3];
 } tclb200_host_args;
 
-/* F here = the number of device frame slots to provision (tclb200_host_args.frame_slots, or the clip's F for a resident bank) */
+/* F here = the number of device frame slots to provision (tclb200_host_args.frame_slots, or the clip's F for a resident bank);
+ * the frame bank takes C*H*W elements of `dtype` per slot (1 byte each for TCLB200_U8) */
 size_t tclb200_host_workspace_bytes(int P, int F, int C, int H, int W, int dtype, int chunk_pairs, int with_mask);
 int tclb200_tcl_forward_host(const tclb200_host_args* args, tclb200_stream_t stream);
 
@@ -219,7 +237,8 @@ int tclb200_tcl_backward_scaled(const float* bf, const float* mask, const float*
  *   workspace: device memory, 16-byte aligned, >= tclb200_backward_workspace_bytes(B,C,H,W,dtype) bytes; only needed for
  *   bf16 frames with grad_x / grad_prev requested (NULL / 0 otherwise; fp32 frames never use it).  Its contents are
  *   irrelevant; it must stay untouched until the call's work on `stream` has completed.
- *   TCLB200_ERR_INVALID for an unknown dtype or a missing / too small / misaligned workspace, before any CUDA call.
+ *   TCLB200_ERR_INVALID for an unknown dtype (TCLB200_U8 included: uint8 frames are scored, never differentiated) or a
+ *   missing / too small / misaligned workspace, before any CUDA call.
  * With dtype = TCLB200_F32 they are tclb200_warp_backward / tclb200_tcl_backward_scaled. */
 size_t tclb200_backward_workspace_bytes(int B, int C, int H, int W, int dtype);  /* 0 for TCLB200_F32 */
 int tclb200_warp_backward_dt(const void* grad_out, const void* x, const float* f, void* grad_x, float* grad_f, int B, int C, int H,
