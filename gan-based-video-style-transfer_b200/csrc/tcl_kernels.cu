@@ -109,12 +109,19 @@ __device__ __forceinline__ PixTaps pix_taps(float u, float v, int x, int y, cons
   return t;
 }
 
+// taps (x0, y0), (x0 + 1, y0), (x0, y0 + 1), (x0 + 1, y0 + 1) inside the W x H image?  (unsigned: negatives are outside,
+// and a saturated x0 + 1 wraps instead of overflowing)
+struct InImage { bool p00, p10, p01, p11; };
+__device__ __forceinline__ InImage in_image(int x0, int y0, int W, int H) {
+  const bool xin0 = (unsigned)x0 < (unsigned)W, xin1 = (unsigned)x0 + 1u < (unsigned)W;
+  const bool yin0 = (unsigned)y0 < (unsigned)H, yin1 = (unsigned)y0 + 1u < (unsigned)H;
+  return InImage{xin0 && yin0, xin1 && yin0, xin0 && yin1, xin1 && yin1};
+}
+
 __device__ __forceinline__ Taps full_taps(const PixTaps& s, const Geo& g) {
   Taps t;
-  const int x1 = (int)((unsigned)s.x0 + 1u), y1 = (int)((unsigned)s.y0 + 1u);
-  const bool xin0 = (unsigned)s.x0 < (unsigned)g.W, xin1 = (unsigned)x1 < (unsigned)g.W;
-  const bool yin0 = (unsigned)s.y0 < (unsigned)g.H, yin1 = (unsigned)y1 < (unsigned)g.H;
-  t.p00 = xin0 && yin0; t.p10 = xin1 && yin0; t.p01 = xin0 && yin1; t.p11 = xin1 && yin1;
+  const InImage in = in_image(s.x0, s.y0, g.W, g.H);
+  t.p00 = in.p00; t.p10 = in.p10; t.p01 = in.p01; t.p11 = in.p11;
   t.o00 = (int)((unsigned)s.y0 * (unsigned)g.W + (unsigned)s.x0);
   t.nw = s.nw; t.ne = s.ne; t.sw = s.sw; t.se = s.se;
   return t;
@@ -161,23 +168,51 @@ __device__ __forceinline__ float frame_value(const FwdParams& p, float raw, int 
   else return raw;
 }
 
-// source box in shared memory, origin (ox,oy), zero-filled outside the image: all four taps are plain reads.
-// fma(0, w, acc) == acc for the finite weights of an in-box pixel, so this equals the predicated form.
+// The four-tap sum with zero substitution: grid_sampler_2d's accumulation order with every tap multiplied, one product and
+// then three fmas (nw, ne, sw, se).  A tap the sampler would skip must read as 0 (fma(0, w, acc) == acc for the finite
+// weights of a sampled pixel).  Not the same operation sequence as combine() / sample_global() of tcl_math.cuh, which skip
+// such taps and start from 0 with an fma.  `v.at<DX, DY>()` loads the tap (x0 + DX, y0 + DY); `w` has the weights.
+template <typename TapLoad, typename Weights>
+__device__ __forceinline__ float tap_sum(const TapLoad& v, const Weights& w) {
+  float acc = __fmul_rn(v.template at<0, 0>(), w.nw);
+  acc = __fmaf_rn(v.template at<1, 0>(), w.ne, acc);
+  acc = __fmaf_rn(v.template at<0, 1>(), w.sw, acc);
+  acc = __fmaf_rn(v.template at<1, 1>(), w.se, acc);
+  return acc;
+}
+// tap loads of tap_sum: through a pointer to the top-left tap, rows `pitch` elements apart ...
+template <typename T>
+struct PtrTaps {
+  const T* q;
+  int pitch;
+  template <int DX, int DY> __device__ __forceinline__ float at() const { return to_f32(q[DY * pitch + DX]); }
+};
+// ... `Src`'s taps where `in` says they lie inside the image and 0 elsewhere (grid_sample's zero padding); U8: each tap
+// inside is normalised (u8_value with channel c of *n) -- a staged box holds byte 0 outside the image, which would
+// normalise to the offset
+template <typename Src, bool U8 = false>
+struct InImageTaps {
+  Src src;
+  InImage in;
+  const FrameNorm* n = nullptr;
+  int c = 0;
+  template <int DX, int DY> __device__ __forceinline__ float at() const {
+    const bool inside = DY ? (DX ? in.p11 : in.p01) : (DX ? in.p10 : in.p00);
+    if constexpr (U8) return inside ? u8_value(src.template at<DX, DY>(), *n, c) : 0.0f;
+    else return inside ? src.template at<DX, DY>() : 0.0f;
+  }
+};
+
+// source box in shared memory, origin (ox,oy), zero-filled outside the image: all four taps are plain reads
 template <typename T, int PITCH, int CH_STRIDE>
 struct SmemSrc {
   const T* base;
   int ox, oy;
   __device__ __forceinline__ float sample(int c, const PixTaps& s) const {
-    const T* q = base + c * CH_STRIDE + (s.y0 - oy) * PITCH + (s.x0 - ox);
-    float acc = __fmul_rn(to_f32(q[0]), s.nw);
-    acc = __fmaf_rn(to_f32(q[1]), s.ne, acc);
-    acc = __fmaf_rn(to_f32(q[PITCH]), s.sw, acc);
-    acc = __fmaf_rn(to_f32(q[PITCH + 1]), s.se, acc);
-    return acc;
+    return tap_sum(PtrTaps<T>{base + c * CH_STRIDE + (s.y0 - oy) * PITCH + (s.x0 - ox), PITCH}, s);
   }
 };
-
-// uint8 frames: normalised per tap; a tap outside the image contributes 0 (the box holds byte 0 there, i.e. the offset)
+// uint8 frames: normalised per tap, a tap outside the image contributes 0
 template <int PITCH, int CH_STRIDE>
 struct SmemSrc<uint8_t, PITCH, CH_STRIDE> {
   const uint8_t* base;
@@ -185,14 +220,8 @@ struct SmemSrc<uint8_t, PITCH, CH_STRIDE> {
   int W, H;
   FrameNorm n;
   __device__ __forceinline__ float sample(int c, const PixTaps& s) const {
-    const uint8_t* q = base + c * CH_STRIDE + (s.y0 - oy) * PITCH + (s.x0 - ox);
-    const bool xin0 = (unsigned)s.x0 < (unsigned)W, xin1 = (unsigned)(s.x0 + 1) < (unsigned)W;
-    const bool yin0 = (unsigned)s.y0 < (unsigned)H, yin1 = (unsigned)(s.y0 + 1) < (unsigned)H;
-    float acc = __fmul_rn(xin0 && yin0 ? u8_value((float)q[0], n, c) : 0.0f, s.nw);
-    acc = __fmaf_rn(xin1 && yin0 ? u8_value((float)q[1], n, c) : 0.0f, s.ne, acc);
-    acc = __fmaf_rn(xin0 && yin1 ? u8_value((float)q[PITCH], n, c) : 0.0f, s.sw, acc);
-    acc = __fmaf_rn(xin1 && yin1 ? u8_value((float)q[PITCH + 1], n, c) : 0.0f, s.se, acc);
-    return acc;
+    const PtrTaps<uint8_t> q{base + c * CH_STRIDE + (s.y0 - oy) * PITCH + (s.x0 - ox), PITCH};
+    return tap_sum(InImageTaps<PtrTaps<uint8_t>, true>{q, in_image(s.x0, s.y0, W, H), &n, c}, s);
   }
 };
 template <typename FrameT, int PITCH, int CH_STRIDE>
@@ -819,10 +848,7 @@ __device__ __noinline__ bool exact_keep(const float* s_bu, const float* s_ff, in
   if (!OCC) return !mob;   // the optimisation-based variant: motion-boundary test only
   const LeanTaps t = lean_taps(xf, yf, u, v, lg);
   const float* f0 = s_ff + (int)__fmaf_rn(__fsub_rn(t.fyf, box_yf), (float)BW, __fsub_rn(t.fxf, box_xf));
-  float a = __fmul_rn(f0[0], t.nw);
-  a = __fmaf_rn(f0[1], t.ne, a); a = __fmaf_rn(f0[BW], t.sw, a); a = __fmaf_rn(f0[BW + 1], t.se, a);
-  float b = __fmul_rn(f0[PL], t.nw);
-  b = __fmaf_rn(f0[PL + 1], t.ne, b); b = __fmaf_rn(f0[PL + BW], t.sw, b); b = __fmaf_rn(f0[PL + BW + 1], t.se, b);
+  const float a = tap_sum(PtrTaps<float>{f0, BW}, t), b = tap_sum(PtrTaps<float>{f0 + PL, BW}, t);
   const bool occ = occluded(a, b, u, v, nb, kV, &m2);
   return !mob && !occ;
 }
@@ -883,26 +909,51 @@ __device__ __forceinline__ float lds_tap(uint32_t a, uint8_t) {
   asm volatile("ld.shared.u8 %0, [%1+%2];" : "=r"(h) : "r"(a), "n"(OFF));
   return (float)h;
 }
-// uint8 frames: one plane of a staged box, normalised per tap; taps outside the image (q.. false: only on tiles whose box
-// crosses the border) contribute 0 -- the box holds byte 0 there, which would normalise to the offset
-template <int OFF, int PITCH>
-__device__ __forceinline__ float staged_tap4_u8(uint32_t a, const LeanTaps& tp, const FrameNorm& n, int c, bool q00, bool q10, bool q01,
-                                                bool q11) {
-  float w = __fmul_rn(q00 ? u8_value(lds_tap<OFF>(a, uint8_t()), n, c) : 0.0f, tp.nw);
-  w = __fmaf_rn(q10 ? u8_value(lds_tap<OFF + 1>(a, uint8_t()), n, c) : 0.0f, tp.ne, w);
-  w = __fmaf_rn(q01 ? u8_value(lds_tap<OFF + PITCH>(a, uint8_t()), n, c) : 0.0f, tp.sw, w);
-  w = __fmaf_rn(q11 ? u8_value(lds_tap<OFF + PITCH + 1>(a, uint8_t()), n, c) : 0.0f, tp.se, w);
-  return w;
-}
-// one plane of a staged box, grid_sampler_2d's accumulation order (zero-filled outside the image: all four taps are plain reads)
+// tap loads of tap_sum: one plane of a staged box at byte offset OFF from the top-left tap's shared address `a`
 template <typename T, int OFF, int PITCH>
-__device__ __forceinline__ float staged_tap4(uint32_t a, const LeanTaps& tp) {
-  constexpr int E = (int)sizeof(T);
-  float w = __fmul_rn(lds_tap<OFF>(a, T()), tp.nw);
-  w = __fmaf_rn(lds_tap<OFF + E>(a, T()), tp.ne, w);
-  w = __fmaf_rn(lds_tap<OFF + PITCH * E>(a, T()), tp.sw, w);
-  w = __fmaf_rn(lds_tap<OFF + PITCH * E + E>(a, T()), tp.se, w);
-  return w;
+struct LdsTaps {
+  uint32_t a;
+  template <int DX, int DY> __device__ __forceinline__ float at() const { return lds_tap<OFF + (DY * PITCH + DX) * (int)sizeof(T)>(a, T()); }
+};
+
+// this lane's column of the flow tile, shared by the staged-tile bodies: rows -1 .. 2 * P - 1 relative to the lane's first row
+// (its own pixels are the odd entries, the even ones belong to the partner lane), and the left / right neighbours of its
+// own pixels (computed masks only)
+template <int P>
+struct FlowColumn {
+  float uc[2 * P + 1], vc[2 * P + 1], ul[P], ur[P], vl[P], vr[P];
+};
+template <int MASK, typename Cfg>
+__device__ __forceinline__ FlowColumn<Cfg::kPPL> flow_column(const float* s_bu, const float* s_bv, int c0) {
+  constexpr int P = Cfg::kPPL, BFW = Cfg::kBfW;
+  FlowColumn<P> f;
+#pragma unroll
+  for (int r = 0; r < 2 * P + 1; ++r) {
+    if (MASK == MASK_COMPUTED || (r & 1)) { f.uc[r] = s_bu[c0 + (r - 1) * BFW]; f.vc[r] = s_bv[c0 + (r - 1) * BFW]; }
+    else { f.uc[r] = 0.0f; f.vc[r] = 0.0f; }
+  }
+#pragma unroll
+  for (int j = 0; j < P; ++j) {
+    if (MASK == MASK_COMPUTED) {
+      f.ul[j] = s_bu[c0 + 2 * j * BFW - 1]; f.ur[j] = s_bu[c0 + 2 * j * BFW + 1];
+      f.vl[j] = s_bv[c0 + 2 * j * BFW - 1]; f.vr[j] = s_bv[c0 + 2 * j * BFW + 1];
+    } else { f.ul[j] = f.ur[j] = f.vl[j] = f.vr[j] = 0.0f; }
+  }
+  return f;
+}
+
+// rare, divergent: mask tests too close to call (ambbits) replay the exact sequences (a few pixels per million)
+template <int MASK, bool OCC, typename Cfg>
+__device__ __forceinline__ void replay_ambiguous(const float* s_bu, const float* s_ff, int c0, float xf, float yf0, const LeanGeo& lg,
+                                                 float box_xf, float box_yf, unsigned ambbits, unsigned& keepbits) {
+  if (MASK == MASK_COMPUTED && __builtin_expect(ambbits != 0, 0)) {
+#pragma unroll
+    for (int k = 0; k < Cfg::kPPL; ++k)
+      if ((ambbits >> k) & 1u) {
+        const bool kp = exact_keep<Cfg, OCC>(s_bu, s_ff, c0 + pix_dy(k) * Cfg::kBfW, xf, yf0 + (float)pix_dy(k), lg, box_xf, box_yf);
+        keepbits = (keepbits & ~(1u << k)) | ((kp ? 1u : 0u) << k);
+      }
+  }
 }
 
 // CT == 3: masked squared error against `cur` (returned); CT == 0: mask-only (fbcCheckTorch), the verdicts go to mask_out
@@ -944,32 +995,18 @@ __device__ __forceinline__ float lean_tile(const FwdParams& p, const float* s_bu
   float wv[OUTS ? P : 1][3];
   unsigned keepbits = 0, ambbits = 0, outbits = 0;
   {
-    // this lane's column of the flow tile: rows -1 .. 2 * P - 1 relative to the lane's first row (its own pixels are the
-    // odd entries, the even ones belong to the partner lane)
-    float uc[2 * P + 1], vc[2 * P + 1], ul[P], ur[P], vl[P], vr[P];
-#pragma unroll
-    for (int r = 0; r < 2 * P + 1; ++r) {
-      if (MASK == MASK_COMPUTED || (r & 1)) { uc[r] = s_bu[c0 + (r - 1) * BFW]; vc[r] = s_bv[c0 + (r - 1) * BFW]; }
-      else { uc[r] = 0.0f; vc[r] = 0.0f; }
-    }
-#pragma unroll
-    for (int j = 0; j < P; ++j) {
-      if (MASK == MASK_COMPUTED) {
-        ul[j] = s_bu[c0 + 2 * j * BFW - 1]; ur[j] = s_bu[c0 + 2 * j * BFW + 1];
-        vl[j] = s_bv[c0 + 2 * j * BFW - 1]; vr[j] = s_bv[c0 + 2 * j * BFW + 1];
-      } else { ul[j] = ur[j] = vl[j] = vr[j] = 0.0f; }
-    }
+    const FlowColumn<P> fc = flow_column<MASK, Cfg>(s_bu, s_bv, c0);
 #pragma unroll
     for (int j = 0; j < P; ++j) {
       const int k = j, dyk = 2 * j;
       const bool inside = !EDGE || (xin && t.y0 + ly0 + dyk < p.row_end);
-      const float u = uc[2 * j + 1], v = vc[2 * j + 1];
+      const float u = fc.uc[2 * j + 1], v = fc.vc[2 * j + 1];
       const float s0 = __fmaf_rn(u, u, __fmul_rn(v, v));
       bool keep = inside, amb = false;
       if (MASK == MASK_COMPUTED) {
         // motion boundary: 4*(|grad u|^2 + |grad v|^2)  vs  4*(0.01*|bf|^2 + 0.002)
-        const float dux = __fsub_rn(ur[j], ul[j]), duy = __fsub_rn(uc[2 * j + 2], uc[2 * j]);
-        const float dvx = __fsub_rn(vr[j], vl[j]), dvy = __fsub_rn(vc[2 * j + 2], vc[2 * j]);
+        const float dux = __fsub_rn(fc.ur[j], fc.ul[j]), duy = __fsub_rn(fc.uc[2 * j + 2], fc.uc[2 * j]);
+        const float dvx = __fsub_rn(fc.vr[j], fc.vl[j]), dvy = __fsub_rn(fc.vc[2 * j + 2], fc.vc[2 * j]);
         const float G = __fmaf_rn(dux, dux, __fmaf_rn(duy, duy, __fmaf_rn(dvx, dvx, __fmul_rn(dvy, dvy))));
         const float Rhi = __fmaf_rn(4.0f * 0.01f * kHi, s0, 4.0f * 0.002f * kHi), Rlo = __fmaf_rn(4.0f * 0.01f * kLo, s0, 4.0f * 0.002f * kLo);
         const bool mob = G > Rhi;
@@ -994,36 +1031,31 @@ __device__ __forceinline__ float lean_tile(const FwdParams& p, const float* s_bu
         fa = ff_base + ((fa - ff_base) & 0xffcu);
 #endif
         if (MASK == MASK_COMPUTED && OCC) {
-          a = staged_tap4<float, 0, BW>(fa, tp);
-          b = staged_tap4<float, PL * 4, BW>(fa, tp);
+          a = tap_sum(LdsTaps<float, 0, BW>{fa}, tp);
+          b = tap_sum(LdsTaps<float, PL * 4, BW>{fa}, tp);
         }
         if constexpr (FE == 1) {
           if (CT == 3) {
             uint32_t pa = (uint32_t)__float2int_rn(__fmaf_rn(tp.fyf, (float)BW, __fmaf_rn(tp.fxf, 1.0f, prev_k)));
             if (EDGE && !inside) pa = prev_base;
-            bool q00 = true, q10 = true, q01 = true, q11 = true;
-            if (box_border) {   // (exact small integers: the placement keeps the box within |2^15|)
-              const int gx = (int)tp.fxf, gy = (int)tp.fyf;
-              const bool xin0 = (unsigned)gx < (unsigned)g.W, xin1 = (unsigned)(gx + 1) < (unsigned)g.W;
-              const bool yin0 = (unsigned)gy < (unsigned)g.H, yin1 = (unsigned)(gy + 1) < (unsigned)g.H;
-              q00 = xin0 && yin0; q10 = xin1 && yin0; q01 = xin0 && yin1; q11 = xin1 && yin1;
-            }
-            const FrameNorm& nrm = u8_norm(p);
-            w3[0] = staged_tap4_u8<0, BW>(pa, tp, nrm, 0, q00, q10, q01, q11);
-            w3[1] = staged_tap4_u8<PL, BW>(pa, tp, nrm, 1, q00, q10, q01, q11);
-            w3[2] = staged_tap4_u8<2 * PL, BW>(pa, tp, nrm, 2, q00, q10, q01, q11);
+            InImage in{true, true, true, true};
+            if (box_border) in = in_image((int)tp.fxf, (int)tp.fyf, g.W, g.H);   // (exact small integers: the placement keeps the box within |2^15|)
+            const FrameNorm* nrm = &u8_norm(p);
+            w3[0] = tap_sum(InImageTaps<LdsTaps<uint8_t, 0, BW>, true>{{pa}, in, nrm, 0}, tp);
+            w3[1] = tap_sum(InImageTaps<LdsTaps<uint8_t, PL, BW>, true>{{pa}, in, nrm, 1}, tp);
+            w3[2] = tap_sum(InImageTaps<LdsTaps<uint8_t, 2 * PL, BW>, true>{{pa}, in, nrm, 2}, tp);
           }
         } else if (CT == 3) {
           if (FE == 4) {   // fp32 frames: the prev planes sit behind the ff planes, the same address register serves them
-            w3[0] = staged_tap4<FrameT, (int)Cfg::kFfStage, BW>(fa, tp);
-            w3[1] = staged_tap4<FrameT, (int)Cfg::kFfStage + PL * FE, BW>(fa, tp);
-            w3[2] = staged_tap4<FrameT, (int)Cfg::kFfStage + 2 * PL * FE, BW>(fa, tp);
+            w3[0] = tap_sum(LdsTaps<FrameT, (int)Cfg::kFfStage, BW>{fa}, tp);
+            w3[1] = tap_sum(LdsTaps<FrameT, (int)Cfg::kFfStage + PL * FE, BW>{fa}, tp);
+            w3[2] = tap_sum(LdsTaps<FrameT, (int)Cfg::kFfStage + 2 * PL * FE, BW>{fa}, tp);
           } else {
             uint32_t pa = (uint32_t)__float2int_rn(__fmaf_rn(tp.fyf, (float)(FE * BW), __fmaf_rn(tp.fxf, (float)FE, prev_k)));
             if (EDGE && !inside) pa = prev_base;
-            w3[0] = staged_tap4<FrameT, 0, BW>(pa, tp);
-            w3[1] = staged_tap4<FrameT, PL * FE, BW>(pa, tp);
-            w3[2] = staged_tap4<FrameT, 2 * PL * FE, BW>(pa, tp);
+            w3[0] = tap_sum(LdsTaps<FrameT, 0, BW>{pa}, tp);
+            w3[1] = tap_sum(LdsTaps<FrameT, PL * FE, BW>{pa}, tp);
+            w3[2] = tap_sum(LdsTaps<FrameT, 2 * PL * FE, BW>{pa}, tp);
           }
         }
       } else {
@@ -1034,44 +1066,27 @@ __device__ __forceinline__ float lean_tile(const FwdParams& p, const float* s_bu
         const FrameT* pp = s_prev + q;
         int rs = BW;
         ptrdiff_t ps = PL, psf = PL;   // plane pitch of the frame / flow planes behind pp / pf
-        bool p00 = true, p10 = true, p01 = true, p11 = true;
+        InImage in{true, true, true, true};
         if (!inbox) {
           const int gx = (int)tp.fxf, gy = (int)tp.fyf;   // top-left tap in the image (sane: the placement checked)
           const ptrdiff_t off = (ptrdiff_t)gy * g.W + gx;
           if (MASK == MASK_COMPUTED) pf = gff + off;
           if (CT == 3) pp = gprev + off;
           rs = g.W; ps = gplane; psf = (ptrdiff_t)p.ff_plane;
-          const bool xin0 = (unsigned)gx < (unsigned)g.W, xin1 = (unsigned)(gx + 1) < (unsigned)g.W;
-          const bool yin0 = (unsigned)gy < (unsigned)g.H, yin1 = (unsigned)(gy + 1) < (unsigned)g.H;
-          p00 = xin0 && yin0; p10 = xin1 && yin0; p01 = xin0 && yin1; p11 = xin1 && yin1;
+          in = in_image(gx, gy, g.W, g.H);
         }
-        auto tap4 = [&](auto* bp) {   // one plane, grid_sampler_2d's accumulation order
-          float w = __fmul_rn(p00 ? to_f32(bp[0]) : 0.0f, tp.nw);
-          w = __fmaf_rn(p10 ? to_f32(bp[1]) : 0.0f, tp.ne, w);
-          w = __fmaf_rn(p01 ? to_f32(bp[rs]) : 0.0f, tp.sw, w);
-          w = __fmaf_rn(p11 ? to_f32(bp[rs + 1]) : 0.0f, tp.se, w);
-          return w;
-        };
-        if (MASK == MASK_COMPUTED && OCC) { a = tap4(pf); b = tap4(pf + psf); }
+        if (MASK == MASK_COMPUTED && OCC) {
+          a = tap_sum(InImageTaps<PtrTaps<float>>{{pf, rs}, in}, tp);
+          b = tap_sum(InImageTaps<PtrTaps<float>>{{pf + psf, rs}, in}, tp);
+        }
         if constexpr (FE == 1) {
           // uint8 frames: in-image predicates for the staged taps too (the box's fill is byte 0), then the normalisation
-          const int gx = (int)tp.fxf, gy = (int)tp.fyf;
-          const bool xin0 = (unsigned)gx < (unsigned)g.W, xin1 = (unsigned)(gx + 1) < (unsigned)g.W;
-          const bool yin0 = (unsigned)gy < (unsigned)g.H, yin1 = (unsigned)(gy + 1) < (unsigned)g.H;
-          const bool r00 = xin0 && yin0, r10 = xin1 && yin0, r01 = xin0 && yin1, r11 = xin1 && yin1;
-          const FrameNorm& nrm = u8_norm(p);
+          const InImage fin = in_image((int)tp.fxf, (int)tp.fyf, g.W, g.H);
 #pragma unroll
-          for (int ch = 0; ch < CT; ++ch) {
-            const FrameT* bp = pp + ch * ps;
-            float w = __fmul_rn(r00 ? u8_value((float)bp[0], nrm, ch) : 0.0f, tp.nw);
-            w = __fmaf_rn(r10 ? u8_value((float)bp[1], nrm, ch) : 0.0f, tp.ne, w);
-            w = __fmaf_rn(r01 ? u8_value((float)bp[rs], nrm, ch) : 0.0f, tp.sw, w);
-            w = __fmaf_rn(r11 ? u8_value((float)bp[rs + 1], nrm, ch) : 0.0f, tp.se, w);
-            w3[ch] = w;
-          }
+          for (int ch = 0; ch < CT; ++ch) w3[ch] = tap_sum(InImageTaps<PtrTaps<FrameT>, true>{{pp + ch * ps, rs}, fin, &u8_norm(p), ch}, tp);
         } else {
 #pragma unroll
-          for (int ch = 0; ch < CT; ++ch) w3[ch] = tap4(pp + ch * ps);
+          for (int ch = 0; ch < CT; ++ch) w3[ch] = tap_sum(InImageTaps<PtrTaps<FrameT>>{{pp + ch * ps, rs}, in}, tp);
         }
       }
       if (MASK == MASK_COMPUTED && OCC) {
@@ -1086,15 +1101,8 @@ __device__ __forceinline__ float lean_tile(const FwdParams& p, const float* s_bu
       }
       float acc = 0.0f;
       float valid = 1.0f;
-      if (MASK == MASK_NONE && validity) {   // fs_lib.warp: times the binarised warp of an all-ones image (fs_lib.py:29-37)
-        const int gx = (int)tp.fxf, gy = (int)tp.fyf;
-        Taps vt;
-        const bool xin0 = (unsigned)gx < (unsigned)g.W, xin1 = (unsigned)(gx + 1) < (unsigned)g.W;
-        const bool yin0 = (unsigned)gy < (unsigned)g.H, yin1 = (unsigned)(gy + 1) < (unsigned)g.H;
-        vt.p00 = xin0 && yin0; vt.p10 = xin1 && yin0; vt.p01 = xin0 && yin1; vt.p11 = xin1 && yin1;
-        vt.nw = tp.nw; vt.ne = tp.ne; vt.sw = tp.sw; vt.se = tp.se; vt.o00 = 0;
-        valid = binarise_validity(ones_sample(vt, kV));
-      }
+      if (MASK == MASK_NONE && validity)   // fs_lib.warp: times the binarised warp of an all-ones image (fs_lib.py:29-37)
+        valid = binarise_validity(ones_sample(full_taps(PixTaps{(int)tp.fxf, (int)tp.fyf, tp.nw, tp.ne, tp.sw, tp.se}, g), kV));
 #pragma unroll
       for (int ch = 0; ch < CT; ++ch) {
         const float w = w3[ch];
@@ -1117,14 +1125,7 @@ __device__ __forceinline__ float lean_tile(const FwdParams& p, const float* s_bu
     }
   }
   // rare, divergent: tests too close to call replay the exact sequences (a few pixels per million) ...
-  if (MASK == MASK_COMPUTED && __builtin_expect(ambbits != 0, 0)) {
-#pragma unroll
-    for (int k = 0; k < P; ++k)
-      if ((ambbits >> k) & 1u) {
-        const bool kp = exact_keep<Cfg, OCC>(s_bu, s_ff, c0 + pix_dy(k) * BFW, xf, yf0 + (float)pix_dy(k), lg, box_xf, box_yf);
-        keepbits = (keepbits & ~(1u << k)) | ((kp ? 1u : 0u) << k);
-      }
-  }
+  if constexpr (MASK == MASK_COMPUTED) replay_ambiguous<MASK, OCC, Cfg>(s_bu, s_ff, c0, xf, yf0, lg, box_xf, box_yf, ambbits, keepbits);
   // ... the same for pixels of a mixed tile whose taps left the boxes: redone from global memory
   if (MIXED && __builtin_expect(outbits != 0, 0)) {
     const size_t plane = (size_t)g.H * g.W;
@@ -1241,33 +1242,20 @@ __device__ __forceinline__ float lean_tile_packed(const FwdParams& p, const floa
   const uint32_t ff_base = smem_u32(s_ff), prev_base = smem_u32(s_prev);
   const float ff_k = __fsub_rn((float)ff_base, 4.0f * __fmaf_rn(box_yf, (float)BW, box_xf));
   const float prev_k = __fsub_rn((float)prev_base, (float)FE * __fmaf_rn(box_yf, (float)BW, box_xf));
-  // this lane's column of the flow tile (see lean_tile)
-  float uc[2 * P + 1], vc[2 * P + 1], ul[P], ur[P], vl[P], vr[P];
-#pragma unroll
-  for (int r = 0; r < 2 * P + 1; ++r) {
-    if (MASK == MASK_COMPUTED || (r & 1)) { uc[r] = s_bu[c0 + (r - 1) * BFW]; vc[r] = s_bv[c0 + (r - 1) * BFW]; }
-    else { uc[r] = 0.0f; vc[r] = 0.0f; }
-  }
-#pragma unroll
-  for (int j = 0; j < P; ++j) {
-    if (MASK == MASK_COMPUTED) {
-      ul[j] = s_bu[c0 + 2 * j * BFW - 1]; ur[j] = s_bu[c0 + 2 * j * BFW + 1];
-      vl[j] = s_bv[c0 + 2 * j * BFW - 1]; vr[j] = s_bv[c0 + 2 * j * BFW + 1];
-    } else { ul[j] = ur[j] = vl[j] = vr[j] = 0.0f; }
-  }
+  const FlowColumn<P> fc = flow_column<MASK, Cfg>(s_bu, s_bv, c0);
   float e[P];
   unsigned keepbits = 0, ambbits = 0, outbits = 0;
 #pragma unroll
   for (int q = 0; q < P / 2; ++q) {
     const int j0 = 2 * q, j1 = 2 * q + 1;   // the pair's pixels: rows ly0 + 2 * j0, ly0 + 2 * j1
-    const float2 u = f2(uc[2 * j0 + 1], uc[2 * j1 + 1]), v = f2(vc[2 * j0 + 1], vc[2 * j1 + 1]);
+    const float2 u = f2(fc.uc[2 * j0 + 1], fc.uc[2 * j1 + 1]), v = f2(fc.vc[2 * j0 + 1], fc.vc[2 * j1 + 1]);
     const float2 s0 = fma2(u, u, mul2(v, v));
     const bool in0 = !EDGE || (xin && 2 * j0 < rows_in), in1 = !EDGE || (xin && 2 * j1 < rows_in);
     bool keep0 = in0, keep1 = in1, amb0 = false, amb1 = false;
     if (MASK == MASK_COMPUTED) {
       // motion boundary: 4*(|grad u|^2 + |grad v|^2)  vs  4*(0.01*|bf|^2 + 0.002)
-      const float2 dux = sub2(f2(ur[j0], ur[j1]), f2(ul[j0], ul[j1])), duy = sub2(f2(uc[2 * j0 + 2], uc[2 * j1 + 2]), f2(uc[2 * j0], uc[2 * j1]));
-      const float2 dvx = sub2(f2(vr[j0], vr[j1]), f2(vl[j0], vl[j1])), dvy = sub2(f2(vc[2 * j0 + 2], vc[2 * j1 + 2]), f2(vc[2 * j0], vc[2 * j1]));
+      const float2 dux = sub2(f2(fc.ur[j0], fc.ur[j1]), f2(fc.ul[j0], fc.ul[j1])), duy = sub2(f2(fc.uc[2 * j0 + 2], fc.uc[2 * j1 + 2]), f2(fc.uc[2 * j0], fc.uc[2 * j1]));
+      const float2 dvx = sub2(f2(fc.vr[j0], fc.vr[j1]), f2(fc.vl[j0], fc.vl[j1])), dvy = sub2(f2(fc.vc[2 * j0 + 2], fc.vc[2 * j1 + 2]), f2(fc.vc[2 * j0], fc.vc[2 * j1]));
       const float2 G = fma2(dux, dux, fma2(duy, duy, fma2(dvx, dvx, mul2(dvy, dvy))));
       const float2 Rhi = fma2(f2(4.0f * 0.01f * kHi), s0, f2(4.0f * 0.002f * kHi)), Rlo = fma2(f2(4.0f * 0.01f * kLo), s0, f2(4.0f * 0.002f * kLo));
       const bool mob0 = G.x > Rhi.x, mob1 = G.y > Rhi.y;
@@ -1361,14 +1349,7 @@ __device__ __forceinline__ float lean_tile_packed(const FwdParams& p, const floa
     if (MIXED) outbits |= (((amb0 || !kFixInLoop) && in0 && !ok0 ? 1u : 0u) << j0) | (((amb1 || !kFixInLoop) && in1 && !ok1 ? 1u : 0u) << j1);
   }
   // rare, divergent: tests too close to call replay the exact sequences (a few pixels per million)
-  if (MASK == MASK_COMPUTED && __builtin_expect(ambbits != 0, 0)) {
-#pragma unroll
-    for (int k = 0; k < P; ++k)
-      if ((ambbits >> k) & 1u) {
-        const bool kp = exact_keep<Cfg, true>(s_bu, s_ff, c0 + pix_dy(k) * BFW, xf, yf0 + (float)pix_dy(k), lg, box_xf, box_yf);
-        keepbits = (keepbits & ~(1u << k)) | ((kp ? 1u : 0u) << k);
-      }
-  }
+  if constexpr (MASK == MASK_COMPUTED) replay_ambiguous<MASK, true, Cfg>(s_bu, s_ff, c0, xf, yf0, lg, box_xf, box_yf, ambbits, keepbits);
   // ... the same for pixels of a mixed tile whose taps left the boxes: redone from global memory
   if (MIXED && __builtin_expect(outbits != 0, 0)) {
     const size_t plane = (size_t)g.H * g.W;
@@ -1663,27 +1644,28 @@ __device__ __forceinline__ void fused_forward_ws(const Params& p, const CUtensor
 #else
     const int mode = ctl->meta[ss][2];
 #endif
-    if (LEAN == kVarMobOnly) {   // nothing staged, nothing sampled: the flow tile alone decides
-      if (t_edge) lean_tile<FrameT, MASK, CT, TCLB200_L2, Cfg, true, false, false>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
-      else lean_tile<FrameT, MASK, CT, TCLB200_L2, Cfg, false, false, false>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
-    } else if (LEAN && mode == 1) {
-      if constexpr (uses_packed(MASK, REDUCE, CT, LEAN) && sizeof(FrameT) != 1) {
-        if (t_edge) err = lean_tile_packed<FrameT, MASK, kLoss, Cfg, true, false, CT>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
-        else err = lean_tile_packed<FrameT, MASK, kLoss, Cfg, false, false, CT>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
-      } else {
-        if (t_edge) err = lean_tile<FrameT, MASK, CT, kLoss, Cfg, true, false, true, LEAN == kVarOutputs>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
-        else err = lean_tile<FrameT, MASK, CT, kLoss, Cfg, false, false, true, LEAN == kVarOutputs>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
-      }
-    } else if (LEAN == kVarOutputs) {   // outputs wanted and the tile is mixed / unstaged: the feature-complete exact path
-      err = full_tile<FrameT, MASK, REDUCE, CT, kVarGeneral, Cfg, true>(p, bf_stage(sb), ff_stage(ss), prev_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk, have_cur, near);
-    } else if (LEAN && mode == 2) {
-      if constexpr (uses_packed(MASK, REDUCE, CT, LEAN) && sizeof(FrameT) != 1) err = lean_tile_packed<FrameT, MASK, kLoss, Cfg, true, true, CT>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
-      else err = lean_tile<FrameT, MASK, CT, kLoss, Cfg, true, true>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
-    } else if (LEAN || t_edge) {
-      err = full_tile<FrameT, MASK, REDUCE, CT, LEAN, Cfg, true>(p, bf_stage(sb), ff_stage(ss), prev_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk, have_cur, near);
-    } else {
-      err = full_tile<FrameT, MASK, REDUCE, CT, LEAN, Cfg, false>(p, bf_stage(sb), ff_stage(ss), prev_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk, have_cur, near);
-    }
+    // the tile bodies with their template flags EDGE (the tile overhangs the image) and MIXED: the staged tiles of the LEAN
+    // variants take lean_tile_packed where uses_packed says so and lean_tile otherwise (kVarMobOnly: nothing staged, nothing
+    // sampled, the flow tile alone decides); every other tile takes full_tile, the exact per-pixel path of variant VAR
+    auto staged = [&](auto edge, auto mixed) -> float {
+      constexpr bool E = decltype(edge)::value, M = decltype(mixed)::value;
+      if constexpr (uses_packed(MASK, REDUCE, CT, LEAN) && sizeof(FrameT) != 1)
+        return lean_tile_packed<FrameT, MASK, kLoss, Cfg, E, M, CT>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
+      else
+        return lean_tile<FrameT, MASK, CT, kLoss, Cfg, E, M, LEAN != kVarMobOnly, LEAN == kVarOutputs && !M>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
+    };
+    auto full = [&](auto var, auto edge) -> float {
+      return full_tile<FrameT, MASK, REDUCE, CT, decltype(var)::value, Cfg, decltype(edge)::value>(p, bf_stage(sb), ff_stage(ss), prev_stage(ss), ctl->meta[ss],
+                                                                                                   t, lx0, ly0, cur, mk, have_cur, near);
+    };
+    // (kVarMobOnly tiles are mask-only, CT == 0: uses_packed is false for them, lean_tile returns 0 and nothing is reduced)
+    const std::true_type yes{};
+    const std::false_type no{};
+    const std::integral_constant<int, LEAN> var{};
+    if (LEAN == kVarMobOnly || (LEAN && mode == 1)) err = t_edge ? staged(yes, no) : staged(no, no);
+    else if (LEAN == kVarOutputs) err = full(std::integral_constant<int, kVarGeneral>(), yes);   // (outputs wanted, the tile is mixed / unstaged)
+    else if (LEAN && mode == 2) err = staged(yes, yes);
+    else err = (LEAN || t_edge) ? full(var, yes) : full(var, no);
     // <= 3 * P fp32 terms per lane; the producer folds the lanes (fixed order, fp64)
     if (REDUCE) asm volatile("st.shared.f32 [%0], %1;" ::"r"(red_s + (uint32_t)(ss * kCWarps * 128)), "f"(err) : "memory");
     __syncwarp();   // every lane is done reading the stages of tile k
