@@ -12,13 +12,14 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 LIB_PATH = os.environ.get("TCL_B200_LIB") or os.path.join(CSRC, "libtcl_b200.so")  # env override: tuning sweeps only
 HEADER = os.path.join(os.path.dirname(_HERE), "include", "tcl_b200.h")
-ABI_VERSION = 7
+ABI_VERSION = 8
 
 # enums mirrored from include/tcl_b200.h
 F32, BF16, U8 = 0, 1, 3
 OCC, MOB, VALIDITY = 1, 2, 4
 L2, L1 = 0, 1
 FIN_MEAN, FIN_RMSE = 0, 1
+CL_FRAMES, CL_FF, CL_BF = 1, 2, 4
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]
@@ -60,6 +61,7 @@ class HostArgs(ctypes.Structure):
         ("dtype", ctypes.c_int), ("flags", ctypes.c_int), ("loss", ctypes.c_int), ("finalize", ctypes.c_int),
         ("chunk_pairs", ctypes.c_int), ("frame_slots", ctypes.c_int),
         ("u8_scale", ctypes.c_float * 3), ("u8_offset", ctypes.c_float * 3),
+        ("channels_last", ctypes.c_int),
     ]
 
 
@@ -122,6 +124,7 @@ _PROTOTYPES = {
     "tclb200_fbcheck": (_c.c_int, [_vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp]),
     "tclb200_tcl_forward": (_c.c_int, [_c.POINTER(TclArgs), _vp]),
     "tclb200_host_workspace_bytes": (_c.c_size_t, [_i, _i, _i, _i, _i, _i, _i, _i]),
+    "tclb200_host_workspace_bytes_cl": (_c.c_size_t, [_i, _i, _i, _i, _i, _i, _i, _i, _i]),
     "tclb200_tcl_forward_host": (_c.c_int, [_c.POINTER(HostArgs), _vp]),
     "tclb200_tcl_backward": (_c.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "tclb200_tcl_backward_scaled": (_c.c_int, [_vp, _vp, _vp, _vp, _vp, _c.c_float, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),

@@ -22,6 +22,18 @@
 // memory for a window of frames only -- (3 + 1) chunks' worth -- not for the whole clip.  Pairs reach their frames
 // through per-pair slot indices written for each chunk.
 //
+// Channels-last host data (tclb200_host_args.channels_last): what decoders and .flo readers produce, (F,H,W,C) frames and
+// (P,H,W,2) flows, crosses PCIe unchanged (each run of consecutive frames is one contiguous block in either layout) and is
+// de-interleaved on the caller's stream right before the fused launch of its chunk:
+//   frames  chunk k's runs go into the staging area of ring slot k % 3 (on the copy stream, after the same done[] wait that
+//           frees its flow slot); the caller's stream de-interleaves them into their bank slots after ready[].  Chunk k + 3
+//           reuses the staging area after done[k % 3], which follows chunk k's conversion and launch; a bank slot is written
+//           by the caller's stream behind every launch that could still read its previous frame.
+//   flows   the ring slot receives the interleaved chunk; the caller's stream de-interleaves it into ONE planar buffer per
+//           field, which the launch reads -- the stream orders convert(k) -> launch(k) -> convert(k + 1).
+// The de-interleave permutes elements and nothing else: the fused launches see the planar bank and flows they would
+// have seen, chunk for chunk, so the results are bit for bit those of planar inputs.
+//
 // The copy stream and the events are kept in a per-device pool and reused by later calls (creating a stream and seven
 // events costs more than a small job).  On any failure the function drains both streams before it returns, so the
 // caller may free or reuse its host buffers as soon as it sees the error.
@@ -46,14 +58,17 @@ constexpr int kMaxDefaultChunk = 128;
 
 inline size_t up256(size_t v) { return (v + 255) & ~(size_t)255; }
 
+constexpr int kClAll = TCLB200_CL_FRAMES | TCLB200_CL_FF | TCLB200_CL_BF;
+
 struct Layout {
-  size_t frames, flows[kRing][2], mask[kRing], prev_idx, cur_idx, vals, sums, scratch, total;
+  size_t frames, flows[kRing][2], mask[kRing], prev_idx, cur_idx, vals, sums, scratch;
+  size_t stage[kRing], planar[2], total;   // channels-last only (empty otherwise): frame staging per ring slot, planar ff / bf
   size_t frame_bytes, flow_bytes, mask_bytes;
   int chunk;
 };
 
-// F = device frame slots provisioned
-Layout make_layout(int P, int F, int C, int H, int W, int dtype, int chunk_pairs, bool with_mask) {
+// F = device frame slots provisioned; cl = TCLB200_CL_* bits
+Layout make_layout(int P, int F, int C, int H, int W, int dtype, int chunk_pairs, bool with_mask, int cl) {
   Layout L;
   memset(&L, 0, sizeof(L));
   const size_t px = (size_t)H * W;
@@ -81,6 +96,13 @@ Layout make_layout(int P, int F, int C, int H, int W, int dtype, int chunk_pairs
   L.vals = o; o += up256(sizeof(float) * (size_t)P);
   L.sums = o; o += up256(sizeof(double) * (size_t)P);
   L.scratch = o; o += up256(tclb200_scratch_bytes(L.chunk, H, W));
+  // a chunk of n pairs uploads at most 2n frames, and never more than there are slots
+  const size_t stage_frames = (cl & TCLB200_CL_FRAMES) ? (size_t)(F < 2 * L.chunk ? F : 2 * L.chunk) : 0;
+  for (int r = 0; r < kRing; ++r) { L.stage[r] = o; o += up256(L.frame_bytes * stage_frames); }
+  for (int j = 0; j < 2; ++j) {
+    L.planar[j] = o;
+    if (cl & (j == 0 ? TCLB200_CL_FF : TCLB200_CL_BF)) o += up256(L.flow_bytes * (size_t)L.chunk);
+  }
   L.total = o;
   return L;
 }
@@ -144,11 +166,74 @@ void release_pipe(Pipe* p) {
   g_pool.push_back(p);
 }
 
+// (N,H,W,C) -> (N,C,H,W) for 1- and 2-byte elements (uint8 frames; bf16 frames as their bit patterns): hwc_split_kernel's
+// scheme.  A CTA reads the interleaved elements of kDeintPx consecutive pixels of one frame as one contiguous, coalesced
+// run into shared memory (one word per element, pitch C | 1: conflict-free for any C), then writes each channel as a
+// coalesced run of its plane.  Element-wise accesses: any H, W and any start address work (staged runs start wherever the
+// previous run ended).
+constexpr int kDeintPx = 256;
+constexpr int kDeintMaxC = 64;
+
+template <typename T>
+__global__ void __launch_bounds__(kDeintPx) hwc_to_chw_kernel(const T* __restrict__ src, T* __restrict__ dst, int C,
+                                                               long long plane, int chunks_per_frame) {
+  extern __shared__ uint32_t s_el[];
+  const int pitch = C | 1;
+  const int n = blockIdx.x / chunks_per_frame;
+  const long long px0 = (long long)(blockIdx.x - n * chunks_per_frame) * kDeintPx;
+  const int npx = (int)min((long long)kDeintPx, plane - px0);
+  const T* s = src + ((long long)n * plane + px0) * C;
+  const int nel = npx * C;
+  for (int i = threadIdx.x; i < nel; i += kDeintPx) {
+    const int px = i / C, c = i - px * C;
+    s_el[px * pitch + c] = __ldcs(s + i);
+  }
+  __syncthreads();
+  const int t = threadIdx.x;
+  if (t >= npx) return;
+  T* d = dst + (long long)n * C * plane + px0 + t;
+  for (int c = 0; c < C; ++c) __stcs(d + (long long)c * plane, (T)s_el[t * pitch + c]);
+}
+
+// N frames (N,H,W,C) of `dtype` at src -> N planar frames (N,C,H,W) at dst, on `s`.  fp32 goes through tclb200_hwc_split.
+int frames_to_planar(const void* src, void* dst, int N, int C, int H, int W, int dtype, cudaStream_t s) {
+  if (dtype == TCLB200_F32) {
+    float* d = reinterpret_cast<float*>(dst);
+    const int c0 = 0;
+    return tclb200_hwc_split(reinterpret_cast<const float*>(src), N, H, W, C, 1, &d, &c0, &C, s);
+  }
+  const long long plane = (long long)H * W, chunks = (plane + kDeintPx - 1) / kDeintPx;
+  if (chunks * N >= 0x7fffffffLL) return hfail(TCLB200_ERR_UNSUPPORTED, "channels-last frames: too many pixels for one launch");
+  const size_t smem = (size_t)kDeintPx * (C | 1) * sizeof(uint32_t);
+  const dim3 grid((unsigned)(chunks * N));
+  cudaError_t e;
+  if (dtype == TCLB200_U8) {
+    if (smem > 48 * 1024 &&
+        (e = cudaFuncSetAttribute(hwc_to_chw_kernel<uint8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess)
+      return hfail(TCLB200_ERR_CUDA, "channels-last frames: ", cudaGetErrorString(e));
+    hwc_to_chw_kernel<uint8_t><<<grid, kDeintPx, smem, s>>>(reinterpret_cast<const uint8_t*>(src), reinterpret_cast<uint8_t*>(dst),
+                                                             C, plane, (int)chunks);
+  } else {
+    if (smem > 48 * 1024 &&
+        (e = cudaFuncSetAttribute(hwc_to_chw_kernel<uint16_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess)
+      return hfail(TCLB200_ERR_CUDA, "channels-last frames: ", cudaGetErrorString(e));
+    hwc_to_chw_kernel<uint16_t><<<grid, kDeintPx, smem, s>>>(reinterpret_cast<const uint16_t*>(src), reinterpret_cast<uint16_t*>(dst),
+                                                              C, plane, (int)chunks);
+  }
+  if ((e = cudaGetLastError()) != cudaSuccess) return hfail(TCLB200_ERR_CUDA, "channels-last frames: ", cudaGetErrorString(e));
+  return TCLB200_OK;
+}
+
 }  // namespace
 
 extern "C" size_t tclb200_host_workspace_bytes(int P, int F, int C, int H, int W, int dtype, int chunk_pairs, int with_mask) {
-  if (P <= 0 || F <= 0 || C <= 0 || H <= 0 || W <= 0) return 0;
-  return make_layout(P, F, C, H, W, dtype, chunk_pairs, with_mask != 0).total;
+  return tclb200_host_workspace_bytes_cl(P, F, C, H, W, dtype, chunk_pairs, with_mask, 0);
+}
+
+extern "C" size_t tclb200_host_workspace_bytes_cl(int P, int F, int C, int H, int W, int dtype, int chunk_pairs, int with_mask,
+                                                  int channels_last) {
+  if (P <= 0 || F <= 0 || C <= 0 || H <= 0 || W <= 0 || (channels_last & ~kClAll)) return 0;
+  return make_layout(P, F, C, H, W, dtype, chunk_pairs, with_mask != 0, channels_last).total;
 }
 
 // on failure: drain both streams (the caller may free its host buffers when it sees the error), give the pipe back
@@ -160,6 +245,7 @@ extern "C" size_t tclb200_host_workspace_bytes(int P, int F, int C, int H, int W
 
 extern "C" int tclb200_tcl_forward_host(const tclb200_host_args* a, tclb200_stream_t stream) {
   if (!a) return hfail(TCLB200_ERR_INVALID, "args is NULL");
+  if (a->channels_last & ~kClAll) return hfail(TCLB200_ERR_INVALID, "channels_last: unknown bits (TCLB200_CL_FRAMES | TCLB200_CL_FF | TCLB200_CL_BF)");
   if (a->P < 0 || a->F < 0) return hfail(TCLB200_ERR_INVALID, "P and F must not be negative");
   if (a->P == 0) return TCLB200_OK;   // a clip of one frame has no pairs: nothing to do, nothing to return
   if (a->F <= 0 || a->C <= 0 || a->H <= 0 || a->W <= 0) return hfail(TCLB200_ERR_INVALID, "F, C, H, W must be positive");
@@ -172,13 +258,16 @@ extern "C" int tclb200_tcl_forward_host(const tclb200_host_args* a, tclb200_stre
       if (!isfinite(a->u8_scale[c]) || !isfinite(a->u8_offset[c])) return hfail(TCLB200_ERR_INVALID, "uint8 frames: u8_scale / u8_offset must be finite");
   }
   if (a->frame_slots < 0) return hfail(TCLB200_ERR_INVALID, "frame_slots must not be negative");
+  const int cl = a->channels_last;
+  if ((cl & TCLB200_CL_FF) && !a->ff) return hfail(TCLB200_ERR_INVALID, "TCLB200_CL_FF without ff");
+  if ((cl & TCLB200_CL_FRAMES) && a->C > kDeintMaxC) return hfail(TCLB200_ERR_UNSUPPORTED, "channels-last frames: at most 64 channels");
   for (int p = 0; p < a->P; ++p)
     if (a->prev_index[p] < 0 || a->prev_index[p] >= a->F || a->cur_index[p] < 0 || a->cur_index[p] >= a->F)
       return hfail(TCLB200_ERR_INVALID, "prev_index / cur_index outside [0, F)");
   const bool with_mask = !a->ff && a->mask_in;
   const int S = (a->frame_slots > 0 && a->frame_slots < a->F) ? a->frame_slots : a->F;   // device frame slots
-  const Layout L = make_layout(a->P, S, a->C, a->H, a->W, a->dtype, a->chunk_pairs, with_mask);
-  if (!a->workspace || a->workspace_bytes < L.total) return hfail(TCLB200_ERR_INVALID, "workspace missing or smaller than tclb200_host_workspace_bytes()");
+  const Layout L = make_layout(a->P, S, a->C, a->H, a->W, a->dtype, a->chunk_pairs, with_mask, cl);
+  if (!a->workspace || a->workspace_bytes < L.total) return hfail(TCLB200_ERR_INVALID, "workspace missing or smaller than tclb200_host_workspace_bytes_cl()");
   if ((reinterpret_cast<uintptr_t>(a->workspace) & 255u) != 0) return hfail(TCLB200_ERR_INVALID, "workspace must be 256-byte aligned");
 
   cudaStream_t comp = reinterpret_cast<cudaStream_t>(stream);
@@ -254,19 +343,41 @@ extern "C" int tclb200_tcl_forward_host(const tclb200_host_args* a, tclb200_stre
     const int slot = k % kRing;
     cudaStream_t cs = pipe->copy[k & 1];
     if (k >= kRing) HOST_TRY(cudaStreamWaitEvent(cs, pipe->done[slot], 0));   // chunk k - kRing has been consumed: its flow slot and the frame slots released with it are free
-    for (const Run& r : uploads[(size_t)k])
-      HOST_TRY(cudaMemcpyAsync(ws + L.frames + (size_t)r.slot * L.frame_bytes, h_frames + (size_t)r.frame * L.frame_bytes,
-                               (size_t)r.count * L.frame_bytes, cudaMemcpyHostToDevice, cs));
+    size_t staged = 0;   // channels-last frames: runs go one after another into the slot's staging area
+    for (const Run& r : uploads[(size_t)k]) {
+      char* dst = (cl & TCLB200_CL_FRAMES) ? ws + L.stage[slot] + staged : ws + L.frames + (size_t)r.slot * L.frame_bytes;
+      HOST_TRY(cudaMemcpyAsync(dst, h_frames + (size_t)r.frame * L.frame_bytes, (size_t)r.count * L.frame_bytes, cudaMemcpyHostToDevice, cs));
+      staged += (size_t)r.count * L.frame_bytes;
+    }
     if (a->ff) HOST_TRY(cudaMemcpyAsync(ws + L.flows[slot][0], a->ff + (size_t)s * 2 * a->H * a->W, (size_t)n * L.flow_bytes, cudaMemcpyHostToDevice, cs));
     HOST_TRY(cudaMemcpyAsync(ws + L.flows[slot][1], a->bf + (size_t)s * 2 * a->H * a->W, (size_t)n * L.flow_bytes, cudaMemcpyHostToDevice, cs));
     if (with_mask) HOST_TRY(cudaMemcpyAsync(ws + L.mask[slot], a->mask_in + (size_t)s * a->H * a->W, (size_t)n * L.mask_bytes, cudaMemcpyHostToDevice, cs));
     HOST_TRY(cudaEventRecord(pipe->ready[slot], cs));
     HOST_TRY(cudaStreamWaitEvent(comp, pipe->ready[slot], 0));
 
+    if (cl & TCLB200_CL_FRAMES) {
+      staged = 0;
+      for (const Run& r : uploads[(size_t)k]) {
+        const int rc = frames_to_planar(ws + L.stage[slot] + staged, ws + L.frames + (size_t)r.slot * L.frame_bytes, r.count, a->C,
+                                        a->H, a->W, a->dtype, comp);
+        if (rc != TCLB200_OK) return bail(rc);
+        staged += (size_t)r.count * L.frame_bytes;
+      }
+    }
+    const float* flow[2] = {reinterpret_cast<const float*>(ws + L.flows[slot][0]), reinterpret_cast<const float*>(ws + L.flows[slot][1])};
+    for (int j = 0; j < 2; ++j)
+      if (cl & (j == 0 ? TCLB200_CL_FF : TCLB200_CL_BF)) {
+        float* planar = reinterpret_cast<float*>(ws + L.planar[j]);
+        const int c0 = 0, cd = 2;
+        const int rc = tclb200_hwc_split(flow[j], n, a->H, a->W, 2, 1, &planar, &c0, &cd, stream);
+        if (rc != TCLB200_OK) return bail(rc);
+        flow[j] = planar;
+      }
+
     tclb200_tcl_args t;
     memset(&t, 0, sizeof(t));
-    t.ff = a->ff ? reinterpret_cast<const float*>(ws + L.flows[slot][0]) : nullptr;
-    t.bf = reinterpret_cast<const float*>(ws + L.flows[slot][1]);
+    t.ff = a->ff ? flow[0] : nullptr;
+    t.bf = flow[1];
     t.mask_in = with_mask ? reinterpret_cast<const float*>(ws + L.mask[slot]) : nullptr;
     t.prev = ws + L.frames; t.cur = ws + L.frames;
     t.prev_index = reinterpret_cast<const int*>(ws + L.prev_idx) + s;

@@ -499,13 +499,24 @@ def free_workspaces():
     _loss_plans.clear()
 
 
-def _host_tensor(t, name, dtype=None):
+def _is_channels_last(t):
+    """True for an (N,C,H,W) tensor that is a permuted view of (N,H,W,C) memory -- what a decoder's or a .flo reader's
+    interleaved array becomes after ``.permute(0, 3, 1, 2)``.  Where the two layouts coincide (C == 1, H*W == 1) it is
+    planar."""
+    return t.dim() == 4 and t.is_contiguous(memory_format=torch.channels_last) and not t.is_contiguous()
+
+
+def _host_tensor(t, name, dtype=None, channels_last_ok=False):
+    """``t`` on the host, of ``dtype``, planar -- or as it is when ``channels_last_ok`` and it is channels-last (the host
+    entry de-interleaves such data on the device)."""
     if t is None:
         return None
     if t.is_cuda:
         raise RuntimeError(f"tcl_b200: {name} must be a host (CPU) tensor for the host-buffer entry")
     if dtype is not None and t.dtype != dtype:
         t = t.to(dtype)
+    if channels_last_ok and _is_channels_last(t):
+        return t
     return t.contiguous()
 
 
@@ -519,6 +530,10 @@ def temporal_error_host(frames, ff, bf, prev_index=None, cur_index=None, mask=No
     (P,2,H,W) fp32; pair p warps ``frames[prev_index[p]]`` by ``bf[p]`` and compares with ``frames[cur_index[p]]``
     under the mask of (``ff[p]``, ``bf[p]``) -- or under ``mask[p]`` (P,1,H,W) when ``ff`` is None
     (utils/metrics/eval.py:137-138).  Default indices: the consecutive pairs of ONE clip (P = F-1).
+    ``frames``, ``ff`` and ``bf`` may be channels-last views of interleaved memory -- ``(F,H,W,C)`` decoded frames or
+    ``(P,H,W,2)`` ``.flo`` payloads after ``.permute(0, 3, 1, 2)``: they are read in place, cross PCIe as they are and are
+    de-interleaved on the GPU, with results bit for bit those of planar copies (frames of more than 64 channels are
+    still made contiguous on the host).
     All tensors are CPU tensors (pinned memory runs at PCIe speed); the result is a pinned CPU tensor (P,) of per-pair
     values per ``finalize``.  One C-ABI call (``tclb200_tcl_forward_host``) pipelines H2D copies and fused launches
     on ``device`` (default: the current CUDA device); there is no CPU arithmetic anywhere.
@@ -530,10 +545,10 @@ def temporal_error_host(frames, ff, bf, prev_index=None, cur_index=None, mask=No
     """
     if not torch.cuda.is_available():
         raise RuntimeError("tcl_b200: temporal_error_host needs a CUDA device; this path has no CPU implementation")
-    frames = _host_tensor(frames, "frames")
+    frames = _host_tensor(frames, "frames", channels_last_ok=frames.dim() == 4 and frames.shape[1] <= 64)
     dt = _eval_frame_dtype(frames)
-    bf = _host_tensor(bf, "bf", torch.float32)
-    ff = _host_tensor(ff, "ff", torch.float32)
+    bf = _host_tensor(bf, "bf", torch.float32, channels_last_ok=True)
+    ff = _host_tensor(ff, "ff", torch.float32, channels_last_ok=True)
     mask = _host_tensor(mask, "mask", torch.float32) if ff is None else None
     if frames.dim() != 4 or bf.dim() != 4 or bf.shape[1] != 2 or bf.shape[2:] != frames.shape[2:]:
         raise RuntimeError(f"tcl_b200: frames {tuple(frames.shape)} / bf {tuple(bf.shape)} must be (F,C,H,W) / (P,2,H,W)")
@@ -558,19 +573,25 @@ def temporal_error_host(frames, ff, bf, prev_index=None, cur_index=None, mask=No
     if P == 0:
         out = torch.empty(0, dtype=torch.float32, pin_memory=True)
         return (out, torch.empty(0, dtype=torch.float64, pin_memory=True)) if return_sums else out
+    cl = ((_cabi.CL_FRAMES if _is_channels_last(frames) else 0) | (_cabi.CL_FF if ff is not None and _is_channels_last(ff) else 0)
+          | (_cabi.CL_BF if _is_channels_last(bf) else 0))
     slots = F_
     ws = _host_ws_cache.get(dev.index)
     with_mask = 1 if mask is not None else 0
     if max_device_frames is not None:
         slots = max(1, min(F_, int(max_device_frames)))
-    elif ws is None or ws.numel() < lib.tclb200_host_workspace_bytes(P, F_, C, H, W, dt, chunk_pairs, with_mask):
+    elif ws is None or ws.numel() < lib.tclb200_host_workspace_bytes_cl(P, F_, C, H, W, dt, chunk_pairs, with_mask, cl):
         # only when a workspace has to be allocated: cudaMemGetInfo costs 1.5 ms at the median and 20-90 ms in one call of ten
         # (measured, tools/e2e_stall_probe.py) -- per step it was the whole difference between a 6 ms step and a 12 ms one
         frame_bytes = C * H * W * frames.element_size()
         free_b = torch.cuda.mem_get_info(dev)[0] + (ws.numel() if ws is not None else 0)
-        if F_ * frame_bytes > free_b // 4:
-            slots = max(1, min(F_, (free_b // 4) // frame_bytes))
-    need = lib.tclb200_host_workspace_bytes(P, slots, C, H, W, dt, chunk_pairs, with_mask)
+        # channels-last data also needs its staging areas and planar flow buffers; with a whole bank they are at their
+        # largest, so a ring sized against them fits too
+        extra = (lib.tclb200_host_workspace_bytes_cl(P, F_, C, H, W, dt, chunk_pairs, with_mask, cl)
+                 - lib.tclb200_host_workspace_bytes(P, F_, C, H, W, dt, chunk_pairs, with_mask))
+        if F_ * frame_bytes + extra > free_b // 4:
+            slots = max(1, min(F_, (free_b // 4 - extra) // frame_bytes))
+    need = lib.tclb200_host_workspace_bytes_cl(P, slots, C, H, W, dt, chunk_pairs, with_mask, cl)
     if ws is None or ws.numel() < need:
         _host_ws_cache.pop(dev.index, None)
         ws = torch.empty(need, dtype=torch.uint8, device=dev)
@@ -586,6 +607,7 @@ def temporal_error_host(frames, ff, bf, prev_index=None, cur_index=None, mask=No
     a.dtype, a.flags, a.loss, a.finalize, a.chunk_pairs = dt, flags, loss, finalize, chunk_pairs
     a.frame_slots = 0 if slots >= F_ else slots
     a.u8_scale[:], a.u8_offset[:] = norm
+    a.channels_last = cl
     with torch.cuda.device(dev):
         stream = torch.cuda.current_stream()
         check(lib.tclb200_tcl_forward_host(ctypes.byref(a), ctypes.c_void_p(stream.cuda_stream)))

@@ -11,7 +11,8 @@
  * boundary: plain device pointers owned by the caller, explicit sizes, an explicit cudaStream_t.
  *
  * Conventions
- *   - all tensors NCHW contiguous; flows are (B,2,H,W) fp32 in pixels, channel 0 = u (x), 1 = v (y);
+ *   - all tensors NCHW contiguous (the host-buffer entry also reads channels-last host arrays, see
+ *     tclb200_host_args.channels_last); flows are (B,2,H,W) fp32 in pixels, channel 0 = u (x), 1 = v (y);
  *     frames are (B,C,H,W) fp32 or bf16 (TCLB200_F32 / TCLB200_BF16); masks are (B,1,H,W) fp32 in {0,1};
  *     the evaluation entries (reductions of tclb200_tcl_forward, tclb200_tcl_forward_host) also score stored 8-bit video:
  *     (B,3,H,W) uint8 frames (TCLB200_U8) with a per-channel normalisation, see tclb200_tcl_args.u8_scale
@@ -31,7 +32,7 @@
 extern "C" {
 #endif
 
-#define TCLB200_ABI_VERSION 7
+#define TCLB200_ABI_VERSION 8
 
 #define TCLB200_OK 0
 #define TCLB200_ERR_INVALID 1     /* bad argument (null pointer, non-positive size, unknown enum) */
@@ -183,7 +184,12 @@ int tclb200_tcl_forward(const tclb200_tcl_args* args, tclb200_stream_t stream);
  * not on the device yet (each frame of the bank crosses PCIe once), H2D of its flows into a 3-slot ring on an internal
  * copy stream, one fused launch (clip mode of tclb200_tcl_forward) per chunk on `stream`, one D2H of the per-pair
  * results at the end -- and returns; pair_vals / pair_sums are valid once `stream` has been synchronised, and the host
- * inputs must stay untouched until then. */
+ * inputs must stay untouched until then.
+ * Channels-last host data (ABI v8): decoders and .flo readers hand over interleaved arrays -- (F,H,W,C) frames, (P,H,W,2)
+ * flows.  The bits of `channels_last` say which of frames / ff / bf are stored that way; the bytes cross PCIe unchanged
+ * and are de-interleaved on the device, on `stream` right before the fused launch of their chunk: frame runs through a
+ * staging area per ring slot into their planar bank slots, flows into one planar buffer per field.  The de-interleave is
+ * a permutation of elements, so the results are bit for bit those of the same call on planar copies. */
 typedef struct tclb200_host_args {
   const float* ff;       /* (P,2,H,W) forward flows, or NULL (then mask_in or no mask) */
   const float* bf;       /* (P,2,H,W) flows the warp samples with; required */
@@ -204,11 +210,25 @@ typedef struct tclb200_host_args {
   /* dtype TCLB200_U8 (ABI v7): as in tclb200_tcl_args.  Each frame crosses PCIe once at 3 B/px instead of 12 (fp32) */
   float u8_scale[3];
   float u8_offset[3];
+  /* layout of the host arrays (ABI v8): 0 = all planar, else TCLB200_CL_* bits.  TCLB200_CL_FRAMES: `frames` is (F,H,W,C)
+   * (C <= 64); TCLB200_CL_FF / TCLB200_CL_BF: that flow is (P,H,W,2) (TCLB200_CL_FF needs `ff`).  Unknown bits are
+   * TCLB200_ERR_INVALID.  The workspace must be sized by tclb200_host_workspace_bytes_cl with the same bits. */
+  int channels_last;
 } tclb200_host_args;
+
+#define TCLB200_CL_FRAMES 1
+#define TCLB200_CL_FF 2
+#define TCLB200_CL_BF 4
 
 /* F here = the number of device frame slots to provision (tclb200_host_args.frame_slots, or the clip's F for a resident bank);
  * the frame bank takes C*H*W elements of `dtype` per slot (1 byte each for TCLB200_U8) */
 size_t tclb200_host_workspace_bytes(int P, int F, int C, int H, int W, int dtype, int chunk_pairs, int with_mask);
+/* the same for channels-last host data (ABI v8): `channels_last` as in tclb200_host_args (0 gives exactly
+ * tclb200_host_workspace_bytes).  TCLB200_CL_FRAMES adds a staging area of min(F, 2 * chunk) frames to each of the three
+ * ring slots; TCLB200_CL_FF and TCLB200_CL_BF each add one planar flow buffer of `chunk` fields (chunk: the pairs per
+ * launch, chunk_pairs or its default, at most P).  Every part is rounded up to 256 bytes.  0 for unknown bits. */
+size_t tclb200_host_workspace_bytes_cl(int P, int F, int C, int H, int W, int dtype, int chunk_pairs, int with_mask,
+                                       int channels_last);
 int tclb200_tcl_forward_host(const tclb200_host_args* args, tclb200_stream_t stream);
 
 /* Backward of the fused training loss  L = grad_scale * sum (m*(cur-warp(prev,bf)))^2   (L2)
