@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 LIB_PATH = os.environ.get("TCL_B200_LIB") or os.path.join(CSRC, "libtcl_b200.so")  # env override: tuning sweeps only
 HEADER = os.path.join(os.path.dirname(_HERE), "include", "tcl_b200.h")
-ABI_VERSION = 8
+ABI_VERSION = 9
 
 # enums mirrored from include/tcl_b200.h
 F32, BF16, U8 = 0, 1, 3
@@ -47,6 +47,7 @@ class TclArgs(ctypes.Structure):
         ("n_bf_fields", ctypes.c_int), ("n_ff_fields", ctypes.c_int), ("pair_group", ctypes.c_int),
         ("row_begin", ctypes.c_int), ("row_end", ctypes.c_int),
         ("u8_scale", ctypes.c_float * 3), ("u8_offset", ctypes.c_float * 3),
+        ("pair_kept", ctypes.c_void_p), ("total_kept", ctypes.c_void_p),
     ]
 
 
@@ -62,6 +63,7 @@ class HostArgs(ctypes.Structure):
         ("chunk_pairs", ctypes.c_int), ("frame_slots", ctypes.c_int),
         ("u8_scale", ctypes.c_float * 3), ("u8_offset", ctypes.c_float * 3),
         ("channels_last", ctypes.c_int),
+        ("pair_kept", ctypes.c_void_p),
     ]
 
 
@@ -117,6 +119,7 @@ _PROTOTYPES = {
     "tclb200_last_error": (_c.c_char_p, []),
     "tclb200_build_info": (_c.c_char_p, []),
     "tclb200_scratch_bytes": (_c.c_size_t, [_i, _i, _i]),
+    "tclb200_scratch_bytes_kept": (_c.c_size_t, [_i, _i, _i]),
     "tclb200_gradient": (_c.c_int, [_vp, _vp, _i, _i, _i, _vp]),
     "tclb200_gradient_strided": (_c.c_int, [_vp, _c.c_size_t, _vp, _i, _i, _i, _vp]),
     "tclb200_warp": (_c.c_int, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
@@ -125,6 +128,7 @@ _PROTOTYPES = {
     "tclb200_tcl_forward": (_c.c_int, [_c.POINTER(TclArgs), _vp]),
     "tclb200_host_workspace_bytes": (_c.c_size_t, [_i, _i, _i, _i, _i, _i, _i, _i]),
     "tclb200_host_workspace_bytes_cl": (_c.c_size_t, [_i, _i, _i, _i, _i, _i, _i, _i, _i]),
+    "tclb200_host_workspace_bytes_kept": (_c.c_size_t, [_i, _i, _i, _i, _i, _i, _i, _i, _i]),
     "tclb200_tcl_forward_host": (_c.c_int, [_c.POINTER(HostArgs), _vp]),
     "tclb200_tcl_backward": (_c.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "tclb200_tcl_backward_scaled": (_c.c_int, [_vp, _vp, _vp, _vp, _vp, _c.c_float, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),

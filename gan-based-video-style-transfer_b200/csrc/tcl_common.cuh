@@ -123,6 +123,16 @@ struct FwdParamsU8 : FwdParams {
 };
 __device__ __forceinline__ const FrameNorm& u8_norm(const FwdParams& p) { return static_cast<const FwdParamsU8&>(p).norm; }
 
+// Kept-pixel sums (tclb200_tcl_args.pair_kept / total_kept, ABI v9): a separate kernel parameter of the kernels that compute
+// them, so that FwdParams -- and the parameter offsets and instructions of every other kernel -- stay as they are.  The
+// partials lie behind the scratch of tclb200_scratch_bytes (tclb200_scratch_bytes_kept sizes both), one per tile like
+// scratch.partials, and are all zero between launches too.
+struct KeptOut {
+  double* partials;
+  double* pair_kept;   // [B] or nullptr
+  double* total_kept;  // [1] or nullptr
+};
+
 __device__ __forceinline__ float finalise_value(double mean, int finalize) {
   return (float)(finalize == TCLB200_FIN_RMSE ? sqrt(mean) : mean);
 }
@@ -131,13 +141,19 @@ __device__ __forceinline__ float finalise_value(double mean, int finalize) {
 // the last CTA of a pair folds that pair's partials in index order, the last pair folds the batch in index
 // order: results do not depend on CTA scheduling (deterministic).  Consumed slots are re-zeroed, so the
 // scratch is all-zero again when the launch retires, whatever (B,H,W) the next call uses.
-__device__ __forceinline__ void reduce_and_finalise(float err, const FwdParams& p, int pair, int tile) {
+// KEPT: `kept` (this thread's kept-pixel sum) goes the same way through k->partials into k->pair_kept / k->total_kept.
+template <bool KEPT = false>
+__device__ __forceinline__ void reduce_and_finalise(float err, const FwdParams& p, int pair, int tile, float kept = 0.0f,
+                                                    const KeptOut* k = nullptr) {
   __shared__ double red[kWarps];
   __shared__ int s_last;
   const double bsum = block_sum((double)err, red);
+  double ksum = 0.0;
+  if constexpr (KEPT) ksum = block_sum((double)kept, red);
   const unsigned tpp = p.tiles_per_pair;
   if (threadIdx.x == 0) {
     __stcg(&p.scratch.partials[(size_t)pair * tpp + tile], bsum);
+    if constexpr (KEPT) __stcg(&k->partials[(size_t)pair * tpp + tile], ksum);
     __threadfence();
     const unsigned tk = atomicAdd(&p.scratch.pair_ticket[pair], 1u);
     s_last = (tk == tpp - 1);
@@ -145,17 +161,28 @@ __device__ __forceinline__ void reduce_and_finalise(float err, const FwdParams& 
   __syncthreads();
   if (!s_last) return;
   __threadfence();
-  double s = 0.0;
+  double s = 0.0, ks = 0.0;
   double* pp = p.scratch.partials + (size_t)pair * tpp;
+  double* kp = KEPT ? k->partials + (size_t)pair * tpp : nullptr;
   for (unsigned i = threadIdx.x; i < tpp; i += kThreads) {
     s += __ldcg(pp + i);
     __stcg(pp + i, 0.0);
+    if constexpr (KEPT) {
+      ks += __ldcg(kp + i);
+      __stcg(kp + i, 0.0);
+    }
   }
   const double S = block_sum(s, red);
+  double KS = 0.0;
+  if constexpr (KEPT) KS = block_sum(ks, red);
   if (threadIdx.x == 0) {
     if (p.pair_sums) p.pair_sums[pair] = S;
     if (p.pair_vals) p.pair_vals[pair] = finalise_value(S * p.inv_count, p.finalize);
     __stcg(pp, S);  // this pair's record for the batch fold
+    if constexpr (KEPT) {
+      if (k->pair_kept) k->pair_kept[pair] = KS;
+      __stcg(kp, KS);
+    }
     p.scratch.pair_ticket[pair] = 0;
     __threadfence();
     const unsigned tk = atomicAdd(p.scratch.batch_ticket, 1u);
@@ -164,19 +191,27 @@ __device__ __forceinline__ void reduce_and_finalise(float err, const FwdParams& 
   __syncthreads();
   if (s_last != 2) return;
   __threadfence();
-  double a = 0.0, b = 0.0;
+  double a = 0.0, b = 0.0, c = 0.0;
   for (int i = threadIdx.x; i < p.B; i += kThreads) {
     double* rec = p.scratch.partials + (size_t)i * tpp;
     const double Si = __ldcg(rec);
     __stcg(rec, 0.0);
     a += Si;
     b += (double)finalise_value(Si * p.inv_count, p.finalize);
+    if constexpr (KEPT) {
+      c += __ldcg(k->partials + (size_t)i * tpp);
+      __stcg(k->partials + (size_t)i * tpp, 0.0);
+    }
   }
   const double A = block_sum(a, red);
   const double Bv = block_sum(b, red);
+  double Cv = 0.0;
+  if constexpr (KEPT) Cv = block_sum(c, red);
   if (threadIdx.x == 0) {
     if (p.total_sums) { p.total_sums[0] = A; p.total_sums[1] = Bv; }
     if (p.total_val) *p.total_val = finalise_value(A * p.inv_count / (double)p.B, p.finalize);
+    if constexpr (KEPT)
+      if (k->total_kept) *k->total_kept = Cv;
     *p.scratch.batch_ticket = 0;
   }
 }

@@ -37,6 +37,9 @@
 // The copy stream and the events are kept in a per-device pool and reused by later calls (creating a stream and seven
 // events costs more than a small job).  On any failure the function drains both streams before it returns, so the
 // caller may free or reuse its host buffers as soon as it sees the error.
+//
+// Kept-pixel sums (tclb200_host_args.pair_kept): each chunk's launch writes its pairs' sums into one device array behind
+// the other regions of the workspace, which goes back with one more D2H copy at the end.
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
@@ -61,14 +64,15 @@ inline size_t up256(size_t v) { return (v + 255) & ~(size_t)255; }
 constexpr int kClAll = TCLB200_CL_FRAMES | TCLB200_CL_FF | TCLB200_CL_BF;
 
 struct Layout {
-  size_t frames, flows[kRing][2], mask[kRing], prev_idx, cur_idx, vals, sums, scratch;
+  size_t frames, flows[kRing][2], mask[kRing], prev_idx, cur_idx, vals, sums, scratch, scratch_bytes;
+  size_t kept;   // pair_kept only (empty otherwise): the per-pair kept-pixel sums
   size_t stage[kRing], planar[2], total;   // channels-last only (empty otherwise): frame staging per ring slot, planar ff / bf
   size_t frame_bytes, flow_bytes, mask_bytes;
   int chunk;
 };
 
-// F = device frame slots provisioned; cl = TCLB200_CL_* bits
-Layout make_layout(int P, int F, int C, int H, int W, int dtype, int chunk_pairs, bool with_mask, int cl) {
+// F = device frame slots provisioned; cl = TCLB200_CL_* bits; with_kept: the call sets pair_kept
+Layout make_layout(int P, int F, int C, int H, int W, int dtype, int chunk_pairs, bool with_mask, int cl, bool with_kept) {
   Layout L;
   memset(&L, 0, sizeof(L));
   const size_t px = (size_t)H * W;
@@ -95,7 +99,8 @@ Layout make_layout(int P, int F, int C, int H, int W, int dtype, int chunk_pairs
   L.cur_idx = o; o += up256(sizeof(int) * (size_t)P);
   L.vals = o; o += up256(sizeof(float) * (size_t)P);
   L.sums = o; o += up256(sizeof(double) * (size_t)P);
-  L.scratch = o; o += up256(tclb200_scratch_bytes(L.chunk, H, W));
+  L.scratch_bytes = with_kept ? tclb200_scratch_bytes_kept(L.chunk, H, W) : tclb200_scratch_bytes(L.chunk, H, W);
+  L.scratch = o; o += up256(L.scratch_bytes);
   // a chunk of n pairs uploads at most 2n frames, and never more than there are slots
   const size_t stage_frames = (cl & TCLB200_CL_FRAMES) ? (size_t)(F < 2 * L.chunk ? F : 2 * L.chunk) : 0;
   for (int r = 0; r < kRing; ++r) { L.stage[r] = o; o += up256(L.frame_bytes * stage_frames); }
@@ -103,6 +108,8 @@ Layout make_layout(int P, int F, int C, int H, int W, int dtype, int chunk_pairs
     L.planar[j] = o;
     if (cl & (j == 0 ? TCLB200_CL_FF : TCLB200_CL_BF)) o += up256(L.flow_bytes * (size_t)L.chunk);
   }
+  L.kept = o;
+  if (with_kept) o += up256(sizeof(double) * (size_t)P);
   L.total = o;
   return L;
 }
@@ -233,7 +240,13 @@ extern "C" size_t tclb200_host_workspace_bytes(int P, int F, int C, int H, int W
 extern "C" size_t tclb200_host_workspace_bytes_cl(int P, int F, int C, int H, int W, int dtype, int chunk_pairs, int with_mask,
                                                   int channels_last) {
   if (P <= 0 || F <= 0 || C <= 0 || H <= 0 || W <= 0 || (channels_last & ~kClAll)) return 0;
-  return make_layout(P, F, C, H, W, dtype, chunk_pairs, with_mask != 0, channels_last).total;
+  return make_layout(P, F, C, H, W, dtype, chunk_pairs, with_mask != 0, channels_last, false).total;
+}
+
+extern "C" size_t tclb200_host_workspace_bytes_kept(int P, int F, int C, int H, int W, int dtype, int chunk_pairs, int with_mask,
+                                                    int channels_last) {
+  if (P <= 0 || F <= 0 || C <= 0 || H <= 0 || W <= 0 || (channels_last & ~kClAll)) return 0;
+  return make_layout(P, F, C, H, W, dtype, chunk_pairs, with_mask != 0, channels_last, true).total;
 }
 
 // on failure: drain both streams (the caller may free its host buffers when it sees the error), give the pipe back
@@ -250,7 +263,8 @@ extern "C" int tclb200_tcl_forward_host(const tclb200_host_args* a, tclb200_stre
   if (a->P == 0) return TCLB200_OK;   // a clip of one frame has no pairs: nothing to do, nothing to return
   if (a->F <= 0 || a->C <= 0 || a->H <= 0 || a->W <= 0) return hfail(TCLB200_ERR_INVALID, "F, C, H, W must be positive");
   if (!a->bf || !a->frames || !a->prev_index || !a->cur_index) return hfail(TCLB200_ERR_INVALID, "bf, frames, prev_index and cur_index are required");
-  if (!a->pair_vals && !a->pair_sums) return hfail(TCLB200_ERR_INVALID, "nothing to return: pair_vals and pair_sums are both NULL");
+  if (!a->pair_vals && !a->pair_sums && !a->pair_kept)
+    return hfail(TCLB200_ERR_INVALID, "nothing to return: pair_vals, pair_sums and pair_kept are all NULL");
   if (a->dtype != TCLB200_F32 && a->dtype != TCLB200_BF16 && a->dtype != TCLB200_U8) return hfail(TCLB200_ERR_INVALID, "unknown dtype");
   if (a->dtype == TCLB200_U8) {   // (the fused launches check the same; here nothing has been enqueued yet)
     if (a->C != 3) return hfail(TCLB200_ERR_INVALID, "uint8 frames must have C == 3");
@@ -266,8 +280,11 @@ extern "C" int tclb200_tcl_forward_host(const tclb200_host_args* a, tclb200_stre
       return hfail(TCLB200_ERR_INVALID, "prev_index / cur_index outside [0, F)");
   const bool with_mask = !a->ff && a->mask_in;
   const int S = (a->frame_slots > 0 && a->frame_slots < a->F) ? a->frame_slots : a->F;   // device frame slots
-  const Layout L = make_layout(a->P, S, a->C, a->H, a->W, a->dtype, a->chunk_pairs, with_mask, cl);
-  if (!a->workspace || a->workspace_bytes < L.total) return hfail(TCLB200_ERR_INVALID, "workspace missing or smaller than tclb200_host_workspace_bytes_cl()");
+  const bool with_kept = a->pair_kept != nullptr;
+  const Layout L = make_layout(a->P, S, a->C, a->H, a->W, a->dtype, a->chunk_pairs, with_mask, cl, with_kept);
+  if (!a->workspace || a->workspace_bytes < L.total)
+    return hfail(TCLB200_ERR_INVALID, with_kept ? "workspace missing or smaller than tclb200_host_workspace_bytes_kept()"
+                                                : "workspace missing or smaller than tclb200_host_workspace_bytes_cl()");
   if ((reinterpret_cast<uintptr_t>(a->workspace) & 255u) != 0) return hfail(TCLB200_ERR_INVALID, "workspace must be 256-byte aligned");
 
   cudaStream_t comp = reinterpret_cast<cudaStream_t>(stream);
@@ -333,7 +350,7 @@ extern "C" int tclb200_tcl_forward_host(const tclb200_host_args* a, tclb200_stre
   HOST_TRY(cudaEventRecord(pipe->fork, comp));
   HOST_TRY(cudaStreamWaitEvent(pipe->copy[0], pipe->fork, 0));
   HOST_TRY(cudaStreamWaitEvent(pipe->copy[1], pipe->fork, 0));
-  HOST_TRY(cudaMemsetAsync(ws + L.scratch, 0, tclb200_scratch_bytes(L.chunk, a->H, a->W), comp));
+  HOST_TRY(cudaMemsetAsync(ws + L.scratch, 0, L.scratch_bytes, comp));
   HOST_TRY(cudaMemcpyAsync(ws + L.prev_idx, h_prev, sizeof(int) * (size_t)a->P, cudaMemcpyHostToDevice, comp));
   HOST_TRY(cudaMemcpyAsync(ws + L.cur_idx, h_cur, sizeof(int) * (size_t)a->P, cudaMemcpyHostToDevice, comp));
 
@@ -385,7 +402,8 @@ extern "C" int tclb200_tcl_forward_host(const tclb200_host_args* a, tclb200_stre
     t.n_prev_frames = S; t.n_cur_frames = S;
     t.pair_vals = reinterpret_cast<float*>(ws + L.vals) + s;
     t.pair_sums = reinterpret_cast<double*>(ws + L.sums) + s;
-    t.scratch = ws + L.scratch; t.scratch_bytes = tclb200_scratch_bytes(L.chunk, a->H, a->W);
+    if (with_kept) t.pair_kept = reinterpret_cast<double*>(ws + L.kept) + s;
+    t.scratch = ws + L.scratch; t.scratch_bytes = L.scratch_bytes;
     t.B = n; t.C = a->C; t.H = a->H; t.W = a->W;
     t.dtype = a->dtype; t.flags = a->flags | TCLB200_THROUGHPUT; t.loss = a->loss; t.finalize = a->finalize;
     memcpy(t.u8_scale, a->u8_scale, sizeof(t.u8_scale)); memcpy(t.u8_offset, a->u8_offset, sizeof(t.u8_offset));
@@ -395,6 +413,7 @@ extern "C" int tclb200_tcl_forward_host(const tclb200_host_args* a, tclb200_stre
   }
   if (a->pair_vals) HOST_TRY(cudaMemcpyAsync(a->pair_vals, ws + L.vals, sizeof(float) * (size_t)a->P, cudaMemcpyDeviceToHost, comp));
   if (a->pair_sums) HOST_TRY(cudaMemcpyAsync(a->pair_sums, ws + L.sums, sizeof(double) * (size_t)a->P, cudaMemcpyDeviceToHost, comp));
+  if (with_kept) HOST_TRY(cudaMemcpyAsync(a->pair_kept, ws + L.kept, sizeof(double) * (size_t)a->P, cudaMemcpyDeviceToHost, comp));
   // the pipe goes back to the pool once its last use (the final ready event the caller's stream waits for) is enqueued;
   // a later call's work on the copy stream is ordered behind this call's by the stream itself
   release_pipe(pipe);

@@ -25,6 +25,7 @@
 // fused_forward_generic_kernel covers shapes TMA cannot describe (W % 4 != 0, unaligned views, C != 3).
 // uint8 frames (evaluation only): fused_forward_ws_u8_kernel / fused_forward_generic_u8_kernel are the same two kernels with
 // the frames normalised per channel as they are loaded (W % 16 == 0 for the TMA one: uint8 box rows are multiples of 16 bytes).
+// Kept-pixel sums (pair_kept / total_kept): the *_kept_kernel instantiations of the same bodies, with a second fp64 partial per tile.
 // warp_backward_kernel: autograd of warp / fused backward of the training loss.  gradient_kernel.  hwc_split_kernel
 // (dataset ingest) and upsample_flow_kernel (RAFT's convex upsampling) are the steps either side of the path.
 // HBM-bound fp32 streaming + gather: no tensor cores, nothing here is a contraction.
@@ -253,13 +254,15 @@ constexpr int kVarOutputs = 4;   // as kVarL2 plus the per-pixel outputs (warp_o
 template <typename FrameT, int MASK, bool REDUCE, int CT, int LEAN, typename FlowSrc, typename FrameSrc>
 __device__ __forceinline__ void finish_pixel(const FwdParams& p, const PixTaps& s, float u, float v, float nb, float keep,
                                              size_t o, size_t plane, int pair, const FlowSrc& fsrc, const FrameSrc& psrc,
-                                             const PairPtrs<FrameT>& io, const float* cv, float& err, unsigned& near) {
+                                             const PairPtrs<FrameT>& io, const float* cv, float& err, unsigned& near,
+                                             float* kept = nullptr) {
   if (MASK == MASK_COMPUTED && (LEAN || (p.flags & TCLB200_OCC))) {
     const float wu = fsrc.sample(0, s), wv = fsrc.sample(1, s);
     float margin;
     if (occluded(wu, wv, u, v, nb, kV, &margin)) keep = 0.0f;
     if (!LEAN) near += fabsf(margin) < kNearBand;
   }
+  if (kept) *kept += keep;   // (the kept-pixel kernels: this pixel's final verdict)
   if ((!LEAN || CT == 0) && p.mask_out) __stcs(p.mask_out + (size_t)pair * plane + o, keep);
   if (p.prev == nullptr) return;
   const bool validity = (!LEAN || MASK == MASK_NONE) && (p.flags & TCLB200_VALIDITY);
@@ -311,8 +314,9 @@ __device__ __forceinline__ PairPtrs<FrameT> pair_ptrs(const FwdParams& p, int pa
 // ---------------------------------------------------------------------------------------------
 // generic forward kernel: one pixel per lane, everything straight from global memory
 // ---------------------------------------------------------------------------------------------
-template <typename FrameT, int MASK, bool REDUCE, int CT, typename Params>
-__device__ __forceinline__ void fused_forward_generic(const Params& p) {
+// KEPT (reducing kernels with a mask): each pixel's final mask value also goes to the kept-pixel sums of `k`
+template <typename FrameT, int MASK, bool REDUCE, int CT, bool KEPT = false, typename Params>
+__device__ __forceinline__ void fused_forward_generic(const Params& p, const KeptOut* k = nullptr) {
   static_assert(std::is_same<FrameT, uint8_t>::value == std::is_same<Params, FwdParamsU8>::value,
                 "uint8 frames come with their normalisation (FwdParamsU8), the other frame types without it");
   const Geo& g = p.geo;
@@ -324,7 +328,7 @@ __device__ __forceinline__ void fused_forward_generic(const Params& p) {
   const int ty = tile / p.tiles_x, tx = tile - ty * p.tiles_x;
   const int x = tx * 32 + lane, y = p.row_begin + ty * kWarps + wrp;   // (band mode: rows [row_begin, row_end) only)
   const int C = CT > 0 ? CT : p.C;
-  float err = 0.0f;
+  float err = 0.0f, kept = 0.0f;
   unsigned near = 0;
   if (x < W && y < p.row_end) {
     const size_t o = (size_t)y * W + x;
@@ -347,10 +351,12 @@ __device__ __forceinline__ void fused_forward_generic(const Params& p) {
     GlobalSrc<float> fsrc{p.ff ? p.ff + (size_t)ff_field(p, pair) * p.ff_batch : nullptr, p.ff_plane, g};
     const GlobalSrc<FrameT> psrc = frame_src<FrameT>(p, p.prev ? reinterpret_cast<const FrameT*>(p.prev) + (size_t)prev_frame(p, pair) * C * plane : nullptr, plane);
     finish_pixel<FrameT, MASK, REDUCE, CT, false>(p, s, u, v, nb, keep, o, plane, pair, fsrc, psrc,
-                                                  pair_ptrs<FrameT>(p, pair, cur_frame(p, pair), C, plane), nullptr, err, near);
+                                                  pair_ptrs<FrameT>(p, pair, cur_frame(p, pair), C, plane), nullptr, err, near,
+                                                  KEPT ? &kept : nullptr);
   }
   count_near(near, p.near_threshold);
-  if (REDUCE) reduce_and_finalise(err, p, pair, tile);
+  if constexpr (KEPT) reduce_and_finalise<true>(err, p, pair, tile, kept, k);
+  else if (REDUCE) reduce_and_finalise(err, p, pair, tile);
 }
 template <typename FrameT, int MASK, bool REDUCE, int CT>
 __global__ void __launch_bounds__(kThreads) fused_forward_generic_kernel(const FwdParams p) {
@@ -360,6 +366,15 @@ __global__ void __launch_bounds__(kThreads) fused_forward_generic_kernel(const F
 template <int MASK>
 __global__ void __launch_bounds__(kThreads) fused_forward_generic_u8_kernel(const FwdParamsU8 p) {
   fused_forward_generic<uint8_t, MASK, true, 3>(p);
+}
+// ... and both with the kept-pixel sums (reductions with a mask only)
+template <typename FrameT, int MASK, int CT>
+__global__ void __launch_bounds__(kThreads) fused_forward_generic_kept_kernel(const FwdParams p, const KeptOut k) {
+  fused_forward_generic<FrameT, MASK, true, CT, true>(p, &k);
+}
+template <int MASK>
+__global__ void __launch_bounds__(kThreads) fused_forward_generic_u8_kept_kernel(const FwdParamsU8 p, const KeptOut k) {
+  fused_forward_generic<uint8_t, MASK, true, 3, true>(p, &k);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -560,6 +575,10 @@ struct WsCtl {              // control block in shared memory
   int box[NB][4];           // per flow stage: extent of x+u, y+v over the tile (ordered-int encoding): xmin, ymin, xmax, ymax
   float red[NS][CW * 32];   // per source stage: every consumer lane's error sum of the tile
 };
+template <int NB, int NS, int CW>
+struct WsCtlKept : WsCtl<NB, NS, CW> {   // (the kept-pixel kernels: the control block's spare bytes hold the warps' kept sums)
+  double kred[NS][CW];      // per source stage: every consumer warp's kept-pixel sum of the tile
+};
 
 // order-preserving float <-> int (total order of IEEE bit patterns; NaNs land beyond +-Inf): lets redux.sync work on
 // float extents
@@ -641,69 +660,103 @@ __device__ __forceinline__ void mbar_wait_s(uint32_t bar, unsigned parity) {
 // atomics on its critical path); this kernel, launched behind it with programmatic dependent launch so that its
 // launch latency overlaps the hot kernel, sums each pair's partials in index order and the pairs in index order
 // (deterministic), finalises (mean / RMSE) and leaves the scratch zeroed as the protocol of tcl_common.cuh wants.
-__global__ void __launch_bounds__(kThreads) fold_partials_kernel(const FwdParams p) {
+// KEPT: the kept-pixel partials of `k` are folded the same way, in the same launch.
+template <bool KEPT>
+__device__ __forceinline__ void fold_partials(const FwdParams& p, const KeptOut& k) {
   __shared__ double red[kWarps];
   __shared__ int s_last;
   asm volatile("griddepcontrol.wait;" ::: "memory");   // all of the hot kernel's stores are visible after this
   const int pair = blockIdx.x;
   const unsigned tpp = p.tiles_per_pair;
   double* pp = p.scratch.partials + (size_t)pair * tpp;
-  double s = 0.0;
+  double* kp = KEPT ? k.partials + (size_t)pair * tpp : nullptr;
+  double s = 0.0, ks = 0.0;
   for (unsigned i = threadIdx.x; i < tpp; i += kThreads) {
     s += __ldcg(pp + i);
     __stcg(pp + i, 0.0);
+    if constexpr (KEPT) {
+      ks += __ldcg(kp + i);
+      __stcg(kp + i, 0.0);
+    }
   }
   const double S = block_sum(s, red);
+  double KS = 0.0;
+  if constexpr (KEPT) KS = block_sum(ks, red);
   if (threadIdx.x == 0) {
     if (p.pair_sums) p.pair_sums[pair] = S;
     if (p.pair_vals) p.pair_vals[pair] = finalise_value(S * p.inv_count, p.finalize);
     __stcg(pp, S);  // this pair's record for the batch fold
+    if constexpr (KEPT) {
+      if (k.pair_kept) k.pair_kept[pair] = KS;
+      __stcg(kp, KS);
+    }
     __threadfence();
     s_last = atomicAdd(p.scratch.batch_ticket, 1u) == (unsigned)p.B - 1;
   }
   __syncthreads();
   if (!s_last) return;
   __threadfence();
-  double a = 0.0, b = 0.0;
+  double a = 0.0, b = 0.0, c = 0.0;
   for (int i = threadIdx.x; i < p.B; i += kThreads) {
     double* rec = p.scratch.partials + (size_t)i * tpp;
     const double Si = __ldcg(rec);
     __stcg(rec, 0.0);
     a += Si;
     b += (double)finalise_value(Si * p.inv_count, p.finalize);
+    if constexpr (KEPT) {
+      c += __ldcg(k.partials + (size_t)i * tpp);
+      __stcg(k.partials + (size_t)i * tpp, 0.0);
+    }
   }
   const double A = block_sum(a, red);
   const double Bv = block_sum(b, red);
+  double Cv = 0.0;
+  if constexpr (KEPT) Cv = block_sum(c, red);
   if (threadIdx.x == 0) {
     if (p.total_sums) { p.total_sums[0] = A; p.total_sums[1] = Bv; }
     if (p.total_val) *p.total_val = finalise_value(A * p.inv_count / (double)p.B, p.finalize);
+    if constexpr (KEPT)
+      if (k.total_kept) *k.total_kept = Cv;
     *p.scratch.batch_ticket = 0;
   }
 }
+__global__ void __launch_bounds__(kThreads) fold_partials_kernel(const FwdParams p) { fold_partials<false>(p, KeptOut{}); }
+__global__ void __launch_bounds__(kThreads) fold_partials_kept_kernel(const FwdParams p, const KeptOut k) { fold_partials<true>(p, k); }
 
 // The same for short launches (<= kFoldSmallPairs pairs, a few thousand partials): ONE CTA, 256 threads per pair and four
 // pairs at a time, no tickets and no second trip through L2 -- about half the latency of the two-level fold above, which
 // matters when the whole launch is 10-20 us.  Same summation order as fold_partials_kernel, so a pair's value does not
 // depend on which of the two folded it.
 constexpr int kFoldSmallPairs = 64, kFoldSmallPartials = 16384, kFoldSmallGroups = 1024 / kThreads;
-__global__ void __launch_bounds__(1024) fold_partials_small_kernel(const FwdParams p) {
+template <bool KEPT>
+__device__ __forceinline__ void fold_partials_small(const FwdParams& p, const KeptOut& k) {
   __shared__ double s_S[kFoldSmallPairs];
+  __shared__ double s_K[KEPT ? kFoldSmallPairs : 1];
   __shared__ double s_red[kFoldSmallGroups][kWarps];
+  __shared__ double s_kred[KEPT ? kFoldSmallGroups : 1][kWarps];
   asm volatile("griddepcontrol.wait;" ::: "memory");
   const int grp = threadIdx.x / kThreads, t = threadIdx.x - grp * kThreads, lane = t & 31, w = t >> 5;
   const unsigned tpp = p.tiles_per_pair;
   for (int base = 0; base < p.B; base += kFoldSmallGroups) {
     const int pair = base + grp;
-    double s = 0.0;
+    double s = 0.0, ks = 0.0;
     if (pair < p.B) {
       double* pp = p.scratch.partials + (size_t)pair * tpp;
       for (unsigned i = t; i < tpp; i += kThreads) {
         s += __ldcg(pp + i);
         __stcg(pp + i, 0.0);
+        if constexpr (KEPT) {
+          ks += __ldcg(k.partials + (size_t)pair * tpp + i);
+          __stcg(k.partials + (size_t)pair * tpp + i, 0.0);
+        }
       }
     }
     s = warp_sum(s);
     if (lane == 0) s_red[grp][w] = s;
+    if constexpr (KEPT) {
+      ks = warp_sum(ks);
+      if (lane == 0) s_kred[grp][w] = ks;
+    }
     __syncthreads();
     if (t == 0 && pair < p.B) {
       double S = 0.0;
@@ -712,17 +765,29 @@ __global__ void __launch_bounds__(1024) fold_partials_small_kernel(const FwdPara
       if (p.pair_sums) p.pair_sums[pair] = S;
       if (p.pair_vals) p.pair_vals[pair] = finalise_value(S * p.inv_count, p.finalize);
       s_S[pair] = S;
+      if constexpr (KEPT) {
+        double KS = 0.0;
+#pragma unroll
+        for (int i = 0; i < kWarps; ++i) KS += s_kred[grp][i];
+        if (k.pair_kept) k.pair_kept[pair] = KS;
+        s_K[pair] = KS;
+      }
     }
     __syncthreads();
   }
   if (grp != 0) return;
-  double a = 0.0, b = 0.0;
+  double a = 0.0, b = 0.0, c = 0.0;
   for (int i = t; i < p.B; i += kThreads) {
     a += s_S[i];
     b += (double)finalise_value(s_S[i] * p.inv_count, p.finalize);
+    if constexpr (KEPT) c += s_K[i];
   }
   a = warp_sum(a); b = warp_sum(b);
   if (lane == 0) { s_red[0][w] = a; s_red[1][w] = b; }
+  if constexpr (KEPT) {
+    c = warp_sum(c);
+    if (lane == 0) s_red[2][w] = c;
+  }
   asm volatile("bar.sync 1, 256;" ::: "memory");   // (the first group's 256 threads only)
   if (t == 0) {
     double A = 0.0, Bv = 0.0;
@@ -730,8 +795,16 @@ __global__ void __launch_bounds__(1024) fold_partials_small_kernel(const FwdPara
     for (int i = 0; i < kWarps; ++i) { A += s_red[0][i]; Bv += s_red[1][i]; }
     if (p.total_sums) { p.total_sums[0] = A; p.total_sums[1] = Bv; }
     if (p.total_val) *p.total_val = finalise_value(A * p.inv_count / (double)p.B, p.finalize);
+    if constexpr (KEPT) {
+      double Cv = 0.0;
+#pragma unroll
+      for (int i = 0; i < kWarps; ++i) Cv += s_red[2][i];
+      if (k.total_kept) *k.total_kept = Cv;
+    }
   }
 }
+__global__ void __launch_bounds__(1024) fold_partials_small_kernel(const FwdParams p) { fold_partials_small<false>(p, KeptOut{}); }
+__global__ void __launch_bounds__(1024) fold_partials_small_kept_kernel(const FwdParams p, const KeptOut k) { fold_partials_small<true>(p, k); }
 
 // Global tile number -> pair and tile.  pair_group G > 1 interleaves the tiles of G consecutive pairs (tile 0 of pairs
 // g*G .. g*G+G-1, then their tiles 1, ...): the evaluations of one target frame's window read the same `cur` tile, the same
@@ -758,11 +831,12 @@ template <typename Cfg>
 __device__ __forceinline__ bool tile_edge(const TileId& t, const Geo& g, int row_end) { return (t.x0 + Cfg::TW > g.W) || (t.y0 + Cfg::TH > row_end); }
 
 // ---- consumer: exact per-pixel path (all features; staged boxes, global gathers, or both in a mixed tile) -------
+// `kept` (kept-pixel kernels, else nullptr): += the final mask value of every pixel of the tile
 template <typename FrameT, int MASK, bool REDUCE, int CT, int LEAN, typename Cfg, bool EDGE>
 __device__ __forceinline__ float full_tile(const FwdParams& p, const float* s_bu, const float* s_ff, const FrameT* s_prev,
                                            const int* meta, const TileId& t, int lx0, int ly0,
                                            const float (&cur)[Cfg::kPPL][Cfg::kC], const float (&mk)[Cfg::kPPL], bool have_cur,
-                                           unsigned& near) {
+                                           unsigned& near, float* kept = nullptr) {
   const Geo& g = p.geo;
   const int W = g.W, H = g.H;
   const size_t plane = (size_t)H * W;
@@ -799,8 +873,8 @@ __device__ __forceinline__ float full_tile(const FwdParams& p, const float* s_bu
     // taps [x0, x0+1] x [y0, y0+1] inside the staged boxes?  (unsigned compare: also catches negatives / saturation)
     const bool inbox = mode == 1 || (mode == 2 && (unsigned)(taps.x0 - ox) < (unsigned)(Cfg::BW - 1) &&
                                      (unsigned)(taps.y0 - oy) < (unsigned)(Cfg::BH - 1));
-    if (inbox) finish_pixel<FrameT, MASK, REDUCE, CT, LEAN>(p, taps, u, v, nb, keep, o, plane, t.pair, fs, ps, io, cv, err, near);
-    else finish_pixel<FrameT, MASK, REDUCE, CT, LEAN>(p, taps, u, v, nb, keep, o, plane, t.pair, fg, pg, io, cv, err, near);   // exact predicated gathers
+    if (inbox) finish_pixel<FrameT, MASK, REDUCE, CT, LEAN>(p, taps, u, v, nb, keep, o, plane, t.pair, fs, ps, io, cv, err, near, kept);
+    else finish_pixel<FrameT, MASK, REDUCE, CT, LEAN>(p, taps, u, v, nb, keep, o, plane, t.pair, fg, pg, io, cv, err, near, kept);   // exact predicated gathers
   }
   return err;
 }
@@ -956,15 +1030,28 @@ __device__ __forceinline__ void replay_ambiguous(const float* s_bu, const float*
   }
 }
 
+// a lane's kept-pixel sum over its P pixels of a staged tile, in pixel order: the final verdicts (computed mask; pixels outside
+// the image have none set) or the dataset mask values (0 outside the image)
+template <int MASK, int P>
+__device__ __forceinline__ float kept_sum(unsigned keepbits, const float (&mk)[P]) {
+  if constexpr (MASK == MASK_COMPUTED) return (float)__popc(keepbits);   // (a count: exact, and two instructions)
+  float s = 0.0f;
+#pragma unroll
+  for (int k = 0; k < P; ++k) s = __fadd_rn(s, MASK == MASK_GIVEN ? mk[k] : (((keepbits >> k) & 1u) ? 1.0f : 0.0f));
+  return s;
+}
+
 // CT == 3: masked squared error against `cur` (returned); CT == 0: mask-only (fbcCheckTorch), the verdicts go to mask_out
 // OCC == false (mask-only): the optimisation-based variant of fbcCheckTorch, motion-boundary test alone -- no source
 // boxes are staged and no sampling position is needed (methods/optimization-based/flowtools.py:34-58)
 // OUTS (staged, non-mixed tiles of the reducing configurations): the optional per-pixel outputs -- warp_out, mask_out,
 // blend_out, whichever pointers are set -- are stored from the same pass (the warped values wait in registers until the
 // mask verdicts are final)
-template <typename FrameT, int MASK, int CT, int LOSS, typename Cfg, bool EDGE, bool MIXED, bool OCC = true, bool OUTS = false>
+// KEPT: *kept = the lane's sum of its pixels' final mask values (the verdicts, or the dataset mask; 0 outside the image)
+template <typename FrameT, int MASK, int CT, int LOSS, typename Cfg, bool EDGE, bool MIXED, bool OCC = true, bool OUTS = false, bool KEPT = false>
 __device__ __forceinline__ float lean_tile(const FwdParams& p, const float* s_bu, const float* s_ff, const int* meta, const TileId& t,
-                                           int lx0, int ly0, const float (&cur)[Cfg::kPPL][Cfg::kC], const float (&mk)[Cfg::kPPL]) {
+                                           int lx0, int ly0, const float (&cur)[Cfg::kPPL][Cfg::kC], const float (&mk)[Cfg::kPPL],
+                                           float* kept = nullptr) {
   constexpr int P = Cfg::kPPL, BW = Cfg::BW, BFW = Cfg::kBfW, PL = Cfg::BH * Cfg::BW;
   constexpr float kHi = 1.0f + kFilterEps, kLo = 1.0f - kFilterEps;
   constexpr int FE = (int)sizeof(FrameT);
@@ -1137,6 +1224,11 @@ __device__ __forceinline__ float lean_tile(const FwdParams& p, const float* s_bu
                                                    reinterpret_cast<const FrameT*>(p.prev) + (size_t)t.pf * 3 * plane, g, t.x0 + lx0,
                                                    t.y0 + ly0 + pix_dy(k), cur[k][0], cur[k][1], cur[k][2], mk[k]);
           keepbits |= 1u << k;   // the verdict is already applied
+          if constexpr (KEPT && MASK == MASK_COMPUTED) {   // (the kept-pixel count needs the verdict itself: e[k] is 0 without it)
+            const float kp = pixel_global<FrameT, MASK, true, LOSS>(p.bf + (size_t)t.bfi * p.bf_batch, p.bf_plane, p.ff + (size_t)t.ffi * p.ff_batch,
+                                                                    p.ff_plane, nullptr, g, t.x0 + lx0, t.y0 + ly0 + pix_dy(k), 0.0f, 0.0f, 0.0f, 0.0f);
+            keepbits = (keepbits & ~(1u << k)) | ((kp != 0.0f ? 1u : 0u) << k);
+          }
         } else {   // (mask-only; and uint8 frames: the loop's error is exact already -- the taps came from global memory with the
                    // predicates -- only the verdict that was too close to call is redone)
           const float kp = pixel_global<FrameT, MASK, true, LOSS>(p.bf + (size_t)t.bfi * p.bf_batch, p.bf_plane, p.ff + (size_t)t.ffi * p.ff_batch, p.ff_plane, nullptr, g,
@@ -1176,6 +1268,7 @@ __device__ __forceinline__ float lean_tile(const FwdParams& p, const float* s_bu
     }
     return 0.0f;
   }
+  if constexpr (KEPT) *kept = kept_sum<MASK, P>(keepbits, mk);
   float err = 0.0f;
 #pragma unroll
   for (int k = 0; k < P; ++k) {
@@ -1211,9 +1304,11 @@ __device__ __forceinline__ float2 staged_tap4x2(uint32_t a0, uint32_t a1, float2
 // EDGE: the tile overhangs the image (pixels outside are computed on a safe address and dropped); MIXED: a motion boundary
 // runs through the tile and the taps of some pixels lie outside the staged boxes -- those pixels are redone one by one
 // from global memory after the loop (pixel_global, exact), every other pixel of the tile keeps the fast path.
-template <typename FrameT, int MASK, int LOSS, typename Cfg, bool EDGE = false, bool MIXED = false, int CT = 3>
+// KEPT: as in lean_tile
+template <typename FrameT, int MASK, int LOSS, typename Cfg, bool EDGE = false, bool MIXED = false, int CT = 3, bool KEPT = false>
 __device__ __forceinline__ float lean_tile_packed(const FwdParams& p, const float* s_bu, const float* s_ff, const int* meta, const TileId& t,
-                                                  int lx0, int ly0, const float (&cur)[Cfg::kPPL][Cfg::kC], const float (&mk)[Cfg::kPPL]) {
+                                                  int lx0, int ly0, const float (&cur)[Cfg::kPPL][Cfg::kC], const float (&mk)[Cfg::kPPL],
+                                                  float* kept = nullptr) {
   constexpr int P = Cfg::kPPL, BW = Cfg::BW, BFW = Cfg::kBfW, PL = Cfg::BH * Cfg::BW;
   constexpr float kHi = 1.0f + kFilterEps, kLo = 1.0f - kFilterEps;
   constexpr int FE = (int)sizeof(FrameT);
@@ -1361,6 +1456,11 @@ __device__ __forceinline__ float lean_tile_packed(const FwdParams& p, const floa
                                                          reinterpret_cast<const FrameT*>(p.prev) + (size_t)t.pf * 3 * plane, g, t.x0 + lx0,
                                                          t.y0 + ly0 + pix_dy(k), cur[k][0], cur[k][CT == 3 ? 1 : 0], cur[k][CT == 3 ? 2 : 0], mk[k]);
           keepbits |= 1u << k;   // the verdict is already applied
+          if constexpr (KEPT && MASK == MASK_COMPUTED) {   // (the kept-pixel count needs the verdict itself: e[k] is 0 without it)
+            const float kp = pixel_global<FrameT, MASK, true, LOSS>(p.bf + (size_t)t.bfi * p.bf_batch, p.bf_plane, p.ff + (size_t)t.ffi * p.ff_batch,
+                                                                    p.ff_plane, nullptr, g, t.x0 + lx0, t.y0 + ly0 + pix_dy(k), 0.0f, 0.0f, 0.0f, 0.0f);
+            keepbits = (keepbits & ~(1u << k)) | ((kp != 0.0f ? 1u : 0u) << k);
+          }
         } else {
           const float kp = pixel_global<FrameT, MASK, true, LOSS>(p.bf + (size_t)t.bfi * p.bf_batch, p.bf_plane, p.ff + (size_t)t.ffi * p.ff_batch, p.ff_plane, nullptr, g,
                                                                   t.x0 + lx0, t.y0 + ly0 + pix_dy(k), 0.0f, 0.0f, 0.0f, 0.0f);
@@ -1375,6 +1475,7 @@ __device__ __forceinline__ float lean_tile_packed(const FwdParams& p, const floa
       if (!EDGE || (xin && 2 * k < rows_in)) __stcs(mo + (ptrdiff_t)pix_dy(k) * g.W, ((keepbits >> k) & 1u) ? 1.0f : 0.0f);
     return 0.0f;
   }
+  if constexpr (KEPT) *kept = kept_sum<MASK, P>(keepbits, mk);
   float err = 0.0f;
 #pragma unroll
   for (int k = 0; k < P; ++k) {
@@ -1401,16 +1502,21 @@ __device__ __forceinline__ float lean_tile_packed(const FwdParams& p, const floa
 //   consumer warps  one pass per pixel: flow + 4 neighbours from the flow tile (vertical strips, see WsCfg),
 //                   motion-boundary test, sampling position, 4 x (2 + C) taps from the source boxes, occlusion test,
 //                   masked error against `cur` (coalesced global loads issued before the wait for the boxes).
-template <typename FrameT, int MASK, bool REDUCE, int CT, int LEAN, typename Cfg, typename Params>
+//   KEPT            (the kept-pixel kernels) each consumer lane also sums its pixels' final mask values in fp32 (a popcount of
+//                   the verdicts for computed masks), each warp folds its lanes (an integer redux for computed masks, a fixed
+//                   fp64 butterfly for dataset masks), and the producer folds the warps in warp order into a second fp64
+//                   partial per tile (kept_partials) next to the error's
+template <typename FrameT, int MASK, bool REDUCE, int CT, int LEAN, typename Cfg, bool KEPT = false, typename Params>
 __device__ __forceinline__ void fused_forward_ws(const Params& p, const CUtensorMap& tm_bf, const CUtensorMap& tm_ff,
-                                                 const CUtensorMap& tm_prev, const CUtensorMap& tm_cur) {
+                                                 const CUtensorMap& tm_prev, const CUtensorMap& tm_cur, double* kept_partials = nullptr) {
   static_assert(std::is_same<FrameT, uint8_t>::value == std::is_same<Params, FwdParamsU8>::value,
                 "uint8 frames come with their normalisation (FwdParamsU8), the other frame types without it");
   constexpr int NB = Cfg::NB, NS = Cfg::NS, P = Cfg::kPPL;
   constexpr int kCWarps = Cfg::CW;
   constexpr int kLoss = LEAN == kVarL1 ? TCLB200_L1 : TCLB200_L2;
-  using Ctl = WsCtl<NB, NS, kCWarps>;
+  using Ctl = std::conditional_t<KEPT, WsCtlKept<NB, NS, kCWarps>, WsCtl<NB, NS, kCWarps>>;
   static_assert(sizeof(Ctl) <= Cfg::kCtlBytes, "control block too large");
+  static_assert(!KEPT || (REDUCE && MASK != MASK_NONE), "kept-pixel sums: reductions with a mask");
   extern __shared__ __align__(128) unsigned char smem_raw[];
   unsigned char* smem = smem_raw + ((128u - (smem_u32(smem_raw) & 127u)) & 127u);  // TMA destinations: 128-byte aligned
   Ctl* ctl = reinterpret_cast<Ctl*>(smem + Cfg::kCtlOff);
@@ -1542,6 +1648,11 @@ __device__ __forceinline__ void fused_forward_ws(const Params& p, const CUtensor
 #pragma unroll
         for (int w = 0; w < kCWarps; ++w) ts += (double)r[32 * w];
       }
+      double kt = 0.0;
+      if constexpr (KEPT) {
+#pragma unroll
+        for (int w = 0; w < kCWarps; ++w) kt += ctl->kred[j % NS][w];
+      }
       __syncwarp();   // (all of red[] is in registers before the stage is handed out again)
       if (lane == 0) {
         if (real(j + NS)) issue_src(j + NS, place_src(j + NS));
@@ -1553,6 +1664,8 @@ __device__ __forceinline__ void fused_forward_ws(const Params& p, const CUtensor
         ts = warp_sum(ts);
         if (lane == 0) __stcg(&p.scratch.partials[(size_t)t.pair * p.tiles_per_pair + t.tile], ts);
       }
+      if constexpr (KEPT)
+        if (lane == 0) __stcg(&kept_partials[(size_t)t.pair * p.tiles_per_pair + t.tile], kt);
     }
     // long launches: the last CTA to run out of tiles re-arms the tile counter for the next launch
     if (dynamic && lane == 0) {
@@ -1647,16 +1760,20 @@ __device__ __forceinline__ void fused_forward_ws(const Params& p, const CUtensor
     // the tile bodies with their template flags EDGE (the tile overhangs the image) and MIXED: the staged tiles of the LEAN
     // variants take lean_tile_packed where uses_packed says so and lean_tile otherwise (kVarMobOnly: nothing staged, nothing
     // sampled, the flow tile alone decides); every other tile takes full_tile, the exact per-pixel path of variant VAR
+    float kept = 0.0f;   // (KEPT: the lane's kept-pixel sum of this tile)
     auto staged = [&](auto edge, auto mixed) -> float {
       constexpr bool E = decltype(edge)::value, M = decltype(mixed)::value;
       if constexpr (uses_packed(MASK, REDUCE, CT, LEAN) && sizeof(FrameT) != 1)
-        return lean_tile_packed<FrameT, MASK, kLoss, Cfg, E, M, CT>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
+        return lean_tile_packed<FrameT, MASK, kLoss, Cfg, E, M, CT, KEPT>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk,
+                                                                          KEPT ? &kept : nullptr);
       else
-        return lean_tile<FrameT, MASK, CT, kLoss, Cfg, E, M, LEAN != kVarMobOnly, LEAN == kVarOutputs && !M>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0, ly0, cur, mk);
+        return lean_tile<FrameT, MASK, CT, kLoss, Cfg, E, M, LEAN != kVarMobOnly, LEAN == kVarOutputs && !M, KEPT>(p, bf_stage(sb), ff_stage(ss), ctl->meta[ss], t, lx0,
+                                                                                                                ly0, cur, mk, KEPT ? &kept : nullptr);
     };
     auto full = [&](auto var, auto edge) -> float {
       return full_tile<FrameT, MASK, REDUCE, CT, decltype(var)::value, Cfg, decltype(edge)::value>(p, bf_stage(sb), ff_stage(ss), prev_stage(ss), ctl->meta[ss],
-                                                                                                   t, lx0, ly0, cur, mk, have_cur, near);
+                                                                                                   t, lx0, ly0, cur, mk, have_cur, near,
+                                                                                                   KEPT ? &kept : nullptr);
     };
     // (kVarMobOnly tiles are mask-only, CT == 0: uses_packed is false for them, lean_tile returns 0 and nothing is reduced)
     const std::true_type yes{};
@@ -1668,6 +1785,10 @@ __device__ __forceinline__ void fused_forward_ws(const Params& p, const CUtensor
     else err = (LEAN || t_edge) ? full(var, yes) : full(var, no);
     // <= 3 * P fp32 terms per lane; the producer folds the lanes (fixed order, fp64)
     if (REDUCE) asm volatile("st.shared.f32 [%0], %1;" ::"r"(red_s + (uint32_t)(ss * kCWarps * 128)), "f"(err) : "memory");
+    if constexpr (KEPT) {   // computed masks: the lanes hold verdict counts, an exact integer sum; dataset masks: a fixed fp64 butterfly
+      const double kw = MASK == MASK_COMPUTED ? (double)__reduce_add_sync(0xffffffffu, (unsigned)kept) : warp_sum((double)kept);
+      if (lane == 0) ctl->kred[ss][warp] = kw;
+    }
     __syncwarp();   // every lane is done reading the stages of tile k
     if (lane == 0) mbar_arrive_s(done_s + 8u * ss);
     if (threadIdx.x == 0) TCL_STAMP(k, 3);
@@ -1690,6 +1811,24 @@ __global__ void __launch_bounds__(Cfg::kThreads, 1) fused_forward_ws_u8_kernel(c
                                                                             const __grid_constant__ CUtensorMap tm_prev,
                                                                             const __grid_constant__ CUtensorMap tm_cur) {
   fused_forward_ws<uint8_t, MASK, REDUCE, CT, LEAN, Cfg>(p, tm_bf, tm_ff, tm_prev, tm_cur);
+}
+// ... and both with the kept-pixel sums (reductions with a mask, variants kVarL2 / kVarL1): the same kernels with the per-tile
+// kept partials next to the error's and the kept-pixel output pointers as a second parameter block
+template <typename FrameT, int MASK, int CT, int LEAN, typename Cfg>
+__global__ void __launch_bounds__(Cfg::kThreads, 1) fused_forward_ws_kept_kernel(const FwdParams p, const KeptOut k,
+                                                                              const __grid_constant__ CUtensorMap tm_bf,
+                                                                              const __grid_constant__ CUtensorMap tm_ff,
+                                                                              const __grid_constant__ CUtensorMap tm_prev,
+                                                                              const __grid_constant__ CUtensorMap tm_cur) {
+  fused_forward_ws<FrameT, MASK, true, CT, LEAN, Cfg, true>(p, tm_bf, tm_ff, tm_prev, tm_cur, k.partials);
+}
+template <int MASK, int CT, int LEAN, typename Cfg>
+__global__ void __launch_bounds__(Cfg::kThreads, 1) fused_forward_ws_u8_kept_kernel(const FwdParamsU8 p, const KeptOut k,
+                                                                                 const __grid_constant__ CUtensorMap tm_bf,
+                                                                                 const __grid_constant__ CUtensorMap tm_ff,
+                                                                                 const __grid_constant__ CUtensorMap tm_prev,
+                                                                                 const __grid_constant__ CUtensorMap tm_cur) {
+  fused_forward_ws<uint8_t, MASK, true, CT, LEAN, Cfg, true>(p, tm_bf, tm_ff, tm_prev, tm_cur, k.partials);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -2110,6 +2249,12 @@ extern "C" size_t tclb200_scratch_bytes(int B, int H, int W) {
   const size_t tpp = (size_t)cdiv(W, 32) * cdiv(H, kWarps);
   return align_up((size_t)B * tpp * sizeof(double), 256) + align_up(((size_t)B + 3) * sizeof(unsigned), 256);
 }
+// ... and with the kept-pixel partials behind it (one more fp64 per tile)
+extern "C" size_t tclb200_scratch_bytes_kept(int B, int H, int W) {
+  if (B <= 0 || H <= 0 || W <= 0) return 0;
+  const size_t tpp = (size_t)cdiv(W, 32) * cdiv(H, kWarps);
+  return tclb200_scratch_bytes(B, H, W) + align_up((size_t)B * tpp * sizeof(double), 256);
+}
 
 // ---- tensor maps -------------------------------------------------------------------------------
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
@@ -2155,7 +2300,8 @@ static int sm_count() {   // of the current device, cached per device index (a p
   return v;
 }
 
-static cudaError_t launch_fold(const FwdParams& p, cudaStream_t s) {   // behind a kernel that stored one fp64 partial per tile
+// behind a kernel that stored one fp64 partial per tile (k: and one kept-pixel partial per tile, or nullptr)
+static cudaError_t launch_fold(const FwdParams& p, const KeptOut* k, cudaStream_t s) {
   ++g_launches;
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
@@ -2165,7 +2311,15 @@ static cudaError_t launch_fold(const FwdParams& p, cudaStream_t s) {   // behind
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr; cfg.numAttrs = 1;
+  if (k) return small ? cudaLaunchKernelEx(&cfg, fold_partials_small_kept_kernel, p, *k) : cudaLaunchKernelEx(&cfg, fold_partials_kept_kernel, p, *k);
   return small ? cudaLaunchKernelEx(&cfg, fold_partials_small_kernel, p) : cudaLaunchKernelEx(&cfg, fold_partials_kernel, p);
+}
+
+// kept-pixel sums of a call without a mask: every evaluated pixel counts 1, so pair b keeps rows * W and the batch B times that
+__global__ void __launch_bounds__(kThreads) fill_kept_kernel(double* pair_kept, double* total_kept, int B, double per_pair) {
+  for (int i = threadIdx.x; i < B; i += kThreads)
+    if (pair_kept) pair_kept[i] = per_pair;
+  if (threadIdx.x == 0 && total_kept) *total_kept = per_pair * (double)B;
 }
 
 extern "C" int tclb200_debug_tile_stats(unsigned long long* out2, int reset) {
@@ -2208,6 +2362,7 @@ struct FwdPlan {
   int mask_kind;
   bool reduce;
   int ct, var, cw;         // CT; variant (kVar*; the direct kernel's loss); consumer warps (TMA kernel: 8 or 16, else 0)
+  bool kept;               // the instantiation also sums the kept pixels (pair_kept / total_kept with a mask)
   WsGeo geo;               // TMA kernel: ws_geo(esize, mask_kind, ct, var, cw)
   int tiles_x, tiles_per_pair;
 };
@@ -2221,6 +2376,8 @@ static FwdPlan plan_forward(const tclb200_tcl_args* a, bool tma_ok) {
   q.mask_kind = a->ff ? MASK_COMPUTED : (a->mask_in ? MASK_GIVEN : MASK_NONE);
   q.reduce = a->cur && (a->pair_sums || a->total_sums || a->pair_vals || a->total_val);
   q.ct = a->prev && a->C == 3 ? 3 : 0;
+  // kept-pixel sums come from the kernels that see the mask (a call without one keeps rows * W pixels: no kernel needed)
+  q.kept = q.reduce && (a->pair_kept || a->total_kept) && q.mask_kind != MASK_NONE;
   const int rows = a->row_begin != 0 || a->row_end != 0 ? a->row_end - a->row_begin : a->H;
   // TMA needs 16-byte aligned bases and row strides; frames need C == 3 (the compiled box depth)
   const bool tma = tma_ok && g_force_generic != 1 && (a->W % 4 == 0) && ((a->W * q.esize) % 16 == 0) && aligned16(a->bf) &&
@@ -2228,7 +2385,7 @@ static FwdPlan plan_forward(const tclb200_tcl_args* a, bool tma_ok) {
                    a->H <= 16384 && a->W <= 16384;   // (box addresses are evaluated in fp32, see lean_tile)
   // short launches of the training loss (dataset mask, reduction only): the direct kernel, no tensor maps needed
   // (uint8 frames have no direct rows: a uint8 frame is a decoded video frame to be scored, not a training batch)
-  const bool direct = tma && g_force_generic != 2 && q.esize != 1 && q.mask_kind == MASK_GIVEN && q.reduce && a->C == 3 && !a->warp_out && !a->mask_out &&
+  const bool direct = tma && g_force_generic != 2 && q.esize != 1 && !q.kept && q.mask_kind == MASK_GIVEN && q.reduce && a->C == 3 && !a->warp_out && !a->mask_out &&
                       !a->blend_out && !a->near_threshold && !(a->flags & (TCLB200_VALIDITY | TCLB200_THROUGHPUT)) && aligned16(a->mask_in) &&
                       ((size_t)a->B * (size_t)rows * a->W <= TCL_DIRECT_MAX_PX || g_force_generic == 3);
   if (!tma) {
@@ -2265,6 +2422,14 @@ static FwdPlan plan_forward(const tclb200_tcl_args* a, bool tma_ok) {
   } else {
     q.var = kVarGeneral;
   }
+  // kept-pixel sums: the TMA kernel in its reducing hot variants; every other configuration takes the generic kernel
+  if (q.kept && q.var != kVarL2 && q.var != kVarL1) {
+    q.path = kPathGeneric;
+    q.var = kVarGeneral;
+    q.tiles_x = cdiv(a->W, 32);
+    q.tiles_per_pair = q.tiles_x * cdiv(rows, kWarps);
+    return q;
+  }
   // Consumer warps per CTA.  The packed-arithmetic configurations with a computed mask on fp32 frames run best with
   // 8 warps x 8 pixels per lane on large frames (Sintel shape: 130 vs 124 Gpix/s); small frames, where a larger share of
   // the tiles straddles a motion boundary and waits for global gathers (256 x 256 training crops: 87 vs 97), bf16 frames
@@ -2276,10 +2441,16 @@ static FwdPlan plan_forward(const tclb200_tcl_args* a, bool tma_ok) {
 }
 
 // ---- launch table --------------------------------------------------------------------------------
-template <int PATH, typename FrameT, int MASK, bool REDUCE, int CT, int VAR, int CW>
-static cudaError_t launch_forward(const FwdParams& p, const CUtensorMap* tm, cudaStream_t s) {
+template <int PATH, typename FrameT, int MASK, bool REDUCE, int CT, int VAR, int CW, bool KEPT = false>
+static cudaError_t launch_forward(const FwdParams& p, const KeptOut& k, const CUtensorMap* tm, cudaStream_t s) {
   const size_t tiles = (size_t)p.B * p.tiles_per_pair;
-  if constexpr (PATH == kPathGeneric && std::is_same<FrameT, uint8_t>::value) {
+  static_assert(!KEPT || (REDUCE && MASK != MASK_NONE && (PATH == kPathGeneric || VAR == kVarL2 || VAR == kVarL1)),
+                "kept-pixel rows: reductions with a mask; the generic kernel or the TMA kernel's reducing hot variants");
+  if constexpr (KEPT && PATH == kPathGeneric && std::is_same<FrameT, uint8_t>::value) {
+    fused_forward_generic_u8_kept_kernel<MASK><<<(unsigned)tiles, kThreads, 0, s>>>(static_cast<const FwdParamsU8&>(p), k);
+  } else if constexpr (KEPT && PATH == kPathGeneric) {
+    fused_forward_generic_kept_kernel<FrameT, MASK, CT><<<(unsigned)tiles, kThreads, 0, s>>>(p, k);
+  } else if constexpr (PATH == kPathGeneric && std::is_same<FrameT, uint8_t>::value) {
     static_assert(REDUCE && CT == 3, "uint8 frames: C == 3, reductions only");
     fused_forward_generic_u8_kernel<MASK><<<(unsigned)tiles, kThreads, 0, s>>>(static_cast<const FwdParamsU8&>(p));
   } else if constexpr (PATH == kPathGeneric) {
@@ -2290,7 +2461,7 @@ static cudaError_t launch_forward(const FwdParams& p, const CUtensorMap* tm, cud
     constexpr WsGeo G = ws_geo((int)sizeof(FrameT), MASK, CT, VAR, CW);
     using Cfg = WsCfg<FrameT, CT, kTW, kTH, G.bw, G.bh, G.nb, G.ns, G.cw, G.ff>;
     // (uint8 frames: the entry that takes FwdParamsU8, i.e. the parameters followed by the normalisation)
-    auto launch = [&](auto kern, const auto& params) -> cudaError_t {
+    auto launch = [&](auto kern, const auto&... params) -> cudaError_t {
       static bool configured[64] = {};  // per instantiation and device (the attribute is a per-device property of the function)
       int dev = 0;
       if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) dev = 63;   // (an uncached slot: set the attribute every time)
@@ -2301,11 +2472,15 @@ static cudaError_t launch_forward(const FwdParams& p, const CUtensorMap* tm, cud
       }
       // persistent: one CTA per SM (or fewer when there are fewer tiles)
       const size_t slots = (size_t)sm_count();
-      kern<<<(unsigned)(tiles < slots ? tiles : slots), Cfg::kThreads, Cfg::kSmemBytes, s>>>(params, tm[0], tm[1], tm[2], tm[3]);
+      kern<<<(unsigned)(tiles < slots ? tiles : slots), Cfg::kThreads, Cfg::kSmemBytes, s>>>(params..., tm[0], tm[1], tm[2], tm[3]);
       return cudaSuccess;
     };
     cudaError_t e0;
-    if constexpr (std::is_same<FrameT, uint8_t>::value) {
+    if constexpr (KEPT && std::is_same<FrameT, uint8_t>::value) {
+      e0 = launch(fused_forward_ws_u8_kept_kernel<MASK, CT, VAR, Cfg>, static_cast<const FwdParamsU8&>(p), k);
+    } else if constexpr (KEPT) {
+      e0 = launch(fused_forward_ws_kept_kernel<FrameT, MASK, CT, VAR, Cfg>, p, k);
+    } else if constexpr (std::is_same<FrameT, uint8_t>::value) {
       static_assert(REDUCE && CT == 3, "uint8 frames: C == 3, reductions only");
       e0 = launch(fused_forward_ws_u8_kernel<MASK, REDUCE, CT, VAR, Cfg>, static_cast<const FwdParamsU8&>(p));
     } else {
@@ -2316,14 +2491,15 @@ static cudaError_t launch_forward(const FwdParams& p, const CUtensorMap* tm, cud
   ++g_launches;
   const cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess || !REDUCE || PATH == kPathGeneric) return e;   // (the generic kernel folds its own partials)
-  return launch_fold(p, s);
+  return launch_fold(p, KEPT ? &k : nullptr, s);
 }
 
 struct FwdRow {
   int path, esize, mask;
   bool reduce;
   int ct, var, cw;
-  cudaError_t (*launch)(const FwdParams&, const CUtensorMap*, cudaStream_t);   // nullptr: not compiled into this build
+  bool kept;
+  cudaError_t (*launch)(const FwdParams&, const KeptOut&, const CUtensorMap*, cudaStream_t);   // nullptr: not compiled into this build
 };
 
 // Tuning builds with TCL_HOT_ONLY (tools/sweep_build.py) compile computeTCL's rows alone, on fp32 (1) or bf16 (2) frames:
@@ -2336,12 +2512,15 @@ constexpr bool row_compiled(int path, int esize, int mask, bool reduce, int ct, 
 #endif
 }
 
-template <int PATH, typename FrameT, int MASK, bool REDUCE, int CT, int VAR, int CW = 0>
+template <int PATH, typename FrameT, int MASK, bool REDUCE, int CT, int VAR, int CW = 0, bool KEPT = false>
 constexpr FwdRow row() {
   constexpr int E = (int)sizeof(FrameT);
-  if constexpr (row_compiled(PATH, E, MASK, REDUCE, CT, VAR)) return {PATH, E, MASK, REDUCE, CT, VAR, CW, launch_forward<PATH, FrameT, MASK, REDUCE, CT, VAR, CW>};
-  else return {PATH, E, MASK, REDUCE, CT, VAR, CW, nullptr};
+  if constexpr (row_compiled(PATH, E, MASK, REDUCE, CT, VAR)) return {PATH, E, MASK, REDUCE, CT, VAR, CW, KEPT, launch_forward<PATH, FrameT, MASK, REDUCE, CT, VAR, CW, KEPT>};
+  else return {PATH, E, MASK, REDUCE, CT, VAR, CW, KEPT, nullptr};
 }
+// a row of the kernels that also sum the kept pixels (pair_kept / total_kept)
+template <int PATH, typename FrameT, int MASK, int CT, int VAR, int CW = 0>
+constexpr FwdRow kept_row() { return row<PATH, FrameT, MASK, true, CT, VAR, CW, true>(); }
 
 using bf16 = __nv_bfloat16;
 // Every forward kernel instantiation there is, each once: the only place that names one.  TMA rows with CT == 0 do not
@@ -2397,11 +2576,26 @@ static constexpr FwdRow kFwdRows[] = {
     row<kPathTma, bf16, MASK_NONE, true, 3, kVarGeneral, 16>(),       row<kPathTma, bf16, MASK_NONE, false, 3, kVarGeneral, 16>(),
     row<kPathTma, bf16, MASK_NONE, false, 3, kVarL2, 16>(),           row<kPathTma, bf16, MASK_NONE, false, 0, kVarGeneral, 16>(),
     row<kPathTma, uint8_t, MASK_NONE, true, 3, kVarGeneral, 16>(),
+    // kept-pixel sums (ABI v9): the TMA kernel's reducing hot variants with the consumer warps plan_forward picks for them ...
+    kept_row<kPathTma, float, MASK_COMPUTED, 3, kVarL2, 8>(),  kept_row<kPathTma, float, MASK_COMPUTED, 3, kVarL2, 16>(),
+    kept_row<kPathTma, float, MASK_COMPUTED, 3, kVarL1, 8>(),  kept_row<kPathTma, float, MASK_COMPUTED, 3, kVarL1, 16>(),
+    kept_row<kPathTma, bf16, MASK_COMPUTED, 3, kVarL2, 16>(),  kept_row<kPathTma, bf16, MASK_COMPUTED, 3, kVarL1, 16>(),
+    kept_row<kPathTma, uint8_t, MASK_COMPUTED, 3, kVarL2, 16>(), kept_row<kPathTma, uint8_t, MASK_COMPUTED, 3, kVarL1, 16>(),
+    kept_row<kPathTma, float, MASK_GIVEN, 3, kVarL2, 16>(),    kept_row<kPathTma, float, MASK_GIVEN, 3, kVarL1, 16>(),
+    kept_row<kPathTma, bf16, MASK_GIVEN, 3, kVarL2, 16>(),     kept_row<kPathTma, bf16, MASK_GIVEN, 3, kVarL1, 16>(),
+    kept_row<kPathTma, uint8_t, MASK_GIVEN, 3, kVarL2, 16>(),  kept_row<kPathTma, uint8_t, MASK_GIVEN, 3, kVarL1, 16>(),
+    // ... and the generic kernel for everything else (shapes TMA cannot describe, C != 3, per-pixel outputs, other tests)
+    kept_row<kPathGeneric, float, MASK_COMPUTED, 3, kVarGeneral>(), kept_row<kPathGeneric, float, MASK_COMPUTED, 0, kVarGeneral>(),
+    kept_row<kPathGeneric, float, MASK_GIVEN, 3, kVarGeneral>(),    kept_row<kPathGeneric, float, MASK_GIVEN, 0, kVarGeneral>(),
+    kept_row<kPathGeneric, bf16, MASK_COMPUTED, 3, kVarGeneral>(),  kept_row<kPathGeneric, bf16, MASK_COMPUTED, 0, kVarGeneral>(),
+    kept_row<kPathGeneric, bf16, MASK_GIVEN, 3, kVarGeneral>(),     kept_row<kPathGeneric, bf16, MASK_GIVEN, 0, kVarGeneral>(),
+    kept_row<kPathGeneric, uint8_t, MASK_COMPUTED, 3, kVarGeneral>(), kept_row<kPathGeneric, uint8_t, MASK_GIVEN, 3, kVarGeneral>(),
 };
 
 static const FwdRow* find_row(const FwdPlan& q) {
   for (const FwdRow& r : kFwdRows)
-    if (r.path == q.path && r.esize == q.esize && r.mask == q.mask_kind && r.reduce == q.reduce && r.ct == q.ct && r.var == q.var && r.cw == q.cw)
+    if (r.path == q.path && r.esize == q.esize && r.mask == q.mask_kind && r.reduce == q.reduce && r.ct == q.ct && r.var == q.var && r.cw == q.cw &&
+        r.kept == q.kept)
       return r.launch ? &r : nullptr;
   return nullptr;
 }
@@ -2434,6 +2628,11 @@ static int run_fused(const tclb200_tcl_args* a, cudaStream_t s) {
     return fail(TCLB200_ERR_INVALID, "band mode needs 0 <= row_begin < row_end <= H");
   if (band && (a->pair_vals || a->total_val)) return fail(TCLB200_ERR_INVALID, "band mode returns sums only (pair_sums / total_sums): a band's mean is not the frame's");
   if ((size_t)a->H * a->W >= (1u << 30)) return fail(TCLB200_ERR_UNSUPPORTED, "H*W must be below 2^30");
+  const bool want_kept = a->pair_kept || a->total_kept;
+  if (want_kept && !(a->cur && (a->pair_sums || a->total_sums || a->pair_vals || a->total_val)))
+    return fail(TCLB200_ERR_INVALID, "pair_kept / total_kept need a reduction (cur and pair_sums / total_sums / pair_vals / total_val)");
+  if (want_kept && (!a->scratch || a->scratch_bytes < tclb200_scratch_bytes_kept(a->B, a->H, a->W)))
+    return fail(TCLB200_ERR_INVALID, "pair_kept / total_kept: scratch missing or smaller than tclb200_scratch_bytes_kept(B,H,W)");
   if (a->ff && !(a->flags & (TCLB200_OCC | TCLB200_MOB)))
     return fail(TCLB200_ERR_INVALID, "ff given but neither TCLB200_OCC nor TCLB200_MOB requested");
   if (!a->prev && !a->mask_out) return fail(TCLB200_ERR_INVALID, "nothing to compute: no frames and no mask_out");
@@ -2493,11 +2692,22 @@ static int run_fused(const tclb200_tcl_args* a, cudaStream_t s) {
     const size_t tiles = (size_t)p.B * p.tiles_per_pair;
     p.scratch.tile_ctr = (plan.path == kPathTma && tiles > 16 * (size_t)sm_count()) ? p.scratch.batch_ticket + 1 : nullptr;
   }
+  KeptOut k;
+  memset(&k, 0, sizeof(k));
+  if (plan.kept) {   // (behind the scratch of tclb200_scratch_bytes: tclb200_scratch_bytes_kept was checked above)
+    k.partials = reinterpret_cast<double*>(reinterpret_cast<char*>(a->scratch) + tclb200_scratch_bytes(a->B, a->H, a->W));
+    k.pair_kept = a->pair_kept; k.total_kept = a->total_kept;
+  }
   const FwdRow* row = find_row(plan);
   if (!row) return fail(TCLB200_ERR_UNSUPPORTED, "no forward kernel is compiled for this configuration (build: %s)", tclb200_build_info());
-  const cudaError_t e = row->launch(p, tm, s);
+  const cudaError_t e = row->launch(p, k, tm, s);
   if (e != cudaSuccess)
     return fail(TCLB200_ERR_CUDA, plan.path == kPathDirect ? "fused forward (direct) launch: %s" : "fused forward launch: %s", cudaGetErrorString(e));
+  if (want_kept && !plan.kept) {   // no mask: every evaluated pixel is kept
+    fill_kept_kernel<<<1, kThreads, 0, s>>>(a->pair_kept, a->total_kept, a->B, (double)(p.row_end - p.row_begin) * a->W);
+    ++g_launches;
+    CUDA_TRY(cudaGetLastError());
+  }
   return TCLB200_OK;
 }
 

@@ -14,6 +14,7 @@ it replaces (upstream paths relative to the repository root):
 * ``warp_blend(...)``                     methods/optimization-based/obst_eval.py:500
 * ``generateMask(simg, prev, flow)``      ConGAN/models/cycle_gan_model.py:136-137 with the warp fused in
 * ``temporal_error_host(...)``            the evaluation loop of utils/sintel_eval.py:206-222 with HOST tensors in and out
+* ``warping_error_per_pair(...)``         the masked warping error normalised by the kept pixels (Lai et al., ECCV 2018)
 
 PyTorch is used for device memory, streams and autograd plumbing only; all arithmetic runs in
 ``csrc/tcl_kernels.cu``.  There is no CPU path: CPU tensors raise, like the reference's hard-coded
@@ -107,9 +108,11 @@ def _u8_norm(dt, u8_scale, u8_offset, C):
     return three(u8_scale, U8_SCALE, "u8_scale"), three(u8_offset, 0.0, "u8_offset")
 
 
-def _scratch(B, H, W, device):
-    """Zero-filled ticket/partials scratch, cached per (device, stream); kernels leave it zeroed."""
-    need = _cabi.lib().tclb200_scratch_bytes(B, H, W)
+def _scratch(B, H, W, device, kept=False):
+    """Zero-filled ticket/partials scratch, cached per (device, stream); kernels leave it zeroed.  ``kept``: large enough for
+    the kept-pixel partials too."""
+    lib = _cabi.lib()
+    need = lib.tclb200_scratch_bytes_kept(B, H, W) if kept else lib.tclb200_scratch_bytes(B, H, W)
     key = (device.index, torch.cuda.current_stream(device).cuda_stream)
     buf = _scratch_cache.get(key)
     if buf is None or buf.numel() < need:
@@ -300,7 +303,8 @@ def upsample_flow(flow, mask):
 # ------------------------------------------------------------------------------------------------
 class FusedResult:
     """Device-resident results of one fused launch (nothing is synchronised)."""
-    __slots__ = ("pair_vals", "total_val", "pair_sums", "total_sums", "warp", "mask", "blend", "near_threshold")
+    __slots__ = ("pair_vals", "total_val", "pair_sums", "total_sums", "warp", "mask", "blend", "near_threshold", "pair_kept",
+                 "total_kept")
 
     def __init__(self):
         for s in self.__slots__:
@@ -320,7 +324,7 @@ def _index(idx, B, n_frames, name, validate=True):
 def fused_forward(bf, prev, cur, ff=None, mask=None, loss=L2, finalize=FIN_RMSE, flags=OCC | MOB,
                   want_warp=False, want_mask=False, want_blend=False, want_near=False, want_sums=True,
                   prev_index=None, cur_index=None, validate_index=True, bf_index=None, ff_index=None, pair_group=0, rows=None,
-                  u8_scale=None, u8_offset=None):
+                  u8_scale=None, u8_offset=None, want_kept=False):
     """One launch: warp ``prev`` by ``bf``, build or read the mask, reduce the masked error against ``cur``.
 
     ``ff`` given -> the mask is computed (fbcCheckTorch semantics, tests per ``flags``);
@@ -340,6 +344,10 @@ def fused_forward(bf, prev, cur, ff=None, mask=None, loss=L2, finalize=FIN_RMSE,
     uint8 frames (B,3,H,W) -- stored video: PNGs, decoded clips -- are scored as ``u.float() * u8_scale + u8_offset`` (per
     channel; a float or 3 floats; default 1/255 and 0, i.e. [0, 1]); the result is the fp32 path's on the normalised frames.
     Reductions only: ``want_warp`` / ``want_blend`` raise, ``want_sums`` must stay on.
+
+    ``want_kept=True`` also fills ``pair_kept`` (B,) and ``total_kept`` (0-dim), fp64 on the device: the sum of the mask over
+    each pair's evaluated pixels (the rows of ``rows`` in band mode) -- the count of pixels the computed mask keeps, the sum
+    of the dataset mask, or the pixel count without a mask.  It needs ``want_sums`` and works in every mode above.
     """
     _require_cuda(bf, prev, cur, ff, mask, bf_index, ff_index)
     bf, bf_plane, bf_batch = _flow_view(bf, "bf")
@@ -373,6 +381,8 @@ def fused_forward(bf, prev, cur, ff=None, mask=None, loss=L2, finalize=FIN_RMSE,
     else:
         mask = None
     res = FusedResult()
+    if want_kept and not want_sums:
+        raise RuntimeError("tcl_b200: want_kept needs want_sums (the kept-pixel sums come with the reduction)")
     if rows is not None:
         r0, r1 = int(rows[0]), int(rows[1])
         if not (0 <= r0 < r1 <= H):
@@ -383,6 +393,9 @@ def fused_forward(bf, prev, cur, ff=None, mask=None, loss=L2, finalize=FIN_RMSE,
         if rows is None:
             f32 = torch.empty(B + 1, dtype=torch.float32, device=dev)
             res.pair_vals, res.total_val = f32[:B], f32[B]
+    if want_kept:
+        k64 = torch.empty(B + 1, dtype=torch.float64, device=dev)
+        res.pair_kept, res.total_kept = k64[:B], k64[B]
     if want_warp:
         res.warp = torch.empty_like(prev) if out_like is None else torch.empty_like(out_like)
     if want_mask:
@@ -392,7 +405,7 @@ def fused_forward(bf, prev, cur, ff=None, mask=None, loss=L2, finalize=FIN_RMSE,
     if want_near:
         res.near_threshold = torch.zeros(1, dtype=torch.int64, device=dev)
     with torch.cuda.device(dev):
-        scratch = _scratch(B, H, W, dev) if want_sums else None
+        scratch = _scratch(B, H, W, dev, kept=want_kept) if want_sums else None
         a = TclArgs()
         a.ff, a.bf, a.mask_in, a.prev, a.cur = _ptr(ff), _ptr(bf), _ptr(mask), _ptr(prev), _ptr(cur)
         a.warp_out, a.mask_out, a.blend_out = _ptr(res.warp), _ptr(res.mask), _ptr(res.blend)
@@ -412,6 +425,7 @@ def fused_forward(bf, prev, cur, ff=None, mask=None, loss=L2, finalize=FIN_RMSE,
         if rows is not None:
             a.row_begin, a.row_end = r0, r1
         a.u8_scale[:], a.u8_offset[:] = norm
+        a.pair_kept, a.total_kept = _ptr(res.pair_kept), _ptr(res.total_kept)
         check(_cabi.lib().tclb200_tcl_forward(ctypes.byref(a), _stream_handle()))
     return res
 
@@ -425,6 +439,24 @@ def temporal_error(ff, bf, prev, cur, u8_scale=None, u8_offset=None):
 def temporal_error_per_pair(ff, bf, prev, cur, u8_scale=None, u8_offset=None):
     """Per-pair RMSE (B,) with the mask computed from (ff,bf) -- the batched form of ``computeTCL``."""
     return fused_forward(bf, prev, cur, ff=ff, finalize=FIN_RMSE, u8_scale=u8_scale, u8_offset=u8_offset).pair_vals
+
+
+def warping_error_per_pair(ff, bf, prev, cur, mask=None, loss=L2, finalize=FIN_RMSE, u8_scale=None, u8_offset=None):
+    """Per-pair warping error normalised by the KEPT pixels (B,) fp32: ``S_b / (C * kept_b)``, square-rooted for
+    ``finalize=FIN_RMSE`` -- the form of the video-consistency literature (Lai et al., ECCV 2018, and the style-transfer
+    papers that follow it).  S_b is the masked error sum of ``pair_sums`` (sum of (m*(cur - warp(prev,bf)))**2 for L2,
+    sum of m*|warp - cur| for L1) and kept_b the sum of the mask m over the pair's pixels.
+
+    ``temporal_error_per_pair`` (``computeTCL``, utils/sintel_eval.py:110) divides the same S_b by all C*H*W values instead,
+    so there a clip with heavy occlusion looks more consistent than one without; here the discarded pixels do not count.
+    The mask is computed from (``ff``, ``bf``) as in ``fbcCheckTorch``; with ``ff=None`` it is the dataset mask ``mask``
+    (B,1,H,W), or 1 everywhere when that is None too.  A soft dataset mask keeps the reference's own numerator,
+    sum of (m*d)**2, over sum of m.  A pair whose mask keeps nothing gives NaN (0/0), as the torch expression does.
+    uint8 frames: ``u8_scale`` / ``u8_offset`` as in ``fused_forward``."""
+    res = fused_forward(bf, prev, cur, ff=ff, mask=mask, loss=loss, finalize=finalize, want_kept=True, u8_scale=u8_scale,
+                        u8_offset=u8_offset)
+    err = res.pair_sums / (prev.shape[1] * res.pair_kept)
+    return (err.sqrt() if finalize == FIN_RMSE else err).float()
 
 
 def temporal_error_clip(frames, ff, bf, u8_scale=None, u8_offset=None):
@@ -522,7 +554,7 @@ def _host_tensor(t, name, dtype=None, channels_last_ok=False):
 
 def temporal_error_host(frames, ff, bf, prev_index=None, cur_index=None, mask=None, loss=L2, finalize=FIN_RMSE,
                         flags=OCC | MOB, chunk_pairs=0, device=None, sync=True, return_sums=False, max_device_frames=None,
-                        u8_scale=None, u8_offset=None):
+                        u8_scale=None, u8_offset=None, return_kept=False):
     """The evaluation loop of utils/sintel_eval.py:206-222 (and solver.py:336-347) on HOST tensors.
 
     ``frames`` (F,C,H,W) fp32/bf16, or (F,3,H,W) uint8 with ``u8_scale`` / ``u8_offset`` as in ``fused_forward`` (a third of
@@ -538,6 +570,9 @@ def temporal_error_host(frames, ff, bf, prev_index=None, cur_index=None, mask=No
     values per ``finalize``.  One C-ABI call (``tclb200_tcl_forward_host``) pipelines H2D copies and fused launches
     on ``device`` (default: the current CUDA device); there is no CPU arithmetic anywhere.
     ``return_sums=True`` returns ``(values, sums)`` with the per-pair float64 sums S_p as well (for pooled statistics).
+    ``return_kept=True`` appends each pair's kept-pixel sum (pinned float64 (P,), as ``fused_forward``'s ``pair_kept``) as the
+    last element: ``(values, kept)`` or ``(values, sums, kept)``; ``sums / (C * kept)`` is then the warping error normalised
+    by the kept pixels (see ``warping_error_per_pair``).
     ``max_device_frames``: device frame slots.  None = the whole frame bank stays resident when it takes at most a
     quarter of the free device memory, else a ring of as many frames as that quarter holds (long or 4K clips: a slot is
     reused once every chunk that reads its frame has completed; at least four chunks' worth of frames must fit).
@@ -571,33 +606,36 @@ def temporal_error_host(frames, ff, bf, prev_index=None, cur_index=None, mask=No
     dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
     lib = _cabi.lib()
     if P == 0:
-        out = torch.empty(0, dtype=torch.float32, pin_memory=True)
-        return (out, torch.empty(0, dtype=torch.float64, pin_memory=True)) if return_sums else out
+        out = (torch.empty(0, dtype=torch.float32, pin_memory=True),)
+        out += (torch.empty(0, dtype=torch.float64, pin_memory=True),) * (int(return_sums) + int(return_kept))
+        return out if len(out) > 1 else out[0]
     cl = ((_cabi.CL_FRAMES if _is_channels_last(frames) else 0) | (_cabi.CL_FF if ff is not None and _is_channels_last(ff) else 0)
           | (_cabi.CL_BF if _is_channels_last(bf) else 0))
     slots = F_
     ws = _host_ws_cache.get(dev.index)
     with_mask = 1 if mask is not None else 0
+    ws_bytes = lib.tclb200_host_workspace_bytes_kept if return_kept else lib.tclb200_host_workspace_bytes_cl
     if max_device_frames is not None:
         slots = max(1, min(F_, int(max_device_frames)))
-    elif ws is None or ws.numel() < lib.tclb200_host_workspace_bytes_cl(P, F_, C, H, W, dt, chunk_pairs, with_mask, cl):
+    elif ws is None or ws.numel() < ws_bytes(P, F_, C, H, W, dt, chunk_pairs, with_mask, cl):
         # only when a workspace has to be allocated: cudaMemGetInfo costs 1.5 ms at the median and 20-90 ms in one call of ten
         # (measured, tools/e2e_stall_probe.py) -- per step it was the whole difference between a 6 ms step and a 12 ms one
         frame_bytes = C * H * W * frames.element_size()
         free_b = torch.cuda.mem_get_info(dev)[0] + (ws.numel() if ws is not None else 0)
         # channels-last data also needs its staging areas and planar flow buffers; with a whole bank they are at their
         # largest, so a ring sized against them fits too
-        extra = (lib.tclb200_host_workspace_bytes_cl(P, F_, C, H, W, dt, chunk_pairs, with_mask, cl)
+        extra = (ws_bytes(P, F_, C, H, W, dt, chunk_pairs, with_mask, cl)
                  - lib.tclb200_host_workspace_bytes(P, F_, C, H, W, dt, chunk_pairs, with_mask))
         if F_ * frame_bytes + extra > free_b // 4:
             slots = max(1, min(F_, (free_b // 4 - extra) // frame_bytes))
-    need = lib.tclb200_host_workspace_bytes_cl(P, slots, C, H, W, dt, chunk_pairs, with_mask, cl)
+    need = ws_bytes(P, slots, C, H, W, dt, chunk_pairs, with_mask, cl)
     if ws is None or ws.numel() < need:
         _host_ws_cache.pop(dev.index, None)
         ws = torch.empty(need, dtype=torch.uint8, device=dev)
         _host_ws_cache[dev.index] = ws
     out = torch.empty(P, dtype=torch.float32, pin_memory=True)
     sums = torch.empty(P, dtype=torch.float64, pin_memory=True) if return_sums else None
+    kept = torch.empty(P, dtype=torch.float64, pin_memory=True) if return_kept else None
     a = HostArgs()
     a.ff, a.bf, a.mask_in, a.frames = _ptr(ff), _ptr(bf), _ptr(mask), _ptr(frames)
     a.prev_index, a.cur_index = _ptr(prev_index), _ptr(cur_index)
@@ -608,6 +646,7 @@ def temporal_error_host(frames, ff, bf, prev_index=None, cur_index=None, mask=No
     a.frame_slots = 0 if slots >= F_ else slots
     a.u8_scale[:], a.u8_offset[:] = norm
     a.channels_last = cl
+    a.pair_kept = _ptr(kept)
     with torch.cuda.device(dev):
         stream = torch.cuda.current_stream()
         check(lib.tclb200_tcl_forward_host(ctypes.byref(a), ctypes.c_void_p(stream.cuda_stream)))
@@ -615,7 +654,8 @@ def temporal_error_host(frames, ff, bf, prev_index=None, cur_index=None, mask=No
             stream.synchronize()
         else:   # the caller synchronises the stream; keep the host inputs alive until then
             out._tcl_keepalive = (frames, ff, bf, mask, prev_index, cur_index)
-    return (out, sums) if return_sums else out
+    res = (out,) + ((sums,) if return_sums else ()) + ((kept,) if return_kept else ())
+    return res if len(res) > 1 else out
 
 
 def temporal_rmse_per_sample(mask, cur, prev, flow, u8_scale=None, u8_offset=None):

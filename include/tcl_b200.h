@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define TCLB200_ABI_VERSION 8
+#define TCLB200_ABI_VERSION 9
 
 #define TCLB200_OK 0
 #define TCLB200_ERR_INVALID 1     /* bad argument (null pointer, non-positive size, unknown enum) */
@@ -75,6 +75,9 @@ const char* tclb200_build_info(void);
 /* bytes of device scratch tclb200_tcl_forward needs for a (B,H,W) problem.  The scratch must be
  * zero-filled once when allocated; every call leaves it zeroed again. */
 size_t tclb200_scratch_bytes(int B, int H, int W);
+/* the same for calls that request kept-pixel sums (tclb200_tcl_args.pair_kept / total_kept, ABI v9): the scratch above plus
+ * one more fp64 partial per tile behind it */
+size_t tclb200_scratch_bytes_kept(int B, int H, int W);
 
 /* gradient(x)  utils/flowtools.py:12-16
  * x (B,H,W) fp32 -> out (2,B,H,W) fp32 = [d/dx, d/dy], zero-padded central differences. */
@@ -172,6 +175,15 @@ typedef struct tclb200_tcl_args {
    * work as for fp32 frames, and the result is the fp32 path's on the normalised frames. */
   float u8_scale[3];
   float u8_offset[3];
+  /* kept-pixel sums (device, NULL to skip; ABI v9): pair_kept[b] = sum of the mask m over pair b's evaluated pixels (band mode:
+   * rows [row_begin, row_end) only), in fp64 -- m is the computed verdict (0 / 1: an exact pixel count), the dataset mask's fp32
+   * value, or 1 without a mask; total_kept[0] = sum_b pair_kept[b].  The summation order is fixed (per tile, then tiles in index
+   * order) and independent of the tile schedule, so band sums add up to the whole frame's exactly.  With them
+   * S_b / (C * pair_kept[b]) is the warping error normalised by the kept pixels (the video-consistency literature's form) where
+   * pair_vals divides by all C*H*W.  They need a reduction (cur and one of pair_sums / total_sums / pair_vals / total_val) and a
+   * scratch of tclb200_scratch_bytes_kept(B,H,W) bytes (TCLB200_ERR_INVALID otherwise, before any CUDA call). */
+  double* pair_kept;    /* [B] */
+  double* total_kept;   /* [1] */
 } tclb200_tcl_args;
 
 int tclb200_tcl_forward(const tclb200_tcl_args* args, tclb200_stream_t stream);
@@ -214,6 +226,9 @@ typedef struct tclb200_host_args {
    * (C <= 64); TCLB200_CL_FF / TCLB200_CL_BF: that flow is (P,H,W,2) (TCLB200_CL_FF needs `ff`).  Unknown bits are
    * TCLB200_ERR_INVALID.  The workspace must be sized by tclb200_host_workspace_bytes_cl with the same bits. */
   int channels_last;
+  /* [P] out, HOST, or NULL (ABI v9): each pair's kept-pixel sum, as tclb200_tcl_args.pair_kept -- the same values whatever the
+   * chunking, frame ring or layout.  The workspace must be sized by tclb200_host_workspace_bytes_kept. */
+  double* pair_kept;
 } tclb200_host_args;
 
 #define TCLB200_CL_FRAMES 1
@@ -229,6 +244,9 @@ size_t tclb200_host_workspace_bytes(int P, int F, int C, int H, int W, int dtype
  * launch, chunk_pairs or its default, at most P).  Every part is rounded up to 256 bytes.  0 for unknown bits. */
 size_t tclb200_host_workspace_bytes_cl(int P, int F, int C, int H, int W, int dtype, int chunk_pairs, int with_mask,
                                        int channels_last);
+/* the same for calls that set pair_kept (ABI v9): one more fp64 per pair and the kept-pixel scratch of each launch */
+size_t tclb200_host_workspace_bytes_kept(int P, int F, int C, int H, int W, int dtype, int chunk_pairs, int with_mask,
+                                         int channels_last);
 int tclb200_tcl_forward_host(const tclb200_host_args* args, tclb200_stream_t stream);
 
 /* Backward of the fused training loss  L = grad_scale * sum (m*(cur-warp(prev,bf)))^2   (L2)
