@@ -15,6 +15,7 @@ from .chains import reconet_output_temporal_loss, ruder_network_input, long_term
 from . import synth  # noqa: F401
 from . import ingest  # noqa: F401
 from . import cv2compat  # noqa: F401
+from . import library  # noqa: F401  (registers the torch.ops.tcl_b200 operators)
 from .ingest import hwc_split, split_fc2_block, flow_hw2_to_planar, load_flo_planar, sintel_occlusion_mask  # noqa: F401
 
 __all__ = ["gradient", "warp", "fbcCheckTorch", "fbcCheckTorch_mob", "fs_warp", "fused_forward",

@@ -16,7 +16,7 @@ import torch
 
 from . import _cabi
 from ._cabi import check
-from .ops import L2, VALIDITY, _flow, _ptr, _require_cuda, _stream_handle, _warp_backward_raw
+from .ops import L2, VALIDITY, _cache_pool, _flow, _ptr, _require_cuda, _stream_handle, _traced, _warp_backward_raw
 
 _scratch = {}
 
@@ -40,19 +40,7 @@ class _ReconetLossFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, styled2, styled1, img2, img1, flow, mask):
-        B, _, H, W = flow.shape
-        lib = _cabi.lib()
-        need = lib.tclb200_reconet_scratch_bytes(B, H, W)
-        key = (flow.device.index, torch.cuda.current_stream().cuda_stream)
-        buf = _scratch.get(key)
-        if buf is None or buf.numel() < need:
-            buf = torch.empty(need, dtype=torch.uint8, device=flow.device)
-            _scratch[key] = buf
-        lum = torch.empty((B, 1, H, W), dtype=torch.float32, device=flow.device)
-        loss = torch.empty((), dtype=torch.float32, device=flow.device)
-        with torch.cuda.device(flow.device):
-            check(lib.tclb200_reconet_loss(_ptr(flow), _ptr(mask), _ptr(styled1), _ptr(styled2), _ptr(img1), _ptr(img2), _ptr(lum), _ptr(loss),
-                                           None, _ptr(buf), buf.numel(), B, H, W, _stream_handle()))
+        loss, lum = _reconet_forward(styled2, styled1, img2, img1, flow, mask)
         ctx.save_for_backward(styled1, styled2, flow, mask, lum)
         return loss
 
@@ -60,17 +48,42 @@ class _ReconetLossFn(torch.autograd.Function):
     @torch.autograd.function.once_differentiable
     def backward(ctx, grad_out):
         styled1, styled2, flow, mask, lum = ctx.saved_tensors
-        B, C, H, W = styled1.shape
-        g2 = torch.empty_like(styled2) if ctx.needs_input_grad[0] else None
-        g1 = torch.empty_like(styled1) if ctx.needs_input_grad[1] else None
-        # d loss / d (styled2 - warp(styled1)) = 2/N * mask^2 * ((styled2 - lum) - warp(styled1)): the fused training-loss
-        # backward with `cur` = styled2 - lum (the luminance term carries no gradient: the images are data)
-        cur = styled2 - lum
-        scale = (grad_out.float() / float(B * C * H * W)).reshape(1).contiguous()
-        with torch.cuda.device(styled1.device):
-            check(_cabi.lib().tclb200_tcl_backward(_ptr(flow), _ptr(mask), _ptr(styled1), _ptr(cur), _ptr(scale), _ptr(g1), _ptr(g2),
-                                                   B, C, H, W, VALIDITY, L2, _stream_handle()))
+        g2, g1 = _reconet_backward(grad_out, styled1, styled2, flow, mask, lum, ctx.needs_input_grad[0], ctx.needs_input_grad[1])
         return g2, g1, None, None, None, None
+
+
+def _reconet_forward(styled2, styled1, img2, img1, flow, mask):
+    """-> (loss, lum): the 0-dim loss and the luminance term its backward reads."""
+    B, _, H, W = flow.shape
+    lib = _cabi.lib()
+    need = lib.tclb200_reconet_scratch_bytes(B, H, W)
+    key = (flow.device.index, torch.cuda.current_stream().cuda_stream)
+    buf = _scratch.get(key)
+    if buf is None or buf.numel() < need:
+        with _cache_pool(flow.device):
+            buf = torch.empty(need, dtype=torch.uint8, device=flow.device)
+        _scratch[key] = buf
+    lum = torch.empty((B, 1, H, W), dtype=torch.float32, device=flow.device)
+    loss = torch.empty((), dtype=torch.float32, device=flow.device)
+    with torch.cuda.device(flow.device):
+        check(lib.tclb200_reconet_loss(_ptr(flow), _ptr(mask), _ptr(styled1), _ptr(styled2), _ptr(img1), _ptr(img2), _ptr(lum), _ptr(loss),
+                                       None, _ptr(buf), buf.numel(), B, H, W, _stream_handle()))
+    return loss, lum
+
+
+def _reconet_backward(grad_out, styled1, styled2, flow, mask, lum, need2, need1):
+    """(grad_styled2, grad_styled1), None where not needed."""
+    B, C, H, W = styled1.shape
+    g2 = torch.empty_like(styled2) if need2 else None
+    g1 = torch.empty_like(styled1) if need1 else None
+    # d loss / d (styled2 - warp(styled1)) = 2/N * mask^2 * ((styled2 - lum) - warp(styled1)): the fused training-loss
+    # backward with `cur` = styled2 - lum (the luminance term carries no gradient: the images are data)
+    cur = styled2 - lum
+    scale = (grad_out.float() / float(B * C * H * W)).reshape(1).contiguous()
+    with torch.cuda.device(styled1.device):
+        check(_cabi.lib().tclb200_tcl_backward(_ptr(flow), _ptr(mask), _ptr(styled1), _ptr(cur), _ptr(scale), _ptr(g1), _ptr(g2),
+                                               B, C, H, W, VALIDITY, L2, _stream_handle()))
+    return g2, g1
 
 
 def reconet_output_temporal_loss(mask, styled2, styled1, img2, img1, flow):
@@ -86,18 +99,15 @@ def reconet_output_temporal_loss(mask, styled2, styled1, img2, img1, flow):
     m = _mask1(mask, B, H, W)
     if torch.is_grad_enabled() and (flow.requires_grad or (m is not None and m.requires_grad) or i1.requires_grad or i2.requires_grad):
         raise RuntimeError("tcl_b200: reconet_output_temporal_loss differentiates w.r.t. the stylised frames only")
+    if _traced(s2, s1, i2, i1, flow, m):
+        return torch.ops.tcl_b200.reconet_loss(s2, s1, i2, i1, flow, m)[0]
     return _ReconetLossFn.apply(s2, s1, i2, i1, flow, m)
 
 
 class _RuderInputFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, styled_prev, img, mask, flow):
-        B, _, H, W = flow.shape
-        cat = torch.empty((B, 7, H, W), dtype=torch.float32, device=flow.device)
-        warped = torch.empty((B, 3, H, W), dtype=torch.float32, device=flow.device)
-        with torch.cuda.device(flow.device):
-            check(_cabi.lib().tclb200_ruder_input(_ptr(img), _ptr(mask), _ptr(styled_prev), _ptr(flow), _ptr(cat), _ptr(warped), B, H, W,
-                                                  _stream_handle()))
+        cat, warped = _ruder_forward(styled_prev, img, mask, flow)
         ctx.save_for_backward(styled_prev, flow)
         ctx.mark_non_differentiable()
         return cat, warped
@@ -115,6 +125,16 @@ class _RuderInputFn(torch.autograd.Function):
         return gx, None, None, None
 
 
+def _ruder_forward(styled_prev, img, mask, flow):
+    B, _, H, W = flow.shape
+    cat = torch.empty((B, 7, H, W), dtype=torch.float32, device=flow.device)
+    warped = torch.empty((B, 3, H, W), dtype=torch.float32, device=flow.device)
+    with torch.cuda.device(flow.device):
+        check(_cabi.lib().tclb200_ruder_input(_ptr(img), _ptr(mask), _ptr(styled_prev), _ptr(flow), _ptr(cat), _ptr(warped), B, H, W,
+                                              _stream_handle()))
+    return cat, warped
+
+
 def ruder_network_input(img, mask, styled_prev, flow):
     """One step of Ruder's chain (fs_ruder.py:50-75): returns ``(torch.cat((img, mask, warped), 1), warped)`` with
     ``warped = warp(styled_prev, flow)`` (fs_lib.warp), written in one pass.  ``warped`` is the ``loss_warped`` of the
@@ -128,6 +148,8 @@ def ruder_network_input(img, mask, styled_prev, flow):
     m = _mask1(mask, B, H, W)
     if torch.is_grad_enabled() and (flow.requires_grad or img.requires_grad or (m is not None and m.requires_grad)):
         raise RuntimeError("tcl_b200: ruder_network_input differentiates w.r.t. styled_prev only (images, masks and flows are data)")
+    if _traced(img, sp, m, flow):
+        return tuple(torch.ops.tcl_b200.ruder_input(sp, img, m, flow))
     return _RuderInputFn.apply(sp, img, m, flow)
 
 

@@ -21,6 +21,8 @@ PyTorch is used for device memory, streams and autograd plumbing only; all arith
 ``.cuda()`` (flowtools.py:25) does on a box without a GPU.
 """
 import ctypes
+import math
+import struct
 
 import torch
 
@@ -28,6 +30,16 @@ from . import _cabi
 from ._cabi import BF16, F32, FIN_MEAN, FIN_RMSE, L1, L2, MOB, OCC, U8, VALIDITY, HostArgs, TclArgs, check
 
 _scratch_cache = {}
+_cache_pools = {}
+
+
+def _cache_pool(device):
+    """The memory pool of the buffers cached across calls.  Such a buffer outlives the CUDA graph capture (or cudagraph-tree
+    warm-up) of the call that first needs it, so it must not come from that graph's private pool."""
+    pool = _cache_pools.get(device.index)
+    if pool is None:
+        pool = _cache_pools[device.index] = torch.cuda.MemPool()
+    return torch.cuda.use_mem_pool(pool, device)
 
 
 def _stream_handle():
@@ -36,6 +48,13 @@ def _stream_handle():
 
 def _ptr(t):
     return ctypes.c_void_p(t.data_ptr()) if t is not None else None
+
+
+def _traced(*tensors):
+    """True when the call is being traced (TorchDynamo, FakeTensor / meta / export tracing, functionalisation): it then goes
+    through the ``torch.ops.tcl_b200`` operators of ``library.py``, which the tracer sees.  Eager calls keep the direct
+    route, which skips the dispatcher's per-call cost (DESIGN.md section 5)."""
+    return torch.compiler.is_compiling() or any(t is not None and type(t) is not torch.Tensor for t in tensors)
 
 
 def _require_cuda(*tensors):
@@ -101,10 +120,13 @@ def _u8_norm(dt, u8_scale, u8_offset, C):
             v = v * 3
         if len(v) != 3:
             raise RuntimeError(f"tcl_b200: {name} must be a float or 3 floats, got {len(v)}")
-        v = torch.tensor(v, dtype=torch.float32)   # (the values the kernels use: rounded to fp32 once)
-        if not bool(torch.isfinite(v).all()):
+        try:   # the values the kernels use: rounded to fp32 once (plain Python, so that tracing sees constants)
+            v = [struct.unpack("f", struct.pack("f", x))[0] for x in v]
+        except OverflowError:   # rounds to +-inf
+            v = [math.inf]
+        if not all(math.isfinite(x) for x in v):
             raise RuntimeError(f"tcl_b200: {name} must be finite")
-        return tuple(float(x) for x in v)
+        return tuple(v)
     return three(u8_scale, U8_SCALE, "u8_scale"), three(u8_offset, 0.0, "u8_offset")
 
 
@@ -116,7 +138,8 @@ def _scratch(B, H, W, device, kept=False):
     key = (device.index, torch.cuda.current_stream(device).cuda_stream)
     buf = _scratch_cache.get(key)
     if buf is None or buf.numel() < need:
-        buf = torch.zeros(max(need, 1 << 16), dtype=torch.uint8, device=device)
+        with _cache_pool(device):
+            buf = torch.zeros(max(need, 1 << 16), dtype=torch.uint8, device=device)
         _scratch_cache[key] = buf
     return buf
 
@@ -129,6 +152,12 @@ def gradient(x):
     _require_cuda(x)
     if x.dim() != 3:
         raise RuntimeError(f"tcl_b200: gradient expects (B,H,W), got {tuple(x.shape)}")
+    if _traced(x):
+        return torch.ops.tcl_b200.gradient(x)
+    return _gradient_launch(x)
+
+
+def _gradient_launch(x):
     x = x.float()
     B, H, W = x.shape
     # one channel of a (B,2,H,W) flow (the reference's gradient(bf[:,0,:,:]), flowtools.py:47): planes are contiguous, only
@@ -213,6 +242,8 @@ def _warp(x, f, flags):
     if f.shape[0] != x.shape[0] or f.shape[2:] != x.shape[2:]:
         raise RuntimeError(f"tcl_b200: x {tuple(x.shape)} and flow {tuple(f.shape)} do not match")
     _frame_dtype(x)
+    if _traced(x, f):
+        return torch.ops.tcl_b200.warp(x, f if f.dtype == torch.float32 else f.float(), flags)
     x = x.contiguous()
     if torch.is_grad_enabled() and (x.requires_grad or f.requires_grad):
         return _WarpFn.apply(x, _flow(f, "f"), flags)
@@ -245,6 +276,18 @@ def _fbcheck(ff, bf, flags, device, return_near=False):
             raise RuntimeError(f"tcl_b200: ff {tuple(ff.shape)} and bf {tuple(bf.shape)} do not match")
     else:
         ff = None
+    if _traced(ff, bf):
+        out = torch.ops.tcl_b200.fbcheck(ff, bf, flags, return_near)
+        mask, near = out[0], (out[1] if return_near else None)
+    else:
+        mask, near = _fbcheck_launch(ff, bf, flags, return_near, ff_plane, ff_batch, bf_plane, bf_batch)
+    if device is not None and torch.device(device) != mask.device and torch.device(device).type != "cuda":
+        mask = mask.to(device)
+    return (mask, near) if return_near else mask
+
+
+def _fbcheck_launch(ff, bf, flags, return_near, ff_plane, ff_batch, bf_plane, bf_batch):
+    """-> (mask, near count or None); ``ff`` / ``bf`` as ``_flow_view`` left them, with its strides."""
     B, _, H, W = bf.shape
     mask = torch.empty((B, 1, H, W), dtype=torch.float32, device=bf.device)
     near = torch.zeros(1, dtype=torch.int64, device=bf.device) if return_near else None
@@ -259,9 +302,7 @@ def _fbcheck(ff, bf, flags, device, return_near=False):
             a.bf_plane_stride, a.bf_batch_stride = bf_plane, bf_batch
             a.ff_plane_stride, a.ff_batch_stride = (ff_plane, ff_batch) if ff is not None else (bf_plane, bf_batch)
             check(_cabi.lib().tclb200_tcl_forward(ctypes.byref(a), _stream_handle()))
-    if device is not None and torch.device(device) != mask.device and torch.device(device).type != "cuda":
-        mask = mask.to(device)
-    return (mask, near) if return_near else mask
+    return mask, near
 
 
 def fbcCheckTorch(ff, bf, device="cuda"):
@@ -291,6 +332,13 @@ def upsample_flow(flow, mask):
     N, _, H, W = flow.shape
     if mask.dim() != 4 or mask.shape != (N, 576, H, W):
         raise RuntimeError(f"tcl_b200: mask must be (N,576,H,W) = {(N, 576, H, W)}, got {tuple(mask.shape)}")
+    if _traced(flow, mask):
+        return torch.ops.tcl_b200.upsample_flow(flow, mask)
+    return _upsample_flow_launch(flow, mask)
+
+
+def _upsample_flow_launch(flow, mask):
+    N, _, H, W = flow.shape
     flow, mask = flow.float().contiguous(), mask.float().contiguous()
     out = torch.empty((N, 2, 8 * H, 8 * W), dtype=torch.float32, device=flow.device)
     with torch.cuda.device(flow.device):
@@ -321,6 +369,46 @@ def _index(idx, B, n_frames, name, validate=True):
     return idx.to(dtype=torch.int32).contiguous()
 
 
+def _fused_args(bf, prev, cur, ff, mask, want_sums, prev_index=None, cur_index=None, validate_index=True, bf_index=None,
+                ff_index=None, rows=None, u8_scale=None, u8_offset=None, want_kept=False):
+    """``fused_forward``'s validation: -> its arguments normalised for the launch, with B, C, H, W."""
+    _require_cuda(bf, prev, cur, ff, mask, bf_index, ff_index)
+    bf, bf_plane, bf_batch = _flow_view(bf, "bf")
+    _, _, H, W = bf.shape
+    B = bf.shape[0] if bf_index is None else int(bf_index.numel())
+    ff, ff_plane, ff_batch = _flow_view(ff, "ff") if ff is not None else (None, 0, 0)
+    bf_index = _index(bf_index, B, bf.shape[0], "bf_index", validate_index)
+    ff_index = _index(ff_index, B, ff.shape[0], "ff_index", validate_index) if ff is not None else None
+    if ff is not None and ff_index is None and ff.shape[0] != B:
+        raise RuntimeError(f"tcl_b200: ff holds {ff.shape[0]} fields for {B} pairs (pass ff_index for a bank of fields)")
+    if prev.dim() != 4 or (prev_index is None and prev.shape[0] != B) or prev.shape[2:] != bf.shape[2:]:
+        raise RuntimeError(f"tcl_b200: prev {tuple(prev.shape)} does not match flow {tuple(bf.shape)}")
+    if cur.dim() != 4 or cur.shape[1:] != prev.shape[1:] or cur.dtype != prev.dtype or (cur_index is None and cur.shape[0] != B):
+        raise RuntimeError("tcl_b200: prev and cur must have the same frame shape and dtype")
+    _require_cuda(prev_index, cur_index)
+    prev_index = _index(prev_index, B, prev.shape[0], "prev_index", validate_index)
+    cur_index = _index(cur_index, B, cur.shape[0], "cur_index", validate_index)
+    dt = _eval_frame_dtype(prev)
+    prev, cur = prev.contiguous(), cur.contiguous()
+    C = prev.shape[1]
+    norm = _u8_norm(dt, u8_scale, u8_offset, C)
+    if mask is not None and ff is None:
+        if mask.shape != (B, 1, H, W):
+            raise RuntimeError(f"tcl_b200: mask must be (B,1,H,W), got {tuple(mask.shape)}")
+        mask = mask.float().contiguous()
+    else:
+        mask = None
+    if want_kept and not want_sums:
+        raise RuntimeError("tcl_b200: want_kept needs want_sums (the kept-pixel sums come with the reduction)")
+    if rows is not None:
+        r0, r1 = int(rows[0]), int(rows[1])
+        if not (0 <= r0 < r1 <= H):
+            raise RuntimeError(f"tcl_b200: rows must satisfy 0 <= r0 < r1 <= H = {H}, got {rows}")
+        rows = (r0, r1)
+    return (bf, bf_plane, bf_batch, ff, ff_plane, ff_batch, prev, cur, mask, prev_index, cur_index, bf_index, ff_index, rows, dt, norm,
+            B, C, H, W)
+
+
 def fused_forward(bf, prev, cur, ff=None, mask=None, loss=L2, finalize=FIN_RMSE, flags=OCC | MOB,
                   want_warp=False, want_mask=False, want_blend=False, want_near=False, want_sums=True,
                   prev_index=None, cur_index=None, validate_index=True, bf_index=None, ff_index=None, pair_group=0, rows=None,
@@ -349,44 +437,15 @@ def fused_forward(bf, prev, cur, ff=None, mask=None, loss=L2, finalize=FIN_RMSE,
     each pair's evaluated pixels (the rows of ``rows`` in band mode) -- the count of pixels the computed mask keeps, the sum
     of the dataset mask, or the pixel count without a mask.  It needs ``want_sums`` and works in every mode above.
     """
-    _require_cuda(bf, prev, cur, ff, mask, bf_index, ff_index)
-    bf, bf_plane, bf_batch = _flow_view(bf, "bf")
-    _, _, H, W = bf.shape
-    B = bf.shape[0] if bf_index is None else int(bf_index.numel())
-    ff, ff_plane, ff_batch = _flow_view(ff, "ff") if ff is not None else (None, 0, 0)
-    bf_index = _index(bf_index, B, bf.shape[0], "bf_index", validate_index)
-    ff_index = _index(ff_index, B, ff.shape[0], "ff_index", validate_index) if ff is not None else None
-    if ff is not None and ff_index is None and ff.shape[0] != B:
-        raise RuntimeError(f"tcl_b200: ff holds {ff.shape[0]} fields for {B} pairs (pass ff_index for a bank of fields)")
-    if prev.dim() != 4 or (prev_index is None and prev.shape[0] != B) or prev.shape[2:] != bf.shape[2:]:
-        raise RuntimeError(f"tcl_b200: prev {tuple(prev.shape)} does not match flow {tuple(bf.shape)}")
-    if cur.dim() != 4 or cur.shape[1:] != prev.shape[1:] or cur.dtype != prev.dtype or (cur_index is None and cur.shape[0] != B):
-        raise RuntimeError("tcl_b200: prev and cur must have the same frame shape and dtype")
-    _require_cuda(prev_index, cur_index)
-    prev_index = _index(prev_index, B, prev.shape[0], "prev_index", validate_index)
-    cur_index = _index(cur_index, B, cur.shape[0], "cur_index", validate_index)
+    (bf, bf_plane, bf_batch, ff, ff_plane, ff_batch, prev, cur, mask, prev_index, cur_index, bf_index, ff_index, rows, dt, norm,
+     B, C, H, W) = _fused_args(bf, prev, cur, ff, mask, want_sums, prev_index, cur_index, validate_index, bf_index, ff_index, rows,
+                               u8_scale, u8_offset, want_kept)
     if (want_warp or want_blend) and (prev_index is not None or cur_index is not None):
         out_like = torch.empty((B,) + tuple(prev.shape[1:]), dtype=prev.dtype, device=prev.device)
     else:
         out_like = None
-    dt = _eval_frame_dtype(prev)
-    prev, cur = prev.contiguous(), cur.contiguous()
-    C = prev.shape[1]
-    norm = _u8_norm(dt, u8_scale, u8_offset, C)
     dev = bf.device
-    if mask is not None and ff is None:
-        if mask.shape != (B, 1, H, W):
-            raise RuntimeError(f"tcl_b200: mask must be (B,1,H,W), got {tuple(mask.shape)}")
-        mask = mask.float().contiguous()
-    else:
-        mask = None
     res = FusedResult()
-    if want_kept and not want_sums:
-        raise RuntimeError("tcl_b200: want_kept needs want_sums (the kept-pixel sums come with the reduction)")
-    if rows is not None:
-        r0, r1 = int(rows[0]), int(rows[1])
-        if not (0 <= r0 < r1 <= H):
-            raise RuntimeError(f"tcl_b200: rows must satisfy 0 <= r0 < r1 <= H = {H}, got {rows}")
     if want_sums:
         f64 = torch.empty(B + 2, dtype=torch.float64, device=dev)
         res.pair_sums, res.total_sums = f64[:B], f64[B:]
@@ -423,22 +482,43 @@ def fused_forward(bf, prev, cur, ff=None, mask=None, loss=L2, finalize=FIN_RMSE,
         a.n_bf_fields, a.n_ff_fields = bf.shape[0], (ff.shape[0] if ff is not None else 0)
         a.pair_group = int(pair_group)
         if rows is not None:
-            a.row_begin, a.row_end = r0, r1
+            a.row_begin, a.row_end = rows
         a.u8_scale[:], a.u8_offset[:] = norm
         a.pair_kept, a.total_kept = _ptr(res.pair_kept), _ptr(res.total_kept)
         check(_cabi.lib().tclb200_tcl_forward(ctypes.byref(a), _stream_handle()))
     return res
 
 
+# what an evaluation helper takes from its fused launch (the ``what`` of ``_evaluate`` and of the ``fused_eval`` operator)
+EVAL_TOTAL, EVAL_PAIRS, EVAL_KEPT, EVAL_BLEND = 0, 1, 2, 3
+
+
+def _evaluate(what, bf, prev, cur, ff=None, mask=None, loss=L2, finalize=FIN_RMSE, u8_scale=None, u8_offset=None):
+    """One fused launch of an evaluation helper -> ``[total_val]``, ``[pair_vals]``, ``[pair_sums, pair_kept]`` or
+    ``[blend]`` for ``what`` = EVAL_TOTAL / EVAL_PAIRS / EVAL_KEPT / EVAL_BLEND."""
+    if _traced(bf, prev, cur, ff, mask):
+        dt, norm = _fused_args(bf, prev, cur, ff, mask, what != EVAL_BLEND, u8_scale=u8_scale, u8_offset=u8_offset,
+                               want_kept=what == EVAL_KEPT)[14:16]
+        scale, offset = (list(norm[0]), list(norm[1])) if dt == U8 else (None, None)   # validated, rounded to fp32
+        return torch.ops.tcl_b200.fused_eval(bf, prev, cur, ff, mask, loss, finalize, what, scale, offset)
+    return _evaluate_launch(what, bf, prev, cur, ff, mask, loss, finalize, u8_scale, u8_offset)
+
+
+def _evaluate_launch(what, bf, prev, cur, ff, mask, loss, finalize, u8_scale, u8_offset):
+    res = fused_forward(bf, prev, cur, ff=ff, mask=mask, loss=loss, finalize=finalize, want_blend=what == EVAL_BLEND,
+                        want_sums=what != EVAL_BLEND, want_kept=what == EVAL_KEPT, u8_scale=u8_scale, u8_offset=u8_offset)
+    return ([res.total_val], [res.pair_vals], [res.pair_sums, res.pair_kept], [res.blend])[what]
+
+
 def temporal_error(ff, bf, prev, cur, u8_scale=None, u8_offset=None):
     """``computeTCL`` minus RAFT and the generator: sqrt(mean((mask*(cur - warp(prev,bf)))**2)), 0-dim tensor.
     (uint8 frames: see ``fused_forward`` for ``u8_scale`` / ``u8_offset``; the same holds for the functions below.)"""
-    return fused_forward(bf, prev, cur, ff=ff, finalize=FIN_RMSE, u8_scale=u8_scale, u8_offset=u8_offset).total_val
+    return _evaluate(EVAL_TOTAL, bf, prev, cur, ff=ff, u8_scale=u8_scale, u8_offset=u8_offset)[0]
 
 
 def temporal_error_per_pair(ff, bf, prev, cur, u8_scale=None, u8_offset=None):
     """Per-pair RMSE (B,) with the mask computed from (ff,bf) -- the batched form of ``computeTCL``."""
-    return fused_forward(bf, prev, cur, ff=ff, finalize=FIN_RMSE, u8_scale=u8_scale, u8_offset=u8_offset).pair_vals
+    return _evaluate(EVAL_PAIRS, bf, prev, cur, ff=ff, u8_scale=u8_scale, u8_offset=u8_offset)[0]
 
 
 def warping_error_per_pair(ff, bf, prev, cur, mask=None, loss=L2, finalize=FIN_RMSE, u8_scale=None, u8_offset=None):
@@ -453,9 +533,9 @@ def warping_error_per_pair(ff, bf, prev, cur, mask=None, loss=L2, finalize=FIN_R
     (B,1,H,W), or 1 everywhere when that is None too.  A soft dataset mask keeps the reference's own numerator,
     sum of (m*d)**2, over sum of m.  A pair whose mask keeps nothing gives NaN (0/0), as the torch expression does.
     uint8 frames: ``u8_scale`` / ``u8_offset`` as in ``fused_forward``."""
-    res = fused_forward(bf, prev, cur, ff=ff, mask=mask, loss=loss, finalize=finalize, want_kept=True, u8_scale=u8_scale,
-                        u8_offset=u8_offset)
-    err = res.pair_sums / (prev.shape[1] * res.pair_kept)
+    pair_sums, pair_kept = _evaluate(EVAL_KEPT, bf, prev, cur, ff=ff, mask=mask, loss=loss, finalize=finalize, u8_scale=u8_scale,
+                                     u8_offset=u8_offset)
+    err = pair_sums / (prev.shape[1] * pair_kept)
     return (err.sqrt() if finalize == FIN_RMSE else err).float()
 
 
@@ -529,6 +609,7 @@ def free_workspaces():
     _scratch_cache.clear()
     _host_ws_cache.clear()
     _loss_plans.clear()
+    _cache_pools.clear()
 
 
 def _is_channels_last(t):
@@ -660,13 +741,13 @@ def temporal_error_host(frames, ff, bf, prev_index=None, cur_index=None, mask=No
 
 def temporal_rmse_per_sample(mask, cur, prev, flow, u8_scale=None, u8_offset=None):
     """FC2 metric: ((mask*(cur - warp(prev,flow)))**2).mean(dim=(1,2,3))**0.5 -> (N,)."""
-    return fused_forward(flow, prev, cur, mask=mask, finalize=FIN_RMSE, u8_scale=u8_scale, u8_offset=u8_offset).pair_vals
+    return _evaluate(EVAL_PAIRS, flow, prev, cur, mask=mask, u8_scale=u8_scale, u8_offset=u8_offset)[0]
 
 
 def warp_blend(mask, prev, flow, img):
     """mask*warp(prev,flow) + (1-mask)*img in one pass (obst_eval.py:500)."""
     _frame_dtype(prev)   # (a warped output: float32 / bfloat16 frames only)
-    return fused_forward(flow, prev, img, mask=mask, want_blend=True, want_sums=False).blend
+    return _evaluate(EVAL_BLEND, flow, prev, img, mask=mask)[0]
 
 
 # The training loss is a ~30 us job called every iteration (solver.py:427-446, twice per step): its wrapper avoids every
@@ -739,47 +820,51 @@ class _TemporalLossFn(torch.autograd.Function):
     @torch.autograd.function.once_differentiable
     def backward(ctx, grad_out):
         prev, cur, flow, mask = ctx.saved_tensors
-        if prev.dtype != torch.float32:
-            return _loss_backward_bf16(ctx, grad_out, prev, cur, flow, mask)
-        B, C, H, W = prev.shape
-        need_prev, need_cur = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
-        gp = torch.empty_like(prev) if need_prev else None
-        gc = torch.empty_like(cur) if need_cur else None
-        # the upstream gradient as it is; the kernel multiplies it by 1/N (one rounded fp32 product, like `grad_out * (1.0 / N)`)
-        scale = grad_out if (grad_out.dtype == torch.float32 and grad_out.is_cuda) else grad_out.to(device=prev.device, dtype=torch.float32)
-        dev = prev.device
-        switch = torch.cuda.current_device() != dev.index
-        if switch:
-            dctx = torch.cuda.device(dev)
-            dctx.__enter__()
-        try:
-            plan = _loss_plan(dev, B, H, W)
-            rc = plan.bwd(flow.data_ptr(), mask.data_ptr(), prev.data_ptr(), cur.data_ptr(), scale.data_ptr(), 1.0 / float(B * C * H * W),
-                          gp.data_ptr() if gp is not None else None, gc.data_ptr() if gc is not None else None,
-                          B, C, H, W, ctx.flags, ctx.loss, plan.stream)
-            if rc != 0:
-                check(rc)
-        finally:
-            if switch:
-                dctx.__exit__(None, None, None)
+        gp, gc = _loss_backward(grad_out, prev, cur, flow, mask, ctx.loss, ctx.flags, ctx.needs_input_grad[0], ctx.needs_input_grad[1])
         return gp, gc, None, None, None, None
 
 
-def _loss_backward_bf16(ctx, grad_out, prev, cur, flow, mask):
-    """``_TemporalLossFn.backward`` for bf16 frames (``tclb200_tcl_backward_dt``): the fp32 gradients of the upcast frames,
-    each rounded once to bf16 -- what autograd gives the reference expression under ``torch.autocast(..., torch.bfloat16)``."""
+def _loss_backward(grad_out, prev, cur, flow, mask, loss, flags, need_prev, need_cur):
+    """(grad_prev, grad_cur) of the training loss, None where not needed."""
+    if prev.dtype != torch.float32:
+        return _loss_backward_bf16(grad_out, prev, cur, flow, mask, loss, flags, need_prev, need_cur)
+    B, C, H, W = prev.shape
+    gp = torch.empty_like(prev) if need_prev else None
+    gc = torch.empty_like(cur) if need_cur else None
+    # the upstream gradient as it is; the kernel multiplies it by 1/N (one rounded fp32 product, like `grad_out * (1.0 / N)`)
+    scale = grad_out if (grad_out.dtype == torch.float32 and grad_out.is_cuda) else grad_out.to(device=prev.device, dtype=torch.float32)
+    dev = prev.device
+    switch = torch.cuda.current_device() != dev.index
+    if switch:
+        dctx = torch.cuda.device(dev)
+        dctx.__enter__()
+    try:
+        plan = _loss_plan(dev, B, H, W)
+        rc = plan.bwd(flow.data_ptr(), mask.data_ptr(), prev.data_ptr(), cur.data_ptr(), scale.data_ptr(), 1.0 / float(B * C * H * W),
+                      gp.data_ptr() if gp is not None else None, gc.data_ptr() if gc is not None else None,
+                      B, C, H, W, flags, loss, plan.stream)
+        if rc != 0:
+            check(rc)
+    finally:
+        if switch:
+            dctx.__exit__(None, None, None)
+    return gp, gc
+
+
+def _loss_backward_bf16(grad_out, prev, cur, flow, mask, loss, flags, need_prev, need_cur):
+    """``_loss_backward`` for bf16 frames (``tclb200_tcl_backward_dt``): the fp32 gradients of the upcast frames, each
+    rounded once to bf16 -- what autograd gives the reference expression under ``torch.autocast(..., torch.bfloat16)``."""
     B, C, H, W = prev.shape
     dt = _frame_dtype(prev)
-    need_prev, need_cur = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
     gp = torch.empty_like(prev) if need_prev else None
     gc = torch.empty_like(cur) if need_cur else None
     scale = grad_out if (grad_out.dtype == torch.float32 and grad_out.is_cuda) else grad_out.to(device=prev.device, dtype=torch.float32)
     with torch.cuda.device(prev.device):
         ws, nbytes = _backward_workspace(B, C, H, W, dt, prev.device) if need_prev else (None, 0)
         check(_cabi.lib().tclb200_tcl_backward_dt(_ptr(flow), _ptr(mask), _ptr(prev), _ptr(cur), _ptr(scale), 1.0 / float(B * C * H * W),
-                                                  _ptr(gp), _ptr(gc), B, C, H, W, dt, ctx.flags, ctx.loss, _ptr(ws), nbytes,
+                                                  _ptr(gp), _ptr(gc), B, C, H, W, dt, flags, loss, _ptr(ws), nbytes,
                                                   _stream_handle()))
-    return gp, gc, None, None, None, None
+    return gp, gc
 
 
 def temporal_loss(mask, cur, prev, flow, loss="l2", validity=False):
@@ -816,19 +901,20 @@ def temporal_loss(mask, cur, prev, flow, loss="l2", validity=False):
     if mask.shape != (B, 1, H, W):
         raise RuntimeError(f"tcl_b200: mask must be (B,1,H,W), got {tuple(mask.shape)}")
     flags = VALIDITY if validity else 0
-    if torch.is_grad_enabled():
-        if flow.requires_grad or mask.requires_grad:
-            # a learnable flow (MoGAN's motion network: warp(fake_B, netM_A(bf)), cycle_gan_model.py:177-178,280) or a soft mask that
-            # is being trained: the fused backward has no gradient for them, so the loss is composed like the reference expression
-            # from the differentiable warp (gradients to the frame and the flow, tclb200_warp_backward) and autograd's elementwise ops.
-            # bf16 frames are upcast first, like autocast does for grid_sampler: the warp and the tail run in fp32 and the value is
-            # an fp32 scalar as on the fused path; autograd rounds the frames' gradients back to bf16
-            if prev.dtype != torch.float32:
-                prev, cur = prev.float(), cur.float()
-            w = _warp(prev, flow, flags)
-            return ((mask * (cur - w)) ** 2).mean() if code == L2 else (mask * torch.abs(w - cur)).mean()
-        if prev.requires_grad or cur.requires_grad:
-            return _TemporalLossFn.apply(prev, cur, flow, mask, code, flags)
+    if torch.is_grad_enabled() and (flow.requires_grad or mask.requires_grad):
+        # a learnable flow (MoGAN's motion network: warp(fake_B, netM_A(bf)), cycle_gan_model.py:177-178,280) or a soft mask that
+        # is being trained: the fused backward has no gradient for them, so the loss is composed like the reference expression
+        # from the differentiable warp (gradients to the frame and the flow, tclb200_warp_backward) and autograd's elementwise ops.
+        # bf16 frames are upcast first, like autocast does for grid_sampler: the warp and the tail run in fp32 and the value is
+        # an fp32 scalar as on the fused path; autograd rounds the frames' gradients back to bf16
+        if prev.dtype != torch.float32:
+            prev, cur = prev.float(), cur.float()
+        w = _warp(prev, flow, flags)
+        return ((mask * (cur - w)) ** 2).mean() if code == L2 else (mask * torch.abs(w - cur)).mean()
+    if _traced(mask, cur, prev, flow):
+        return torch.ops.tcl_b200.temporal_loss(prev, cur, flow, mask, code, flags)
+    if torch.is_grad_enabled() and (prev.requires_grad or cur.requires_grad):
+        return _TemporalLossFn.apply(prev, cur, flow, mask, code, flags)
     return _loss_forward(prev, cur, flow, mask, code, flags)
 
 
